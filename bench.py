@@ -4,6 +4,10 @@
     python bench.py --gpus 1 --steps K --warmup W               # this repo's CUDA path
     python bench.py --impl reference --gpus 1 --steps K --warmup W   # CPU arm (oracle port on host cores)
     torchrun ... bench.py --gpus N ...                           # one rank per GPU, weak scaling
+    python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR  # also write the last timed step's results
+
+The benchmark writes nothing into the source tree (which may be read-only): network specialisations that
+build() did not compile are cached in a temporary directory for the run.
 
 A "step" is one pbn_step launch over one batch of 2^20 env instances (per GPU): apply the
 agent's gene flips, draw predictor selections + perturbations from Philox, synchronous
@@ -18,13 +22,17 @@ stream; max over ranks.  The L2 (126 MB) is defeated by rotating over R independ
 batches whose combined working set exceeds it, plus a pool of distinct action buffers.
 """
 import argparse
+import atexit
 import json
 import os
+import shutil
 import sys
+import tempfile
 import threading
 import time
 from pathlib import Path
 
+sys.dont_write_bytecode = True   # no __pycache__ in the source tree
 ROOT = Path(__file__).resolve().parent
 if str(ROOT) not in sys.path:
     sys.path.insert(0, str(ROOT))
@@ -62,6 +70,19 @@ def load_workload(name):
 
 ENV_KW = dict(horizon=20, bins=3, perturb_p=0.001, perturb_mode="A", r_success=5.0, r_step=0.0, r_action=-1.0,
               seed=0x5EED)
+
+
+def use_private_jit_cache():
+    """Point the library's cubin cache (PBN_B200_CACHE) at a temporary directory that links the cubins build() left in
+    pbn_rl_b200/_jit_cache/, so that specialisations compiled at run time land there and not in the source tree.
+    The directory is removed at exit.  An explicit PBN_B200_CACHE is left alone."""
+    if os.environ.get("PBN_B200_CACHE"):
+        return
+    tmp = tempfile.mkdtemp(prefix="pbn_b200_cache_")
+    atexit.register(shutil.rmtree, tmp, True)
+    for cubin in (ROOT / "pbn_rl_b200" / "_jit_cache").glob("*.cubin"):
+        os.symlink(cubin, os.path.join(tmp, cubin.name))
+    os.environ["PBN_B200_CACHE"] = tmp
 
 
 # ----------------------------------------------------------------------------------------------
@@ -300,6 +321,31 @@ def time_steps(envs, pool, K, G, Wm, stream, world):
         return ev0.elapsed_time(ev1)
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(env, out_dir):
+    """Write what the last timed step returned to its caller, for the env batch it stepped, as DIR/<name>.npy:
+    state_u32 (float64 [E, 2W]: each int64 state word as its low and high 32-bit halves, exact in float64), reward,
+    terminated and truncated (float32 [E]).  A batch whose arrays exceed 64 MB is cut to a fixed seeded sample of envs;
+    env_index (float64) then lists the envs kept."""
+    import numpy as np
+    words = env.state.cpu().numpy().view(np.uint64)
+    e = words.shape[0]
+    out = {"state_u32": np.stack([words & 0xFFFFFFFF, words >> 32], axis=-1).reshape(e, -1).astype(np.float64),
+           "reward": env.reward.cpu().numpy().astype(np.float32),
+           "terminated": env.terminated.cpu().numpy().astype(np.float32),
+           "truncated": env.truncated.cpu().numpy().astype(np.float32)}
+    per_env = sum(a.nbytes for a in out.values()) // e
+    if per_env * e > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(e, size=DUMP_BYTES // (per_env + 8), replace=False))
+        out = {k: a[keep] for k, a in out.items()}
+        out["env_index"] = keep.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def max_over_ranks(ms, device, world):
     import torch
     import torch.distributed as dist
@@ -346,6 +392,9 @@ def run_gpu(args):
     sampler.start()
     ms = time_steps(envs, pool, K, G, Wm, stream, world)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # every replay restarts the step index at 0: the last timed step is step (K % G or G) - 1 of its graph
+        dump_outputs(envs[((K % G or G) - 1) % R], args.dump_outputs)
 
     # episode statistics: the only cross-GPU exchange of the path (one small NCCL all-reduce)
     for e in envs:
@@ -657,7 +706,14 @@ def main():
     ap.add_argument("--chain", action="store_true", help="plane-resident state with tile-chained launches (PBN_STEP_CHAIN)")
     ap.add_argument("--strong", action="store_true", help="also time the strong-scaling form at N = 1 (envs / N per GPU)")
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE configs (pbn10 x 4096, pbn70, rollout)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step (rank 0) as DIR/<name>.npy; the inputs are seeded, so two "
+                         "builds run with the same arguments can be compared output for output")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         args.steps_ref = args.steps if args.steps is not None else 20
         args.warmup_ref = args.warmup if args.warmup is not None else 3
@@ -665,6 +721,7 @@ def main():
         return
     args.steps = args.steps if args.steps is not None else 6400
     args.warmup = args.warmup if args.warmup is not None else 64
+    use_private_jit_cache()
     run_gpu(args)
 
 

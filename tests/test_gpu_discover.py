@@ -188,3 +188,30 @@ def test_bench_runs_on_a_small_configuration():
     assert d["steps"] == 10 and d["gpu_launches"] == 10 and d["value"] > 0 and d["roofline"]["bound"] == "hbm"
     assert d["e2e"]["h2d_bytes_per_step"] == 8192 * 2 and d["e2e"]["d2h_bytes_per_step"] == 8192 * 4   # packed host form
     assert d["strong"]["total_envs"] == 8192 and d["strong"]["value"] > 0 and d["configs"] is None
+
+
+def test_bench_dumps_the_same_outputs_from_run_to_run(tmp_path):
+    """bench.py --dump-outputs: the last timed step's results, identical for identical arguments; --steps is the number
+    of timed steps also when it is not a multiple of the graph length."""
+    import json
+    import subprocess
+    import sys
+    from pathlib import Path
+    root = Path(__file__).resolve().parent.parent
+    dumps = []
+    for run in ("a", "b"):
+        out = subprocess.run([sys.executable, str(root / "bench.py"), "--envs", "8192", "--batches", "2", "--steps", "7",
+                              "--graph-steps", "4", "--warmup", "3", "--no-cpu-baseline", "--no-configs", "--e2e-steps", "2",
+                              "--dump-outputs", str(tmp_path / run)], capture_output=True, text=True, timeout=600, cwd=str(root))
+        assert out.returncode == 0, out.stderr[-2000:]
+        d = json.loads(out.stdout)
+        assert d["steps"] == 7 and d["gpu_launches"] == 7
+        dumps.append({p.stem: np.load(p) for p in (tmp_path / run).glob("*.npy")})
+    a, b = dumps
+    assert sorted(a) == ["reward", "state_u32", "terminated", "truncated"]
+    assert a["state_u32"].shape == (8192, 2) and a["state_u32"].dtype == np.float64
+    assert a["state_u32"][:, 0].max() < 2**28 and not a["state_u32"][:, 1].any()   # 28-gene states
+    assert a["state_u32"][:, 0].any() and a["reward"].any()
+    assert set(np.unique(a["terminated"])) <= {0.0, 1.0} and set(np.unique(a["truncated"])) <= {0.0, 1.0}
+    for name in a:
+        assert np.array_equal(a[name], b[name]), name
