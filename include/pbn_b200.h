@@ -358,6 +358,56 @@ int pbn_replay_commit(pbn_handle* h, const pbn_replay* r, int64_t head, const ui
  * may be NULL.  The target state is the first state of the attractor with '*' -> 0 (env.reset()'s `target`). */
 int pbn_replay_sample(pbn_handle* h, const pbn_replay* r, const int64_t* index, int64_t batch, float* obs,
                       float* next_obs, int64_t* actions, float* reward, float* done, void* stream);
+/* ---- Prioritised replay over the ring's slots (proportional PER, Schaul et al.; the sum / min segment trees of
+ * the reference's data_structures.py and ddqn_per/, SURVEY.md section 2 rows 13-14, in the form of OpenAI baselines).
+ * Parity with the reference is not pinned (its tests are stale); this contract is the project's own.
+ *
+ * Layout.  L = the smallest power of two >= capacity, D = log2 L.  `tree` holds pbn_per_tree_floats(capacity) = 5L
+ * words of caller-owned DEVICE memory, every binary level of both trees stored as a heap (node k has children 2k and
+ * 2k+1, the root is node 1, leaf of slot i is node L + i):
+ *   tree[k]            k in [1, 2L)  sum tree S: leaves p[i] (fp32), S(node) = S(2 node) + S(2 node + 1), one fp32 add
+ *                                    with round-to-nearest; total = tree[1]
+ *   tree[2L + k]       k in [1, 2L)  min tree M: the same shape built with fminf; pmin = tree[2L + 1]
+ *   tree[0]                          scratch of the kernels (a completion ticket, zero between calls)
+ *   tree[4L .. 5L)                   scratch of the kernels (int32 owner per leaf, -1 between calls)
+ * Unwritten leaves are 0 in S and +inf in M.  max_p (DEVICE, one float) is the largest raw priority seen, 1.0
+ * initially.  pbn_per_init establishes this state; nothing else may write the arrays.
+ *
+ * push(head, n), after pbn_replay_commit with the same head: slots (head + e) mod capacity, e < n, get the leaf
+ *   powf(max_p, alpha), and all their ancestors are rebuilt.
+ * update(index[B], td[B], eps): raw = fminf(fmaxf(fabsf(td), 0) + eps, 1e30f) (NaN -> eps, +-inf -> 1e30, so the
+ *   trees never hold NaN or inf); the leaf becomes powf(raw, alpha); max_p = max(max_p, raw) over the valid entries.
+ *   When a slot occurs more than once the LAST occurrence in batch order wins.  Indices outside [0, capacity) are
+ *   ignored (a device-side index cannot be validated without a synchronisation).  eps > 0.
+ * sample(u[B], beta) -> index[B] (int64), weight[B] (fp32); u in [0, 1) fp32 from the caller, B <= 2^24:
+ *   seg = total / B; mass_b = fl(fl(u_b * seg) + fl(b * seg)) (no FMA); descent from the root: go left if
+ *   left > mass or right == 0, else mass = fl(mass - left) and go right -- every visited node has a positive sum,
+ *   so the result is a written slot; weight_b = powf(pmin / p[index_b], beta), which is baselines'
+ *   (P * size)^-beta / max_w with size and total cancelled: no host-side size, so the call can be captured in a
+ *   CUDA graph (with beta frozen into it).
+ * All calls run on the caller's stream without synchronising; calls on one tree must be ordered on one stream.
+ * alpha >= 0 and beta >= 0, finite; capacity <= 2^30. */
+typedef struct {
+  float* tree;           /* [pbn_per_tree_floats(capacity)] sum tree, min tree and scratch (layout above) */
+  float* max_p;          /* [1] largest raw priority so far */
+  int64_t capacity;      /* slots of the replay ring the trees index */
+  float alpha;           /* priority exponent */
+  float reserved;
+} pbn_per;
+
+/* Words of the tree array for a ring of `capacity` slots (5 * L), or a negative status. */
+int64_t pbn_per_tree_floats(int64_t capacity);
+/* Empty trees (S = 0, M = +inf), max_p = 1.0, scratch cleared. */
+int pbn_per_init(pbn_handle* h, const pbn_per* p, void* stream);
+/* New transitions enter at the running maximum priority. */
+int pbn_per_push(pbn_handle* h, const pbn_per* p, int64_t head, int64_t n, void* stream);
+/* New priorities from TD errors for ring slots index[0..B) (DEVICE int64 / fp32). */
+int pbn_per_update(pbn_handle* h, const pbn_per* p, const int64_t* index, const float* td_error, int64_t batch,
+                   float eps, void* stream);
+/* Stratified proportional sample of B slots and their importance weights (DEVICE arrays). */
+int pbn_per_sample(pbn_handle* h, const pbn_per* p, const float* u, int64_t batch, float beta, int64_t* index,
+                   float* weight, void* stream);
+
 /* The agent's network input for the live envs (predict(), bdq_model/__init__.py:92-93):
  * obs [2,E,N] float32 = (state bits, target-state bits). */
 int pbn_observe(pbn_handle* h, const uint64_t* state, const int32_t* target_id, float* obs, int64_t n_envs,

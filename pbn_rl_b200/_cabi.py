@@ -10,7 +10,7 @@ import os
 from pathlib import Path
 from typing import Optional
 
-__all__ = ["lib", "load_library", "PbnError", "NetDesc", "StepArgs", "HostIO", "Replay", "check", "LIB_PATH", "EXPORTS"]
+__all__ = ["lib", "load_library", "PbnError", "NetDesc", "StepArgs", "HostIO", "Replay", "Per", "check", "LIB_PATH", "EXPORTS"]
 
 LIB_PATH = Path(__file__).resolve().parent / "libpbn_b200.so"
 
@@ -35,6 +35,7 @@ EXPORTS = (
     "pbn_visit_count", "pbn_successor_sets", "pbn_closure_expand", "pbn_closure_reach",
     "pbn_predraw", "pbn_planes_words", "pbn_rollout",
     "pbn_resident_words", "pbn_resident_import", "pbn_resident_export", "pbn_reward_table", "pbn_attractor_hash_slots",
+    "pbn_per_tree_floats", "pbn_per_init", "pbn_per_push", "pbn_per_update", "pbn_per_sample",
 )
 
 
@@ -134,6 +135,16 @@ class Replay(C.Structure):
     ]
 
 
+class Per(C.Structure):
+    _fields_ = [
+        ("tree", C.c_void_p),
+        ("max_p", C.c_void_p),
+        ("capacity", C.c_int64),
+        ("alpha", C.c_float),
+        ("reserved", C.c_float),
+    ]
+
+
 _lib: Optional[C.CDLL] = None
 
 
@@ -166,6 +177,16 @@ def load_library(path: Optional[os.PathLike] = None) -> C.CDLL:
     lib.pbn_replay_commit.restype = C.c_int
     lib.pbn_replay_sample.argtypes = [vp, C.POINTER(Replay), vp, i64, vp, vp, vp, vp, vp, vp]
     lib.pbn_replay_sample.restype = C.c_int
+    lib.pbn_per_tree_floats.argtypes = [i64]
+    lib.pbn_per_tree_floats.restype = i64
+    lib.pbn_per_init.argtypes = [vp, C.POINTER(Per), vp]
+    lib.pbn_per_init.restype = C.c_int
+    lib.pbn_per_push.argtypes = [vp, C.POINTER(Per), i64, i64, vp]
+    lib.pbn_per_push.restype = C.c_int
+    lib.pbn_per_update.argtypes = [vp, C.POINTER(Per), vp, vp, i64, C.c_float, vp]
+    lib.pbn_per_update.restype = C.c_int
+    lib.pbn_per_sample.argtypes = [vp, C.POINTER(Per), vp, i64, C.c_float, vp, vp, vp]
+    lib.pbn_per_sample.restype = C.c_int
     lib.pbn_observe.argtypes = [vp, vp, vp, vp, i64, vp]
     lib.pbn_observe.restype = C.c_int
     lib.pbn_in_target.argtypes = [vp, vp, vp, vp, i64, vp]

@@ -18,6 +18,7 @@
 #include "evaluate.cuh"
 #include "discover.cuh"
 #include "resident.cuh"
+#include "per.cuh"
 
 using namespace pbn;
 
@@ -1349,6 +1350,118 @@ int pbn_replay_sample(pbn_handle* h, const pbn_replay* r, const int64_t* index, 
     PBN_CUDA(cudaGetLastError());
     h->launches += 1, g_last_advance = nullptr;
   }
+  return PBN_OK;
+}
+
+static int64_t per_leaves(int64_t capacity) {
+  int64_t L = 1;
+  while (L < capacity) L <<= 1;
+  return L;
+}
+
+int64_t pbn_per_tree_floats(int64_t capacity) {
+  if (capacity < 1 || capacity > (int64_t(1) << 30)) return fail(PBN_ERR_INVALID, "PER capacity=%lld outside 1..2^30", (long long)capacity);
+  return 5 * per_leaves(capacity);
+}
+
+static int check_per(const pbn_handle* h, const pbn_per* p, PerView* v) {
+  if (!h || !p || !p->tree || !p->max_p) return fail(PBN_ERR_INVALID, "PER: null argument");
+  if (p->capacity < 1 || p->capacity > (int64_t(1) << 30)) return fail(PBN_ERR_INVALID, "PER capacity=%lld outside 1..2^30", (long long)p->capacity);
+  if (!(p->alpha >= 0.0f) || std::isinf(p->alpha)) return fail(PBN_ERR_INVALID, "PER alpha=%g must be finite and >= 0", p->alpha);
+  if (reinterpret_cast<uintptr_t>(p->tree) & 3u || reinterpret_cast<uintptr_t>(p->max_p) & 3u) return fail(PBN_ERR_INVALID, "PER arrays must be 4-byte aligned");
+  v->L = per_leaves(p->capacity);
+  v->D = 0;
+  while ((int64_t(1) << v->D) < v->L) ++v->D;
+  v->sum = p->tree;
+  v->mn = p->tree + 2 * v->L;
+  v->owner = reinterpret_cast<int*>(p->tree + 4 * v->L);
+  v->ticket = reinterpret_cast<unsigned int*>(p->tree);
+  v->max_p = p->max_p;
+  v->capacity = p->capacity;
+  v->alpha = p->alpha;
+  return PBN_OK;
+}
+
+// One launch of the tile rebuild over slot ranges [a0, b0) and [a1, b1) (each tile of the grid exactly once).
+static int per_rebuild(pbn_handle* h, const PerView& v, int64_t a0, int64_t b0, int64_t a1, int64_t b1, int fill,
+                       const int64_t* reset_index, int64_t reset_n, cudaStream_t stream) {
+  PerRanges r{};
+  r.a0 = a0, r.b0 = b0, r.a1 = a1, r.b1 = b1, r.fill = fill;
+  r.lt = std::min(v.D, kPerTileLog2);
+  r.t0 = a0 >> r.lt;
+  r.n0 = ((b0 - 1) >> r.lt) - r.t0 + 1;
+  int64_t t1_end = b1 > a1 ? ((b1 - 1) >> r.lt) + 1 : 0;
+  r.t1 = a1 >> r.lt;
+  if (t1_end > r.t0) t1_end = r.t0;   // a tile the first range already covers
+  const int64_t n1 = std::max<int64_t>(0, t1_end - r.t1);
+  per_rebuild_kernel<<<(unsigned)(r.n0 + n1), kPerRebuildThreads, 0, stream>>>(v, r, reset_index, reset_n);
+  PBN_CUDA(cudaGetLastError());
+  h->launches += 1, g_last_advance = nullptr;
+  return PBN_OK;
+}
+
+int pbn_per_init(pbn_handle* h, const pbn_per* p, void* stream_) {
+  PerView v;
+  int rc = check_per(h, p, &v);
+  if (rc != PBN_OK) return rc;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  per_init_kernel<<<grid_for(h, 2 * v.L, 256, 8), 256, 0, stream>>>(v);
+  PBN_CUDA(cudaGetLastError());
+  h->launches += 1, g_last_advance = nullptr;
+  return PBN_OK;
+}
+
+int pbn_per_push(pbn_handle* h, const pbn_per* p, int64_t head, int64_t n, void* stream_) {
+  PerView v;
+  int rc = check_per(h, p, &v);
+  if (rc != PBN_OK) return rc;
+  if (head < 0 || head >= p->capacity || n < 0 || n > p->capacity) return fail(PBN_ERR_INVALID, "PER push: head=%lld, n=%lld, capacity=%lld", (long long)head, (long long)n, (long long)p->capacity);
+  if (n == 0) return PBN_OK;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  const int64_t end = head + n;
+  if (end <= p->capacity) return per_rebuild(h, v, head, end, 0, 0, 1, nullptr, 0, stream);
+  return per_rebuild(h, v, head, p->capacity, 0, end - p->capacity, 1, nullptr, 0, stream);
+}
+
+int pbn_per_update(pbn_handle* h, const pbn_per* p, const int64_t* index, const float* td_error, int64_t batch, float eps,
+                   void* stream_) {
+  PerView v;
+  int rc = check_per(h, p, &v);
+  if (rc != PBN_OK) return rc;
+  if (!index || !td_error || batch < 0 || batch > 0x7FFFFFFF) return fail(PBN_ERR_INVALID, "bad arguments");
+  if (!(eps > 0.0f) || std::isinf(eps)) return fail(PBN_ERR_INVALID, "PER eps=%g must be finite and > 0", eps);
+  if (batch == 0) return PBN_OK;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  if (batch <= kPerUpdateOneCta) {
+    per_update_cta_kernel<<<1, kPerUpdateThreads, 0, stream>>>(v, index, td_error, (int)batch, eps);
+    PBN_CUDA(cudaGetLastError());
+    h->launches += 1, g_last_advance = nullptr;
+    return PBN_OK;
+  }
+  per_update_claim_kernel<<<grid_for(h, batch, 256, 8), 256, 0, stream>>>(v, index, batch);
+  PBN_CUDA(cudaGetLastError());
+  per_update_write_kernel<<<grid_for(h, batch, 256, 8), 256, 0, stream>>>(v, index, td_error, batch, eps);
+  PBN_CUDA(cudaGetLastError());
+  h->launches += 2, g_last_advance = nullptr;
+  return per_rebuild(h, v, 0, v.L, 0, 0, 0, index, batch, stream);
+}
+
+int pbn_per_sample(pbn_handle* h, const pbn_per* p, const float* u, int64_t batch, float beta, int64_t* index,
+                   float* weight, void* stream_) {
+  PerView v;
+  int rc = check_per(h, p, &v);
+  if (rc != PBN_OK) return rc;
+  if (!u || !index || !weight || batch < 0 || batch > (int64_t(1) << 24)) return fail(PBN_ERR_INVALID, "bad arguments");
+  if (!(beta >= 0.0f) || std::isinf(beta)) return fail(PBN_ERR_INVALID, "PER beta=%g must be finite and >= 0", beta);
+  if (batch == 0) return PBN_OK;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  per_sample_kernel<<<grid_for(h, batch * 32, 256, 8), 256, 0, stream>>>(v, u, batch, beta, index, weight);
+  PBN_CUDA(cudaGetLastError());
+  h->launches += 1, g_last_advance = nullptr;
   return PBN_OK;
 }
 
