@@ -187,17 +187,10 @@ typedef struct {
   int64_t n_envs;               /* E */
   uint32_t flags;               /* PBN_STEP_* */
   uint32_t reserved;
-  const uint32_t* sel_planes;   /* [pbn_planes_words()] predictor-selection planes of THIS step drawn earlier by
-                                   pbn_predraw (sliced kernel only), or NULL: the step draws them itself */
   uint32_t* resident;           /* [pbn_resident_words()] plane-resident env state (see pbn_resident_import) or NULL.
                                    When given, it replaces state / target_id / t (which must be NULL): the step
                                    reads and writes the env state in the resident block; the per-env results
                                    reward / terminated / truncated are produced as usual */
-  uint32_t* packed_out;         /* [E] or NULL (N <= 30, row-format state): per env one word = state bits [N-1:0] of
-                                   args->state after the step (after the auto-reset, if enabled) | terminated << 30 |
-                                   truncated << 31, written by the step kernel itself.  May be a device pointer to
-                                   mapped page-locked HOST memory: the results then cross PCIe as posted writes of
-                                   the step kernel, no export pass follows (pbn_step_host's packed form) */
 } pbn_step_args;
 
 /* gym.make(...) construction: upload truth tables and constants, pick the kernel. */
@@ -266,16 +259,6 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* args, const pbn_host_io* i
 /* reward = table[n_flips + (bins + 1) * terminated], n_flips = number of distinct action values in 1..N of the env
  * (the fp32 values pbn_step writes): out[2 * (bins + 1)] (HOST). */
 int pbn_reward_table(const pbn_handle* h, float* out, int32_t n);
-
-/* Split launch (sliced kernel): the predictor-selection planes of a step depend only on (seed, env ids,
- * step counter), never on the state, so they can be drawn ahead of time -- pbn_predraw for step k+1 on a
- * second stream runs concurrently with pbn_step for step k (its Philox multiplies use the FMA pipe, the
- * step's logic the ALU pipe).  pbn_predraw reads args->step_ctr / step_ctr_dev / env_offset / n_envs exactly
- * as the pbn_step call that will consume the planes (same values => bit-identical results to the fused
- * step); planes: DEVICE buffer of pbn_planes_words(h, n_envs) 32-bit words, passed to that pbn_step as
- * args->sel_planes.  Returns PBN_ERR_UNSUPPORTED for handles running the scalar kernel. */
-int pbn_predraw(pbn_handle* h, const pbn_step_args* args, uint32_t* planes, void* stream);
-int64_t pbn_planes_words(const pbn_handle* h, int64_t n_envs);
 
 /* ---- Plane-resident env state (sliced kernel) -----------------------------------------------------------
  * The env state an agent never looks at between steps -- packed states, target ids, episode counters -- can

@@ -33,7 +33,7 @@ EXPORTS = (
     "pbn_advance_counter", "pbn_step_host", "pbn_replay_observe", "pbn_replay_commit", "pbn_replay_sample",
     "pbn_observe", "pbn_in_target", "pbn_rollout_track", "pbn_rollout_reduce",
     "pbn_visit_count", "pbn_successor_sets", "pbn_closure_expand", "pbn_closure_reach",
-    "pbn_predraw", "pbn_planes_words", "pbn_rollout",
+    "pbn_rollout",
     "pbn_resident_words", "pbn_resident_import", "pbn_resident_export", "pbn_reward_table", "pbn_attractor_hash_slots",
     "pbn_per_tree_floats", "pbn_per_init", "pbn_per_push", "pbn_per_update", "pbn_per_sample",
 )
@@ -99,9 +99,7 @@ class StepArgs(C.Structure):
         ("n_envs", C.c_int64),
         ("flags", C.c_uint32),
         ("reserved", C.c_uint32),
-        ("sel_planes", C.c_void_p),
         ("resident", C.c_void_p),
-        ("packed_out", C.c_void_p),
     ]
 
 
@@ -203,10 +201,6 @@ def load_library(path: Optional[os.PathLike] = None) -> C.CDLL:
     lib.pbn_closure_expand.restype = C.c_int
     lib.pbn_closure_reach.argtypes = [vp, vp, i64, vp, vp, vp, vp, i64, vp, vp]
     lib.pbn_closure_reach.restype = C.c_int
-    lib.pbn_predraw.argtypes = [vp, C.POINTER(StepArgs), vp, vp]
-    lib.pbn_predraw.restype = C.c_int
-    lib.pbn_planes_words.argtypes = [vp, i64]
-    lib.pbn_planes_words.restype = i64
     lib.pbn_attractor_hash_slots.argtypes = [vp]
     lib.pbn_attractor_hash_slots.restype = C.c_int
     lib.pbn_reward_table.argtypes = [vp, vp, i32]

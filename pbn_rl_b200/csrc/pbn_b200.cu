@@ -125,7 +125,6 @@ struct pbn_handle {
   cudaKernel_t jit_kernel_gen[2] = {nullptr, nullptr};  // pbn_step_sliced_gen (hash set / global table / r_wrong)
   cudaKernel_t planes_kernel[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};  // [injected][0: 4 warps, 1: 8 warps] pbn_step_planes_w*
   uint32_t planes_smem_opt_in[2][2] = {{48u * 1024u, 48u * 1024u}, {48u * 1024u, 48u * 1024u}};
-  cudaKernel_t predraw_kernel = nullptr;  // pbn_predraw_sliced of the own-RNG specialisation
   cudaKernel_t rollout_kernel = nullptr;  // pbn_rollout_sliced
   uint32_t rollout_smem_opt_in = 48u * 1024u;
   std::vector<uint32_t> surv_sliced_host;  // copied into every loaded specialisation's constant memory
@@ -136,14 +135,14 @@ struct pbn_handle {
   // pbn_step_host: two copy streams + per-chunk events (created on first use)
   static constexpr int kMaxChunks = 16;
   cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
-  static constexpr int kMaxLanes = 8;
+  static constexpr int kMaxLanes = 4;
   cudaStream_t s_lane[kMaxLanes] = {};   // lanes 2.. of the packed path (lanes 0 and 1 are s_h2d and s_d2h)
   // packed path with a device step counter: the whole step (uploads, unpack, step, export kernels of all lanes, counter
   // update) is captured once per distinct argument set and replayed as one CUDA graph launch afterwards
   struct HostGraph {
     pbn_step_args a;
     pbn_host_io io;
-    int lanes = 0, seen = 0;
+    int seen = 0;
     uint64_t launches = 0, last_use = 0;
     cudaGraphExec_t exec = nullptr;
   };
@@ -152,8 +151,6 @@ struct pbn_handle {
   uint64_t host_graph_clock = 0;
   cudaStream_t s_origin = nullptr;
   cudaEvent_t ev_done = nullptr, ev_fork = nullptr;
-  uint32_t* d_packed = nullptr;   // device staging of the packed results (copy-engine download, PBN_B200_PACKED_DMA)
-  int64_t d_packed_envs = 0;
   cudaEvent_t ev_entry = nullptr, ev_in[kMaxChunks] = {}, ev_k[kMaxChunks] = {};
 };
 
@@ -249,7 +246,6 @@ static int load_sliced(pbn_handle* h, int injected) {
   }
   PBN_CUDA(cudaLibraryGetKernel(&h->jit_kernel[injected], h->jit_lib[injected], "pbn_step_sliced"));
   PBN_CUDA(cudaLibraryGetKernel(&h->jit_kernel_gen[injected], h->jit_lib[injected], "pbn_step_sliced_gen"));
-  if (!injected) PBN_CUDA(cudaLibraryGetKernel(&h->predraw_kernel, h->jit_lib[0], "pbn_predraw_sliced"));
   if (!injected) PBN_CUDA(cudaLibraryGetKernel(&h->rollout_kernel, h->jit_lib[0], "pbn_rollout_sliced"));
   h->sliced_threads = jit::sliced_threads(h->gen);
   h->sliced_min_blocks = jit::sliced_min_blocks(h->gen);
@@ -411,9 +407,7 @@ static int launch_planes(pbn_handle* h, StepParams& p, bool injected, cudaStream
   // One tile per CTA.  (CTAs that walk two tiles were the better form for tile-chained sequences while every handle ran
   // its own copy of the kernel code -- 7.1 vs 7.6 us per 2^17-env step; with the shared module one tile per CTA wins,
   // 3.8 vs 4.25 us.)
-  int tpc = 1;
-  if (const char* env = getenv("PBN_B200_PLANES_TILES_PER_CTA")) tpc = atoi(env) > 0 ? atoi(env) : tpc;
-  int64_t grid = (tiles + tpc - 1) / tpc;
+  int64_t grid = tiles;
   const int64_t cap = (int64_t)h->num_sms * 64;
   if (grid > cap) grid = cap;
   const unsigned threads = v ? 256u : 128u;
@@ -483,7 +477,6 @@ void pbn_destroy(pbn_handle* h) {
     if (h->s_origin) cudaStreamDestroy(h->s_origin);
     if (h->ev_done) cudaEventDestroy(h->ev_done);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-    cudaFree(h->d_packed);
     if (h->ev_entry) cudaEventDestroy(h->ev_entry);
     for (int i = 0; i < pbn_handle::kMaxChunks; ++i) {
       if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]);
@@ -774,19 +767,15 @@ static int step_common(pbn_handle* h, const pbn_step_args* a, void* stream_, boo
   if (!h || !a) return fail(PBN_ERR_INVALID, "null argument");
   if (a->n_envs < 0) return fail(PBN_ERR_INVALID, "n_envs=%lld", (long long)a->n_envs);
   if (a->n_envs == 0) return PBN_OK;
-  if (a->packed_out && (h->net.n_genes > 30 || a->resident || (reinterpret_cast<uintptr_t>(a->packed_out) & 15u)))
-    return fail(PBN_ERR_INVALID, "packed_out needs N <= 30, row-format state and a 16-byte aligned array");
   if (a->resident) {
-    if (a->state || a->target_id || a->t || a->final_state || a->sel_planes)
-      return fail(PBN_ERR_INVALID, "plane-resident step: state / target_id / t / final_state / sel_planes must be null (the block holds them)");
+    if (a->state || a->target_id || a->t || a->final_state)
+      return fail(PBN_ERR_INVALID, "plane-resident step: state / target_id / t / final_state must be null (the block holds them)");
     if (h->kernel != PBN_KERNEL_SLICED) return fail(PBN_ERR_UNSUPPORTED, "plane-resident state needs the sliced kernel");
   } else if (!a->state) {
     return fail(PBN_ERR_INVALID, "state is null");
   }
   if (injected && !a->sel) return fail(PBN_ERR_INVALID, "pbn_step_injected needs args->sel");
   if (!injected && (a->sel || a->pert_mask)) return fail(PBN_ERR_INVALID, "pbn_step: sel/pert_mask must be null (use pbn_step_injected)");
-  if (a->sel_planes && (injected || h->kernel != PBN_KERNEL_SLICED)) return fail(PBN_ERR_UNSUPPORTED, "sel_planes: pre-drawn selection planes are taken by pbn_step with the sliced kernel only");
-  if (a->sel_planes && (reinterpret_cast<uintptr_t>(a->sel_planes) & 15u)) return fail(PBN_ERR_INVALID, "sel_planes must be 16-byte aligned");
   if (a->env_offset < 0 || (a->env_offset & 1023)) return fail(PBN_ERR_INVALID, "env_offset=%lld must be a non-negative multiple of 1024", (long long)a->env_offset);
   if (a->target_id && h->net.n_attr == 0) return fail(PBN_ERR_NO_ATTRACTORS, "target_id given but no attractor table uploaded");
   {
@@ -897,35 +886,21 @@ int pbn_rollout(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t step_c
   return PBN_OK;
 }
 
-int64_t pbn_planes_words(const pbn_handle* h, int64_t n_envs) {
-  if (!h || n_envs < 0) return fail(PBN_ERR_INVALID, "bad arguments");
-  if (h->kernel != PBN_KERNEL_SLICED) return fail(PBN_ERR_UNSUPPORTED, "selection planes exist for the sliced kernel only");
-  const int64_t tiles = (n_envs + 1023) / 1024;
-  const int64_t words = tiles * jit::sel_bits(h->gen) * jit::n_sel_slots(h->gen) * 32;
-  return words > 0 ? words : 4;  // never an empty buffer
-}
-
-int pbn_predraw(pbn_handle* h, const pbn_step_args* a, uint32_t* planes, void* stream_) {
-  if (!h || !a || !planes) return fail(PBN_ERR_INVALID, "null argument");
-  if (h->kernel != PBN_KERNEL_SLICED) return fail(PBN_ERR_UNSUPPORTED, "pbn_predraw: the handle runs the scalar kernel");
-  if (a->n_envs < 0 || a->env_offset < 0 || (a->env_offset & 1023)) return fail(PBN_ERR_INVALID, "bad n_envs / env_offset");
-  if (reinterpret_cast<uintptr_t>(planes) & 15u) return fail(PBN_ERR_INVALID, "planes must be 16-byte aligned");
-  if (a->n_envs == 0 || jit::n_sel_slots(h->gen) == 0) return PBN_OK;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  DeviceGuard guard(h->device);
-  int rc = load_sliced(h, 0);
-  if (rc != PBN_OK) return rc;
-  StepParams p;
-  p.a = *a;
-  p.n = h->net;
-  p.ticket = h->d_ticket;
-  int64_t grid = (a->n_envs + 1023) / 1024;
-  const int64_t cap = (int64_t)h->num_sms * 32;
-  if (grid > cap) grid = cap;
-  void* args[] = {&p, &planes};
-  PBN_CUDA(cudaLaunchKernel(reinterpret_cast<const void*>(h->predraw_kernel), dim3((unsigned)grid), dim3((unsigned)h->sliced_threads), args, 0, stream));
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+// The step arguments of envs [e0, e0 + n) of a row-format batch; actions: the device actions of the whole batch or null.
+static pbn_step_args env_range(const pbn_handle* h, const pbn_step_args* a, const uint8_t* actions, int64_t e0, int64_t n) {
+  pbn_step_args s = *a;
+  s.state = a->state + e0 * h->W;
+  s.actions = actions ? actions + e0 * h->net.bins : nullptr;
+  if (a->target_id) s.target_id = a->target_id + e0;
+  if (a->source_id) s.source_id = a->source_id + e0;
+  if (a->t) s.t = a->t + e0;
+  if (a->reward) s.reward = a->reward + e0;
+  if (a->terminated) s.terminated = a->terminated + e0;
+  if (a->truncated) s.truncated = a->truncated + e0;
+  if (a->final_state) s.final_state = a->final_state + e0 * h->W;
+  s.env_offset = a->env_offset + e0;
+  s.n_envs = n;
+  return s;
 }
 
 int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, void* stream_) {
@@ -988,23 +963,20 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
     }
   }
   // only the packed word is wanted.  (Measured: letting the step kernel write it straight into the mapped host buffer
-  // through args->packed_out -- 1024 CTAs posting 16-byte writes -- is slower over PCIe, 0.200 ms per 2^20 envs, than
-  // the 16-CTA export kernel, 0.176 ms: PBN_B200_FUSED_PACKED=1 keeps that form available for experiments.)
+  // -- 1024 CTAs posting 16-byte writes -- is slower over PCIe, 0.200 ms per 2^20 envs, than the 16-CTA export kernel,
+  // 0.176 ms.)
   const bool packed_only = zc_packed && !io->state && !io->reward && !io->terminated && !io->truncated && !io->state32 && !io->done;
-  const bool fused_packed = packed_only && (reinterpret_cast<uintptr_t>(zc_packed) & 15u) == 0 && getenv("PBN_B200_FUSED_PACKED") != nullptr;
   const int64_t E = a->n_envs, tiles = (E + 1023) / 1024;
-  // Two-lane form of the packed path: each half of the batch runs copy -> unpack -> step -> export in order on its own
-  // library stream, so nothing inside a lane needs an event, and PCIe (full duplex) carries lane 1's upload under
-  // lane 0's results.  The lanes' step kernels run concurrently, so the launch-counting update of a device step
-  // counter is not available here (host counter, or PDL sequences that advance it explicitly).
-  if (packed_only && !fused_packed && io->actions16 && io->n_chunks <= 0 && E >= (1 << 18)) {
+  // Lane form of the packed path: each lane (a slice of the batch) runs copy -> unpack -> step -> export in order on its
+  // own library stream, so nothing inside a lane needs an event, and PCIe (full duplex) carries one lane's upload under
+  // another lane's results.  The lanes' step kernels run concurrently, so they cannot each advance a device step
+  // counter: they share one counter value (see own_count below).
+  if (packed_only && io->actions16 && io->n_chunks <= 0 && E >= (1 << 18)) {
     // graph replay needs call-invariant arguments: a device counter (the host part of the step counter constant)
-    const bool graphable = a->step_ctr_dev != nullptr && getenv("PBN_B200_NO_HOST_GRAPH") == nullptr;
-    // measured on B200 / PCIe Gen5, 2^20 envs (scripts/host_lanes_probe.py): replayed graph 0.166 / 0.158 / 0.161 /
-    // 0.148 / 0.158 ms with 1 / 2 / 3 / 4 / 6 lanes; stream launches 0.175 / 0.169 / 0.167 / 0.173 / 0.189 ms
-    int lanes = graphable ? 4 : 2;
-    if (const char* env = getenv("PBN_B200_HOST_LANES")) lanes = atoi(env);
-    lanes = lanes < 1 ? 1 : (lanes > pbn_handle::kMaxLanes ? pbn_handle::kMaxLanes : lanes);
+    const bool graphable = a->step_ctr_dev != nullptr;
+    // measured on B200 / PCIe Gen5, 2^20 envs: replayed graph 0.166 / 0.158 / 0.161 / 0.148 / 0.158 ms with
+    // 1 / 2 / 3 / 4 / 6 lanes; stream launches 0.175 / 0.169 / 0.167 / 0.173 / 0.189 ms
+    const int lanes = graphable ? 4 : 2;
     const int64_t per = ((tiles + lanes - 1) / lanes) * 1024;   // envs per lane: whole tiles
     // a device step counter that the steps themselves advance (no PDL sequence): the lanes share one counter value
     // (PBN_STEP_NO_COUNT) and one small launch adds 1 after they have joined
@@ -1017,64 +989,28 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
     for (int c = 2; c < lanes; ++c)
       if (!h->s_lane[c]) PBN_CUDA(cudaStreamCreateWithFlags(&h->s_lane[c], cudaStreamNonBlocking));
     // everything of one step on the library's streams, forked from and joined into s_origin
-    // PBN_B200_HOST_TRACE=1 (development; eager launches only): time stamps after every operation of every lane
-    static const bool trace = getenv("PBN_B200_HOST_TRACE") != nullptr;
-    static cudaEvent_t tev[pbn_handle::kMaxLanes][5], tev0;
-    static bool tev_made = false;
-    if (trace && !tev_made) {
-      cudaEventCreate(&tev0);
-      for (auto& row : tev) for (auto& e : row) cudaEventCreate(&e);
-      tev_made = true;
-    }
-    static const bool dma = getenv("PBN_B200_PACKED_DMA") != nullptr;
-    static const int export_ctas = getenv("PBN_B200_EXPORT_CTAS") ? atoi(getenv("PBN_B200_EXPORT_CTAS")) : 16;
-    if (dma && h->d_packed_envs < E) {
-      cudaFree(h->d_packed);
-      h->d_packed = nullptr;
-      h->d_packed_envs = 0;
-      PBN_CUDA(cudaMalloc(&h->d_packed, (size_t)E * 4));
-      h->d_packed_envs = E;
-    }
     auto enqueue = [&]() -> int {
       PBN_CUDA(cudaEventRecord(h->ev_fork, h->s_origin));
-      if (trace) cudaEventRecord(tev0, h->s_origin);
       for (int c = 0; c < lanes; ++c) {
         const int64_t e0 = c * per, n = (E - e0 < per) ? E - e0 : per;
         if (n <= 0) continue;
         cudaStream_t S = c == 0 ? h->s_h2d : (c == 1 ? h->s_d2h : h->s_lane[c]);
         PBN_CUDA(cudaStreamWaitEvent(S, h->ev_fork, 0));
-        if (trace) cudaEventRecord(tev[c][0], S);
         PBN_CUDA(cudaMemcpyAsync(io->actions16_dev + e0, io->actions16 + e0, (size_t)n * 2, cudaMemcpyHostToDevice, S));
-        if (trace) cudaEventRecord(tev[c][1], S);
         unpack_actions16_kernel<<<grid_for(h, n / 4 + 1, 256, 4), 256, 0, S>>>(io->actions16_dev + e0, io->actions_dev + e0 * h->net.bins, n);
         PBN_CUDA(cudaGetLastError());
-        if (trace) cudaEventRecord(tev[c][2], S);
-        pbn_step_args s = *a;
-        s.state = a->state + e0 * h->W;
-        s.actions = io->actions_dev + e0 * h->net.bins;
-        if (a->target_id) s.target_id = a->target_id + e0;
-        if (a->source_id) s.source_id = a->source_id + e0;
-        if (a->t) s.t = a->t + e0;
-        if (a->reward) s.reward = a->reward + e0;
-        s.terminated = a->terminated + e0;
-        s.truncated = a->truncated + e0;
-        if (a->final_state) s.final_state = a->final_state + e0 * h->W;
-        s.env_offset = a->env_offset + e0;
-        s.n_envs = n;
+        pbn_step_args s = env_range(h, a, io->actions_dev, e0, n);
         s.flags = (a->flags & ~PBN_STEP_PDL) | PBN_STEP_NO_COUNT;
         const int rc = step_common(h, &s, S, false);
         if (rc != PBN_OK) return rc;
-        if (trace) cudaEventRecord(tev[c][3], S);
         ExportArgs x{};
         x.state64 = a->state + e0;
         x.term = a->terminated + e0;
         x.trunc = a->truncated + e0;
-        x.packed = dma ? h->d_packed + e0 : zc_packed + e0;
+        x.packed = zc_packed + e0;
         x.n_envs = n;
-        export_kernel<<<dma ? 4 * h->num_sms : export_ctas, 256, 0, S>>>(x);
+        export_kernel<<<16, 256, 0, S>>>(x);
         PBN_CUDA(cudaGetLastError());
-        if (dma) PBN_CUDA(cudaMemcpyAsync(io->packed + e0, h->d_packed + e0, (size_t)n * 4, cudaMemcpyDeviceToHost, S));
-        if (trace) cudaEventRecord(tev[c][4], S);
         h->launches += 2;   // (+ the step kernel, counted by step_common)
         PBN_CUDA(cudaEventRecord(h->ev_k[c], S));
         PBN_CUDA(cudaStreamWaitEvent(h->s_origin, h->ev_k[c], 0));
@@ -1092,7 +1028,7 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
     if (graphable) {
       pbn_handle::HostGraph* lru = &h->host_graph[0];
       for (auto& g : h->host_graph) {
-        if (g.seen && g.lanes == lanes && memcmp(&g.a, a, sizeof(*a)) == 0 && memcmp(&g.io, io, sizeof(*io)) == 0) slot = &g;
+        if (g.seen && memcmp(&g.a, a, sizeof(*a)) == 0 && memcmp(&g.io, io, sizeof(*io)) == 0) slot = &g;
         if (g.last_use < lru->last_use) lru = &g;
       }
       if (!slot) {
@@ -1101,7 +1037,6 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
         *slot = pbn_handle::HostGraph{};
         memcpy(&slot->a, a, sizeof(*a));
         memcpy(&slot->io, io, sizeof(*io));
-        slot->lanes = lanes;
       }
       slot->last_use = ++h->host_graph_clock;
     }
@@ -1137,14 +1072,6 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
     PBN_CUDA(cudaEventRecord(h->ev_done, h->s_origin));
     PBN_CUDA(cudaStreamWaitEvent(stream, h->ev_done, 0));   // later work on the caller's stream sees the step
     PBN_CUDA(cudaEventSynchronize(h->ev_done));
-    if (trace && !(slot && slot->exec)) {
-      for (int c = 0; c < lanes; ++c) {
-        float t[5];
-        for (int k = 0; k < 5; ++k) cudaEventElapsedTime(&t[k], tev0, tev[c][k]);
-        fprintf(stderr, "[pbn host trace] lane %d: start %.1f  upload done %.1f  unpack %.1f  step %.1f  export %.1f us\n", c,
-                t[0] * 1e3f, t[1] * 1e3f, t[2] * 1e3f, t[3] * 1e3f, t[4] * 1e3f);
-      }
-    }
     return PBN_OK;
   }
   int64_t nc = io->n_chunks > 0 ? io->n_chunks : (E >= (1 << 18) ? 2 : 1);  // measured best on B200 / PCIe Gen5 (scripts/host_path_probe.py)
@@ -1171,24 +1098,11 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
       PBN_CUDA(cudaEventRecord(h->ev_in[c], h->s_h2d));
       PBN_CUDA(cudaStreamWaitEvent(stream, h->ev_in[c], 0));
     }
-    pbn_step_args s = *a;
-    s.state = a->state + e0 * W;
-    s.actions = (io->actions || io->actions16) ? io->actions_dev + e0 * bins : nullptr;
-    if (a->target_id) s.target_id = a->target_id + e0;
-    if (a->source_id) s.source_id = a->source_id + e0;
-    if (a->t) s.t = a->t + e0;
-    if (a->reward) s.reward = a->reward + e0;
-    if (a->terminated) s.terminated = a->terminated + e0;
-    if (a->truncated) s.truncated = a->truncated + e0;
-    if (a->final_state) s.final_state = a->final_state + e0 * W;
-    s.env_offset = a->env_offset + e0;
-    s.n_envs = n;
+    pbn_step_args s = env_range(h, a, (io->actions || io->actions16) ? io->actions_dev : nullptr, e0, n);
     // the chunks are one logical step: one counter value; PDL only orders kernels, which the event waits already do
     s.flags = (a->flags & ~PBN_STEP_PDL) | ((last && !(a->flags & PBN_STEP_PDL)) ? 0u : PBN_STEP_NO_COUNT);
-    if (fused_packed) s.packed_out = zc_packed + e0;   // the step kernel writes the results over PCIe itself
     const int rc = step_common(h, &s, stream_, false);
     if (rc != PBN_OK) return rc;
-    if (fused_packed) continue;
     PBN_CUDA(cudaEventRecord(h->ev_k[c], stream));
     PBN_CUDA(cudaStreamWaitEvent(h->s_d2h, h->ev_k[c], 0));
     if (zero_copy) {
@@ -1221,11 +1135,6 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
     if (io->reward) PBN_CUDA(cudaMemcpyAsync(io->reward + e0, a->reward + e0, (size_t)n * 4, cudaMemcpyDeviceToHost, h->s_d2h));
     if (io->terminated) PBN_CUDA(cudaMemcpyAsync(io->terminated + e0, a->terminated + e0, (size_t)n, cudaMemcpyDeviceToHost, h->s_d2h));
     if (io->truncated) PBN_CUDA(cudaMemcpyAsync(io->truncated + e0, a->truncated + e0, (size_t)n, cudaMemcpyDeviceToHost, h->s_d2h));
-  }
-  if (fused_packed) {
-    PBN_CUDA(cudaEventRecord(h->ev_k[0], stream));
-    PBN_CUDA(cudaEventSynchronize(h->ev_k[0]));
-    return PBN_OK;
   }
   PBN_CUDA(cudaStreamSynchronize(h->s_d2h));
   return PBN_OK;

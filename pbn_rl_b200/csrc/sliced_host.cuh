@@ -230,7 +230,6 @@ inline int scratch_words(const GenNet& g) {
 
 inline int sliced_threads(const GenNet&) { return 128; }  // four warps per 1024-env tile
 inline int sliced_min_blocks(const GenNet& g) {
-  if (const char* env = getenv("PBN_B200_MIN_BLOCKS")) return atoi(env);  // tuning experiments
   // one-word states: 7 CTAs per SM (72 registers) -- a 2^20-env step is 1024 tiles on 148 SMs, 6.9 per SM: with 8 slots
   // the CTAs of the next launch pile up on the SMs that finish first (5..8 per SM) and the slowest SM sets the period
   // (measured 16.5 -> 16.1 us per step)
@@ -500,7 +499,6 @@ inline void generate_parts(const GenNet& g, std::string& u) {
 
 // CTAs per SM the plane-resident kernel is compiled for (register cap = 65536 / (threads * blocks))
 inline int planes_min_blocks(const GenNet& g, int warps) {
-  if (const char* env = getenv(warps == 4 ? "PBN_B200_PLANES_BLOCKS_W4" : "PBN_B200_PLANES_BLOCKS_W8")) return atoi(env);
   if (warps == 4) return g.n_genes <= 32 ? 8 : 4;
   return g.n_genes <= 32 ? 4 : 3;
 }
@@ -729,7 +727,7 @@ inline bool profile_build() {
 }
 
 // Compile (or fetch from the cache) the specialisation; returns 0 or PBN_ERR_JIT with *err set.
-// part 0: the row-format kernels (pbn_step_sliced, pbn_rollout_sliced, pbn_predraw_sliced); part 1: the plane-resident
+// part 0: the row-format kernels (pbn_step_sliced, pbn_rollout_sliced); part 1: the plane-resident
 // kernels (pbn_step_planes_w4 / _w8), compiled and loaded on first use -- two programs, so that an env that never
 // uses one family never pays its compile time.
 inline int compile(const GenNet& g, bool injected, int part, std::vector<char>* cubin, std::string* err) {
@@ -737,12 +735,9 @@ inline int compile(const GenNet& g, bool injected, int part, std::vector<char>* 
   generate(g, injected, &gen_h, &upd);
   const std::string main_src = main_source();
   const bool profile = profile_build();
-  // PBN_B200_EXP=<n>: development experiments compiled into the kernels (never set in production)
-  std::string exp_opt = "-DPBN_EXP=0";
-  if (const char* env = getenv("PBN_B200_EXP")) exp_opt = std::string("-DPBN_EXP=") + env;
-  const char* opts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo", "-default-device", exp_opt.c_str(),
+  const char* opts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo", "-default-device",
                         part ? "-DPBN_BUILD=1" : "-DPBN_BUILD=0", "-DPBN_PROFILE=1"};
-  const int n_opts = profile ? 7 : 6;
+  const int n_opts = profile ? 6 : 5;
   std::string key = gen_h + upd + main_src + kSrc_step_sliced + kSrc_step_planes + kSrc_pbn_common + kSrc_philox + kSrc_pbn_b200_h;
   for (int i = 0; i < n_opts; ++i) key += opts[i];
   char name[64];

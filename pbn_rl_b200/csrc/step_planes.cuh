@@ -227,10 +227,7 @@ __device__ __forceinline__ void step_planes_body(const StepParams& p, const Plan
       hi[k] = s1;
     }
 #else
-    if (PBN_EXP == 5) {
-#pragma unroll
-      for (int k = 0; k < PBN_MAXS4; ++k) { lo[k] = (uint32_t)gid * 2654435761u + k; hi[k] = ~lo[k] & ((uint32_t)step_ctr + k * 77u); }
-    } else if (WARPS == 4) {
+    if (WARPS == 4) {
       pbn_draw_group(w, gid, step_ctr, n.rk, lo, hi);
     } else if (w >= 4u) {
       // 8-warp variant: warp g + 4 draws the private blocks of group g's odd slots while warp g draws the even ones,
@@ -362,7 +359,6 @@ __device__ __forceinline__ void step_planes_body(const StepParams& p, const Plan
 #pragma unroll
       for (int g = 0; g < GPT; ++g) {
         nfb[g] = 0u;
-        if (PBN_EXP == 6) continue;
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
           const uint32_t bit = bit0 << (4 * g + c);
@@ -442,10 +438,6 @@ __device__ __forceinline__ void step_planes_body(const StepParams& p, const Plan
 #pragma unroll
       for (int h = 0; h < PARTS; ++h) {
         const uint32_t q = w + (uint32_t)WARPS * h;
-#if PBN_EXP == 4
-        d |= pbn_eval_part<PBN_PERT_A>(q, X, O, TG, m, lo, hi);
-        continue;
-#endif
         if (pm == PBN_PERT_NONE) d |= pbn_eval_part<PBN_PERT_NONE>(q, X, O, TG, m, lo, hi);
         else if (pm == PBN_PERT_A) d |= pbn_eval_part<PBN_PERT_A>(q, X, O, TG, m, lo, hi);
         else if (pm == PBN_PERT_B) d |= pbn_eval_part<PBN_PERT_B>(q, X, O, TG, m, lo, hi);
@@ -534,7 +526,7 @@ __device__ __forceinline__ void step_planes_body(const StepParams& p, const Plan
     //      read-modify-write of its own word -- no atomics (two finished envs of a column share the word, but the
     //      thread owns the whole word), no bank conflicts (lane == bank).  [the first form wrote every bit of a
     //      finished env with a pair of shared-memory atomics: 4 N + 16 per env, a third of the step at N = 70]
-    if ((a.flags & PBN_STEP_AUTORESET) && PBN_EXP != 2) {
+    if (a.flags & PBN_STEP_AUTORESET) {
       uint16_t* const jobs = reinterpret_cast<uint16_t*>(sm + kPlJobs) + w * (32 * 4 * GPT);
       uint32_t* const rinfo = sm + kPlRinfo;
       const uint32_t cnt = (uint32_t)__popc(Dm);

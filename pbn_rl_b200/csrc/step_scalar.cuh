@@ -246,7 +246,6 @@ __global__ void __launch_bounds__(256) step_scalar_kernel(const __grid_constant_
 #pragma unroll
     for (int w = 0; w < W; ++w) a.state[e * W + w] = nx[w];
     if (a.t != nullptr) a.t[e] = (uint16_t)tt;
-    if (a.packed_out != nullptr) a.packed_out[e] = (uint32_t)nx[0] | (hit ? 1u << 30 : 0u) | (trunc ? 1u << 31 : 0u);
   }
 
   if (a.stats != nullptr) {

@@ -79,13 +79,11 @@ constexpr uint32_t kEvCap = kEvPerWord * kEvWords;   // 4 events for N <= 31, el
 constexpr uint32_t kEvMask = (1u << kEvBits) - 1u;
 constexpr uint32_t kPreEvOverflow = 0u;
 static_assert(kSlots < (int)kEvMask, "pre-drawn event positions do not fit their field");
-constexpr int kPlaneWords = PBN_SELBITS * PBN_NSEL * 32;   // pre-drawn selection planes of one tile: [sel0 | sel1 (| sel2)][slot][lane]
 #if PBN_SELBITS == 3
 #define PBN_SEL2_OF(sel1) (sel1) + PBN_NSEL * 32,
 #else
 #define PBN_SEL2_OF(sel1)
 #endif
-static_assert((kScrSel0 * 4) % 16 == 0, "TMA destination of the selection planes must be 16-byte aligned");
 static_assert(kScrWords == PBN_SCRATCH_WORDS, "host and device disagree on the scratch size");
 static_assert(PBN_THREADS == 32 * kWarps, "one tile per 4-warp CTA");
 
@@ -415,11 +413,6 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
   uint32_t* sel1 = scr + kScrSel1 + lane;
   uint32_t* s_stat = scr + kScrStat;
 
-#if PBN_INJECTED
-  constexpr bool planes_given = false;
-#else
-  const bool planes_given = a.sel_planes != nullptr;  // block-uniform
-#endif
   phase_stamp(a, 0);
   // ---- A0. start the tile's input traffic (consumed after C1, which hides the latency) ---------------
   // full tiles: one thread issues two TMA bulk copies (8 KB*W of state, 1024*BINS action bytes) into the
@@ -427,12 +420,9 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
   if (FULL && threadIdx.x == 0) {
     fence_proxy_async();  // the previous tile's generic-proxy reads of the staging buffers are done
     const uint32_t sbytes = 1024u * 8u * kW64, abytes = 1024u * PBN_BINS;
-    const uint32_t pbytes = (planes_given && PBN_NSEL > 0) ? kPlaneWords * 4u : 0u;
-    mbar_expect_tx(mbar, sbytes + (a.actions != nullptr ? abytes : 0u) + pbytes);
+    mbar_expect_tx(mbar, sbytes + (a.actions != nullptr ? abytes : 0u));
     tma_load_1d(st_state, a.state + tile * 1024 * kW64, sbytes, mbar);
     if (a.actions != nullptr) tma_load_1d(st_act, a.actions + tile * 1024 * PBN_BINS, abytes, mbar);
-    // selection planes drawn ahead of time by pbn_predraw: straight into the SEL scratch ([sel0 | sel1][slot][lane])
-    if (pbytes) tma_load_1d(scr + kScrSel0, a.sel_planes + tile * kPlaneWords, pbytes, mbar);
   }
   uint32_t nfp = 0u;     // 4-bit flip counts of the 8 envs
   uint32_t flips = 0u;
@@ -467,7 +457,7 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
   // b, b + #SMs, b + 2 #SMs, ... land on the same SM; the tile parity would not mix: 148 is even)
   unsigned int nsm;
   asm("mov.u32 %0, %%nsmid;" : "=r"(nsm));
-  const bool c1_first = !pre_drawn && !planes_given && ((tile / (int64_t)nsm) & 1) == 0;
+  const bool c1_first = !pre_drawn && ((tile / (int64_t)nsm) & 1) == 0;
   if (stage && !c1_first) stage_tables<ASMEM>(n, L, s_surv, s_rew, s_aoffs, s_aent, s_stat);
   phase_stamp(a, 2);
   const uint64_t gid = (uint64_t)(((a.env_offset >> 10) + tile) * 32 + lane);
@@ -593,18 +583,7 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
   }
 
   phase_stamp(a, 6);
-  if (!c1_first && !pre_drawn && !planes_given) draw_selection_planes<FULL>(a, n, sel0, sel1, gid, step_ctr, e0, w);
-  if (!FULL && planes_given) {  // ragged tile: no TMA, plain loads of the pre-drawn planes
-    const uint32_t* gp = a.sel_planes + tile * kPlaneWords + lane;
-#pragma unroll 1
-    for (int r = (int)w; r < PBN_NSEL; r += kWarps) {
-      sel0[r * 32] = gp[r * 32];
-      sel1[r * 32] = gp[(PBN_NSEL + r) * 32];
-#if PBN_SELBITS == 3
-      sel1[(PBN_NSEL + r) * 32] = gp[(2 * PBN_NSEL + r) * 32];
-#endif
-    }
-  }
+  if (!c1_first && !pre_drawn) draw_selection_planes<FULL>(a, n, sel0, sel1, gid, step_ctr, e0, w);
   __syncthreads();  // (2) all input planes (and selection planes) are in scratch; S1 rows are dead
 
   // ---- C2. synchronous update of this warp's genes: generated LOP3 trees -> OPL planes ----------
@@ -903,10 +882,6 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
         for (int q = 0; q < 2 * kW64; ++q)
           fp[q] = make_ulonglong2(y[(2 * q) / kW64][(2 * q) % kW64], y[(2 * q + 1) / kW64][(2 * q + 1) % kW64]);
       }
-      if (PBN_EXP != 7 && a.packed_out != nullptr)   // (kW64 == 1: the host admits N <= 30 only)
-        *reinterpret_cast<uint4*>(a.packed_out + e) =
-            make_uint4((uint32_t)y[0][0] | ((hbits & 1u) << 30) | ((tbits & 1u) << 31), (uint32_t)y[1][0] | (((hbits >> 1) & 1u) << 30) | (((tbits >> 1) & 1u) << 31),
-                       (uint32_t)y[2][0] | (((hbits >> 2) & 1u) << 30) | (((tbits >> 2) & 1u) << 31), (uint32_t)y[3][0] | (((hbits >> 3) & 1u) << 30) | (((tbits >> 3) & 1u) << 31));
       if (a.reward != nullptr) *reinterpret_cast<float4*>(a.reward + e) = make_float4(rw[0], rw[1], rw[2], rw[3]);
       if (a.terminated != nullptr) *reinterpret_cast<uint32_t*>(a.terminated + e) = hbytes;
       if (a.truncated != nullptr) *reinterpret_cast<uint32_t*>(a.truncated + e) = tbytes;
@@ -922,7 +897,6 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
           a.state[(e + c) * kW64 + wd] = y[c][wd];
           if (a.final_state != nullptr) a.final_state[(e + c) * kW64 + wd] = y[c][wd];
         }
-        if (PBN_EXP != 7 && a.packed_out != nullptr) a.packed_out[e + c] = (uint32_t)y[c][0] | (((hbits >> c) & 1u) << 30) | (((tbits >> c) & 1u) << 31);
         if (a.reward != nullptr) a.reward[e + c] = rw[c];
         if (a.terminated != nullptr) a.terminated[e + c] = (uint8_t)((hbits >> c) & 1u);
         if (a.truncated != nullptr) a.truncated[e + c] = (uint8_t)((tbits >> c) & 1u);
@@ -935,15 +909,6 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
   // ---- G. auto-reset of finished envs (sparse: scattered writes after the vector stores) ----------
   uint32_t D = (H | TR) & VALID;
   if (a.stats != nullptr) {
-#if PBN_EXP == 8
-    const uint32_t v[7] = {(uint32_t)__popc(VALID), (uint32_t)__popc(D), (uint32_t)__popc(H & VALID),
-                           (uint32_t)__popc(TR & VALID), len_sum, flips, npert};
-#pragma unroll
-    for (int q = 0; q < 7; ++q) {
-      const uint32_t x = __reduce_add_sync(0xFFFFFFFFu, v[q]);
-      if (lane == 0u && x != 0u) atomicAdd(&s_stat[q], x);
-    }
-#else
     // the per-thread counts are small (8 envs): two 16-bit fields per warp reduction
     const uint32_t x0 = __reduce_add_sync(0xFFFFFFFFu, (uint32_t)__popc(VALID) | ((uint32_t)__popc(H & VALID) << 16));
     const uint32_t x1 = __reduce_add_sync(0xFFFFFFFFu, (uint32_t)__popc(TR & VALID) | (npert << 16));
@@ -959,10 +924,9 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
       if (x2) atomicAdd(&s_stat[PBN_STAT_FLIPS], x2);
       if (x1 >> 16) atomicAdd(&s_stat[PBN_STAT_PERTURBED], x1 >> 16);
     }
-#endif
   }
   if (a.flags & PBN_STEP_AUTORESET) {
-    auto do_reset = [&](int64_t env, const Philox4& r, uint32_t flag_bits) {
+    auto do_reset = [&](int64_t env, const Philox4& r) {
       uint64_t s[kW64];
       int src, tgt;
       if (attr_in_smem) {
@@ -981,7 +945,6 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
       a.target_id[env] = tgt;
       if (a.source_id != nullptr) a.source_id[env] = src;
       a.t[env] = 0;
-      if (PBN_EXP != 7 && a.packed_out != nullptr) a.packed_out[env] = (uint32_t)s[0] | flag_bits;   // the state after the reset, the flags of the step
     };
     // The finished envs of the warp (about 13 of its 256 per step) are dealt out over its lanes, one per lane and
     // trip: a single Philox pass instead of a per-lane serial loop that runs for as long as the unluckiest lane.
@@ -1006,14 +969,13 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
       L = min(L, 31u);
       const uint32_t eL = __shfl_sync(0xFFFFFFFFu, excl, (int)L);
       const uint32_t DL = __shfl_sync(0xFFFFFFFFu, D, (int)L);
-      const uint32_t HL = PBN_EXP != 7 ? __shfl_sync(0xFFFFFFFFu, H, (int)L) : 0u;
       if (j < total) {
         uint32_t m = DL;
         for (uint32_t k = j - eL; k != 0u; --k) m &= m - 1u;   // drop the k lowest finished envs of the owner
         const int i = __ffs(m) - 1;
         const int64_t env = tile * 1024 + 4 * (int64_t)L + 128 * (2 * (int)w + (i >> 2)) + (i & 3);
         const Philox4 r = philox_stream_rk((uint64_t)(a.env_offset + env), step_ctr, PBN_RNG_RESET, 0, n.rk);
-        do_reset(env, r, ((HL >> i) & 1u) ? (1u << 30) : (1u << 31));
+        do_reset(env, r);
       }
     }
   }
@@ -1067,11 +1029,9 @@ __device__ __forceinline__ void step_sliced_body(const StepParams& p, const Slic
       const uint64_t gid = (uint64_t)(((a.env_offset >> 10) + tile) * 32 + lane);
       // (measured: letting only every other CTA of an SM draw here and the rest after phase B -- so that their
       // Philox overlaps the others' main phases -- is slower, 23.1 vs 19.1 us: time before the wait is free)
-      if (a.sel_planes == nullptr) {
-        draw_selection_planes<false>(a, n, scr + kScrSel0 + lane, scr + kScrSel1 + lane, gid, step_ctr,
-                                     tile * 1024 + 4 * (int64_t)lane, w);
-        pre_drawn = true;
-      }
+      draw_selection_planes<false>(a, n, scr + kScrSel0 + lane, scr + kScrSel1 + lane, gid, step_ctr,
+                                   tile * 1024 + 4 * (int64_t)lane, w);
+      pre_drawn = true;
 #if !PBN_INJECTED
       draw_pert_events(n, scr + kScrEv + threadIdx.x, gid, step_ctr, w, reinterpret_cast<unsigned char*>(scr + kScrPm) + 4u * lane + w);
       ev_drawn = true;
@@ -1291,21 +1251,6 @@ pbn_rollout_sliced(const __grid_constant__ RolloutParams p) {
   if (p.stats != nullptr && threadIdx.x == 0) {
     atomicAdd(&p.stats[PBN_STAT_STEPS], (unsigned long long)s_stat[0] * (unsigned long long)p.n_steps);
     if (s_stat[1]) atomicAdd(&p.stats[PBN_STAT_PERTURBED], (unsigned long long)s_stat[1]);
-  }
-}
-
-// pbn_predraw: the selection planes of one step for every tile, into global memory.  Needs no shared
-// memory and few registers, so its CTAs fit next to the step kernel's on every SM.
-extern "C" __global__ void __launch_bounds__(PBN_THREADS, 8)
-pbn_predraw_sliced(const __grid_constant__ StepParams p, uint32_t* __restrict__ planes) {
-  const pbn_step_args& a = p.a;
-  const uint64_t step_ctr = effective_step(a);
-  const int64_t n_tiles = (a.n_envs + 1023) >> 10;
-  const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
-  for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-    const uint64_t gid = (uint64_t)(((a.env_offset >> 10) + tile) * 32 + lane);
-    uint32_t* base = planes + tile * kPlaneWords + lane;
-    draw_selection_planes<true>(a, p.n, base, base + PBN_NSEL * 32, gid, step_ctr, tile * 1024 + 4 * (int64_t)lane, w);
   }
 }
 #endif

@@ -19,7 +19,7 @@ from ._cabi import NetDesc, StepArgs, check
 from .attractors import AttractorSet
 from .network import PBNNetwork
 
-__all__ = ["VecPBNEnv", "StepPipeline", "survival_table", "pair_thresholds", "make_desc", "precompile", "jit_source"]
+__all__ = ["VecPBNEnv", "survival_table", "pair_thresholds", "make_desc", "precompile", "jit_source"]
 
 
 def survival_table(p: float, n_genes: int) -> np.ndarray:
@@ -98,48 +98,6 @@ def jit_source(network: PBNNetwork, bins: int = 3, injected: bool = False) -> st
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
     return None if t is None else t.data_ptr()
-
-
-class StepPipeline:
-    """Split-launch stepping of a :class:`VecPBNEnv` (sliced kernel): ``pbn_predraw`` for step k+1 runs on a
-    side stream concurrently with ``pbn_step`` for step k -- the Philox multiplies of the selection planes
-    (FMA pipe, few registers, no shared memory) fill the issue slots the step's logic (ALU pipe) leaves
-    idle.  Results are bit-identical to fused steps.  Works inside CUDA-graph capture (the fork/join
-    becomes graph edges).  Call :meth:`flush` whenever the step counter base changes behind the
-    pipeline's back (``advance_counter``, ``reset`` with a device counter)."""
-
-    def __init__(self, env: "VecPBNEnv"):
-        self.env = env
-        self.bufs = [env.planes_buffer(), env.planes_buffer()]
-        self.side = torch.cuda.Stream(env.device)
-        self.cur = 0
-        self.ready = False
-
-    def flush(self) -> None:
-        self.ready = False
-
-    def step(self, actions: Optional[torch.Tensor], last: bool = False, **kw):
-        """``env.step(actions)``; ``last=True`` ends the sequence (nothing is drawn ahead)."""
-        env = self.env
-        main = torch.cuda.current_stream(env.device)
-        if not self.ready:
-            env.predraw(self.bufs[self.cur])          # first step of a sequence: drawn in line
-        if not last:
-            fork = torch.cuda.Event()
-            fork.record(main)                          # everything before this step (incl. the reader of bufs[nxt]) is done
-            self.side.wait_event(fork)
-            with torch.cuda.stream(self.side):
-                env.predraw(self.bufs[self.cur ^ 1], ahead=1)
-                join = torch.cuda.Event()
-                join.record(self.side)
-        out = env.step(actions, planes=self.bufs[self.cur], **kw)
-        if not last:
-            main.wait_event(join)
-            self.cur ^= 1
-            self.ready = True
-        else:
-            self.ready = False
-        return out
 
 
 class VecPBNEnv:
@@ -378,35 +336,14 @@ class VecPBNEnv:
             raise ValueError("actions must hold num_envs*bins = %d bytes" % (self.num_envs * self.bins))
         return actions
 
-    def planes_buffer(self) -> torch.Tensor:
-        """A device buffer for the predictor-selection planes of one step (``pbn_predraw``)."""
-        n = int(self.lib.pbn_planes_words(self._h, self.num_envs))
-        if n < 0:
-            check(n)
-        return torch.empty((n,), dtype=torch.int32, device=self.device)
-
-    def predraw(self, planes: torch.Tensor, ahead: int = 0) -> None:
-        """Draw the selection planes of the step ``ahead`` steps after the next one into ``planes`` on the
-        current stream (``pbn_predraw``).  They depend only on the seed, the env ids and the step counter, so
-        this may run on another stream while earlier steps execute; pass the buffer to that step as
-        ``step(..., planes=planes)``.  Needs a step counter that is fixed while the planes are in flight:
-        the host-side counter or ``pdl=True`` sequences."""
-        if self.step_ctr_dev is not None and not self.pdl:
-            raise RuntimeError("predraw needs the host-side step counter or pdl=True (the device counter moves with every launch)")
-        a = self._args(None, None, False)
-        a.step_ctr += int(ahead)
-        check(self.lib.pbn_predraw(self._h, C.byref(a), planes.data_ptr(), self._stream()))
-
     def step(self, actions: Optional[torch.Tensor], final_state: Optional[torch.Tensor] = None,
-             stats: bool = True, planes: Optional[torch.Tensor] = None):
+             stats: bool = True):
         """One ``env.step`` for every instance.  ``actions``: uint8 ``[E, bins]`` with values in
         ``[0, N]`` (0 = no-op, k flips gene k-1), or ``None`` for an uncontrolled update
         (``env.step([])``).  Returns ``(state, reward, terminated, truncated)`` -- views of the
         env's own tensors, overwritten by the next call."""
         actions = self._check_actions(actions)
         a = self._args(actions, final_state, stats)
-        if planes is not None:
-            a.sel_planes = planes.data_ptr()
         check(self.lib.pbn_step(self._h, C.byref(a), self._stream()))
         if self.step_ctr_dev is None:
             self.step_ctr += 1
@@ -461,10 +398,6 @@ class VecPBNEnv:
                                    _ptr(self.stats_buf) if stats else None, self._stream()))
         self.step_ctr += n_steps
         return self.state
-
-    def pipeline(self) -> "StepPipeline":
-        """Two-stream stepping: the selection planes of step k+1 are drawn while step k runs."""
-        return StepPipeline(self)
 
     def advance_counter(self) -> None:
         """Close a sequence of ``pdl`` steps: add the number of steps taken since the last call to the

@@ -13,7 +13,7 @@ import bench  # noqa: E402
 from pbn_rl_b200 import VecPBNEnv  # noqa: E402
 
 
-def time_config(net, attrs, envs, kernel, p, auto_reset, stats, actions, batches=8, graph_steps=32, reps=20, pdl=False, split=False, resident=False, chain=False, streams=1):
+def time_config(net, attrs, envs, kernel, p, auto_reset, stats, actions, batches=8, graph_steps=32, reps=20, pdl=False, resident=False, chain=False, streams=1):
     dev = torch.device("cuda:0")
     es = []
     for b in range(batches):
@@ -27,24 +27,14 @@ def time_config(net, attrs, envs, kernel, p, auto_reset, stats, actions, batches
         es.append(e)
     g = torch.Generator(device=dev).manual_seed(99)
     pool = [torch.randint(0, net.n_genes + 1, (envs, 3), generator=g, device=dev, dtype=torch.uint8) for _ in range(8)]
-    pipes = [e.pipeline() for e in es] if split else None
-    bufs = [e.planes_buffer() for e in es] if split in ("main", "draw") else None
 
-    def step(i, n_total):
-        act = pool[i % 8] if actions else None
-        if split == "main":      # the step kernel alone, planes taken from a (stale) buffer
-            es[i % batches].step(act, stats=stats, planes=bufs[i % batches])
-        elif split == "draw":    # the predraw kernel alone
-            es[i % batches].predraw(bufs[i % batches])
-        elif split:
-            pipes[i % batches].step(act, last=(i >= n_total - batches), stats=stats)
-        else:
-            es[i % batches].step(act, stats=stats)
+    def step(i):
+        es[i % batches].step(pool[i % 8] if actions else None, stats=stats)
 
     s = torch.cuda.Stream()
     with torch.cuda.stream(s):
         for i in range(batches):
-            step(i, batches)
+            step(i)
         for e in es:
             e.advance_counter()
         s.synchronize()
@@ -58,7 +48,7 @@ def time_config(net, attrs, envs, kernel, p, auto_reset, stats, actions, batches
             with torch.cuda.graph(gr, stream=ls):
                 for i in range(graph_steps):
                     if (i % batches) % streams == k:
-                        step(i, graph_steps)
+                        step(i)
                 for b, e in enumerate(es):
                     if b % streams == k:
                         e.advance_counter()
@@ -95,7 +85,6 @@ def main():
     ap.add_argument("--quick", action="store_true")
     ap.add_argument("--big-attractor", type=int, default=0, help="add one attractor of this many random states (hash-set membership)")
     ap.add_argument("--pdl", action="store_true")
-    ap.add_argument("--split", default="", help="'pipe': pbn_predraw on a side stream + pbn_step with pre-drawn planes; 'main' / 'draw': either kernel alone")
     ap.add_argument("--graph-steps", type=int, default=32)
     ap.add_argument("--streams", type=int, default=1, help="env batches stepped concurrently on this many streams")
     ap.add_argument("--chain", action="store_true", help="tile-level chaining of resident steps (PBN_STEP_CHAIN)")
@@ -121,7 +110,7 @@ def main():
         rows = rows[:1]
     for kernel in args.kernels.split(","):
         for label, p, ar, st, act in rows:
-            us = time_config(net, attrs, args.envs, kernel, p, ar, st, act, pdl=args.pdl, split=args.split, graph_steps=args.graph_steps, resident=args.resident or args.chain, chain=args.chain, batches=args.batches)
+            us = time_config(net, attrs, args.envs, kernel, p, ar, st, act, pdl=args.pdl, graph_steps=args.graph_steps, resident=args.resident or args.chain, chain=args.chain, batches=args.batches)
             gbs = bench.BYTES_PER_STEP[W] * args.envs / us / 1e3
             print(("chain " if args.chain else "resident " if args.resident else "") + "%-8s %-30s %9.2f us/step  %8.3e steps/s  %7.1f GB/s" % (kernel, label, us, args.envs / us * 1e6, gbs), flush=True)
 

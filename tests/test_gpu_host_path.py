@@ -149,50 +149,6 @@ def test_step_host_compact_results(e):
     dut.close()
 
 
-@pytest.mark.parametrize("name,e", [("pbn28", 8192 + 300), ("pbn70", 2048), ("pbn7", 5)])
-@pytest.mark.parametrize("mode", ["host_counter", "pdl"])
-def test_predrawn_selection_planes_give_identical_steps(name, e, mode):
-    """Split launch (pbn_predraw on a side stream + pbn_step with sel_planes) == fused pbn_step, bit for bit."""
-    import torch
-    pdl = mode == "pdl"
-    ref = _mk(name, e, auto_reset=True, device_counter=pdl, pdl=pdl)
-    dut = _mk(name, e, auto_reset=True, device_counter=pdl, pdl=pdl)
-    assert dut.kernel == "sliced"
-    _seed_env(ref, name, e, 21)
-    _seed_env(dut, name, e, 21)
-    pipe = dut.pipeline()
-    rng = np.random.default_rng(22)
-    n = product_net(name).n_genes
-    for seq in range(2):
-        for step in range(5):
-            act = torch.from_numpy(rng.integers(0, n + 1, size=(e, 3), dtype=np.uint8)).cuda()
-            ref.step(act)
-            pipe.step(act, last=(step == 4))
-            torch.cuda.synchronize()
-            assert torch.equal(ref.state, dut.state), (seq, step)
-            assert torch.equal(ref.reward, dut.reward) and torch.equal(ref.terminated, dut.terminated)
-            assert torch.equal(ref.t, dut.t) and torch.equal(ref.target_id, dut.target_id)
-        ref.advance_counter()
-        dut.advance_counter()
-        pipe.flush()
-    assert ref.stats() == dut.stats()
-    ref.close()
-    dut.close()
-
-
-def test_predraw_refused_where_it_cannot_be_exact():
-    import torch
-    from pbn_rl_b200 import _cabi
-    env = _mk("pbn28", 1024, kernel="scalar")
-    with pytest.raises(_cabi.PbnError):
-        env.planes_buffer()
-    env.close()
-    env = _mk("pbn28", 1024, device_counter=True)           # device counter moves with every launch
-    with pytest.raises(RuntimeError):
-        env.predraw(env.planes_buffer())
-    env.close()
-
-
 @pytest.mark.parametrize("name,e", [("pbn28", 5000), ("pbn10", 4096), ("pbn7", 1025)])
 @pytest.mark.parametrize("chunks", [0, 3])
 def test_packed_host_form_matches_oracle(name, e, chunks):
