@@ -101,7 +101,7 @@ enum {
    * handle's pbn_advance_counter is launched fully serialised (it reads the counter that launch writes). */
   PBN_STEP_PDL = 2u,
   /* Do not increment *step_ctr_dev when the launch completes (several launches that belong to the same
-   * logical step, e.g. the chunks of pbn_step_host, share one counter value). */
+   * logical step, e.g. the lanes of pbn_step_host, share one counter value). */
   PBN_STEP_NO_COUNT = 4u,
   /* Tile-level chaining of plane-resident steps (args->resident; implies the PBN_STEP_PDL conventions: position in
    * the sequence as step_ctr, pbn_advance_counter at its end).  A launch at position >= 1 does not wait for the
@@ -227,7 +227,7 @@ typedef struct {
   float* reward;            /* HOST [E] out */
   uint8_t* terminated;      /* HOST [E] out */
   uint8_t* truncated;       /* HOST [E] out */
-  int32_t n_chunks;         /* pipeline depth; 0 = library default */
+  int32_t n_chunks;         /* number of lanes; 0 = library default */
   int32_t reserved;
   /* Compact forms of the same results (fewer PCIe bytes per env-step); page-locked memory only. */
   uint32_t* state32;        /* HOST [E] out: the state word narrowed to 32 bits; networks with N <= 32 only */
@@ -242,18 +242,19 @@ typedef struct {
 
 /* env.step(action) with HOST buffers, end to end: copies the actions to the device, steps all
  * n_envs instances (exactly as pbn_step with args->actions = io->actions_dev) and copies the
- * results back.  The batch is cut into n_chunks ranges of whole 1024-env tiles; the action
- * upload of chunk c+1, the step kernel of chunk c and the result download of chunk c-1 run
- * concurrently on two library-owned copy streams and the caller's stream (envs are independent,
- * so the result does not depend on n_chunks).  Unlike the device entry points this call BLOCKS
- * until the host outputs are complete (like the reference's env.step it returns values); it waits
- * on its own streams only, never on the whole device.
- * Lane form: when only `packed` is requested, with actions16, n_chunks <= 0 and n_envs >= 2^18, the batch is cut into
- * lanes (library streams) that each run upload -> unpack -> step -> export in order.  With args->step_ctr_dev set and
- * without PBN_STEP_PDL the lanes share one counter value and the call adds 1 to *step_ctr_dev when they have joined;
- * the arguments are then the same from call to call, and the library captures the whole step the second time it sees
- * an (args, io) pair and replays it as one CUDA graph launch afterwards (8 pairs are kept; keep the buffers alive
- * while the handle may still replay them). */
+ * results back.  The batch is cut into lanes, ranges of whole 1024-env tiles; each lane runs action
+ * upload -> step -> result download in order on its own library stream, and the lanes run
+ * concurrently, so one lane's upload overlaps another lane's download.  n_chunks sets the number of
+ * lanes (at most 16 and the number of tiles); 0 picks 1 below 2^18 envs, else 2, or 4 for the
+ * graph-replayed calls below.  Envs are independent, so the result does not depend on the number of
+ * lanes.  Unlike the device entry points this call BLOCKS until the host outputs are complete (like
+ * the reference's env.step it returns values); it waits on its own streams only, never on the whole
+ * device, and later work on `stream` is ordered after the step.
+ * The lanes share one counter value.  With args->step_ctr_dev set and neither PBN_STEP_PDL nor PBN_STEP_NO_COUNT,
+ * the call adds 1 to *step_ctr_dev itself once the lanes have joined, so its arguments can stay the same from call to
+ * call.  When only `packed` is requested, with actions16 and args->step_ctr_dev set, the library captures the whole
+ * step the second time it sees an (args, io) pair and replays it as one CUDA graph launch afterwards (8 pairs are kept;
+ * keep the buffers alive while the handle may still replay them). */
 int pbn_step_host(pbn_handle* h, const pbn_step_args* args, const pbn_host_io* io, void* stream);
 
 /* reward = table[n_flips + (bins + 1) * terminated], n_flips = number of distinct action values in 1..N of the env

@@ -5,6 +5,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <functional>
 #include <new>
 #include <map>
 #include <mutex>
@@ -132,12 +133,11 @@ struct pbn_handle {
   uint32_t jit_smem_opt_in[2][2] = {{48u * 1024u, 48u * 1024u}, {48u * 1024u, 48u * 1024u}};  // [injected][gen]
   uint64_t launches = 0;
   bool scalar_smem_opted = false;
-  // pbn_step_host: two copy streams + per-chunk events (created on first use)
-  static constexpr int kMaxChunks = 16;
-  cudaStream_t s_h2d = nullptr, s_d2h = nullptr;
-  static constexpr int kMaxLanes = 4;
-  cudaStream_t s_lane[kMaxLanes] = {};   // lanes 2.. of the packed path (lanes 0 and 1 are s_h2d and s_d2h)
-  // packed path with a device step counter: the whole step (uploads, unpack, step, export kernels of all lanes, counter
+  // pbn_step_host: one stream and one join event per lane (created on first use)
+  static constexpr int kMaxLanes = 16;
+  cudaStream_t s_lane[kMaxLanes] = {};
+  cudaEvent_t ev_k[kMaxLanes] = {};
+  // packed form with a device step counter: the whole step (uploads, unpack, step, export kernels of all lanes, counter
   // update) is captured once per distinct argument set and replayed as one CUDA graph launch afterwards
   struct HostGraph {
     pbn_step_args a;
@@ -150,8 +150,7 @@ struct pbn_handle {
   HostGraph host_graph[kHostGraphs];
   uint64_t host_graph_clock = 0;
   cudaStream_t s_origin = nullptr;
-  cudaEvent_t ev_done = nullptr, ev_fork = nullptr;
-  cudaEvent_t ev_entry = nullptr, ev_in[kMaxChunks] = {}, ev_k[kMaxChunks] = {};
+  cudaEvent_t ev_entry = nullptr, ev_fork = nullptr, ev_done = nullptr;
 };
 
 // Loaded specialisations are shared between the handles of a process: env batches of the same network (the bench
@@ -468,20 +467,16 @@ void pbn_destroy(pbn_handle* h) {
       release_module(h->jit_key[i]);
       release_module(h->jit_key_planes[i]);
     }
-    if (h->s_h2d) cudaStreamDestroy(h->s_h2d);
-    if (h->s_d2h) cudaStreamDestroy(h->s_d2h);
-    for (cudaStream_t ls : h->s_lane)
-      if (ls) cudaStreamDestroy(ls);
+    for (int c = 0; c < pbn_handle::kMaxLanes; ++c) {
+      if (h->s_lane[c]) cudaStreamDestroy(h->s_lane[c]);
+      if (h->ev_k[c]) cudaEventDestroy(h->ev_k[c]);
+    }
     for (auto& g : h->host_graph)
       if (g.exec) cudaGraphExecDestroy(g.exec);
     if (h->s_origin) cudaStreamDestroy(h->s_origin);
     if (h->ev_done) cudaEventDestroy(h->ev_done);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
     if (h->ev_entry) cudaEventDestroy(h->ev_entry);
-    for (int i = 0; i < pbn_handle::kMaxChunks; ++i) {
-      if (h->ev_in[i]) cudaEventDestroy(h->ev_in[i]);
-      if (h->ev_k[i]) cudaEventDestroy(h->ev_k[i]);
-    }
   }
   delete h;
 }
@@ -903,6 +898,81 @@ static pbn_step_args env_range(const pbn_handle* h, const pbn_step_args* a, cons
   return s;
 }
 
+// The device alias of a page-locked host buffer; null for a null or pageable one (the failed query's error is cleared).
+static void* mapped(void* host) {
+  void* dev = nullptr;
+  if (host && (cudaHostGetDevicePointer(&dev, host, 0) != cudaSuccess || !dev)) {
+    cudaGetLastError();
+    dev = nullptr;
+  }
+  return dev;
+}
+
+// Envs [e0, e0 + n) of the export of a whole batch of W-word states.
+static ExportArgs export_range(ExportArgs x, int W, int64_t e0, int64_t n) {
+  const int64_t row[4] = {8 * W, 4, 1, 1};   // bytes per env of the state words, reward, terminated, truncated
+  for (int k = 0; k < 4; ++k) {
+    if (x.dst[k]) x.src[k] += e0 * row[k], x.dst[k] += e0 * row[k];
+    x.bytes[k] = (unsigned long long)(n * row[k]);
+  }
+  x.state64 += e0 * W;
+  if (x.state32) x.state32 += e0;
+  if (x.term) x.term += e0;
+  if (x.trunc) x.trunc += e0;
+  if (x.done) x.done += e0;
+  if (x.packed) x.packed += e0;
+  x.n_envs = n;
+  return x;
+}
+
+// Runs `enqueue` (one step's work, forked from and joined into h->s_origin) through the handle's graph cache, keyed by
+// the (args, io) pair: the first call with a pair runs eagerly, the second (every kernel it needs is loaded by then)
+// captures the work, and from the third on it is replayed as one graph launch.  The least recently used slot is evicted.
+static int run_host_graph(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, const std::function<int()>& enqueue) {
+  pbn_handle::HostGraph* slot = nullptr;
+  pbn_handle::HostGraph* lru = &h->host_graph[0];
+  for (auto& g : h->host_graph) {
+    if (g.seen && memcmp(&g.a, a, sizeof(*a)) == 0 && memcmp(&g.io, io, sizeof(*io)) == 0) slot = &g;
+    if (g.last_use < lru->last_use) lru = &g;
+  }
+  if (!slot) {
+    slot = lru;
+    if (slot->exec) cudaGraphExecDestroy(slot->exec);
+    *slot = pbn_handle::HostGraph{};
+    memcpy(&slot->a, a, sizeof(*a));
+    memcpy(&slot->io, io, sizeof(*io));
+  }
+  slot->last_use = ++h->host_graph_clock;
+  if (slot->exec) {
+    PBN_CUDA(cudaGraphLaunch(slot->exec, h->s_origin));
+    h->launches += slot->launches;
+  } else if (slot->seen >= 1) {
+    const uint64_t launches_before = h->launches;
+    cudaGraph_t graph = nullptr;
+    PBN_CUDA(cudaStreamBeginCapture(h->s_origin, cudaStreamCaptureModeThreadLocal));
+    const int rc = enqueue();
+    const cudaError_t ce = cudaStreamEndCapture(h->s_origin, &graph);
+    if (rc != PBN_OK) {
+      if (graph) cudaGraphDestroy(graph);
+      return rc;
+    }
+    if (ce != cudaSuccess) return fail(PBN_ERR_CUDA, "pbn_step_host: graph capture failed: %s", cudaGetErrorString(ce));
+    const cudaError_t ie = cudaGraphInstantiate(&slot->exec, graph, 0);
+    cudaGraphDestroy(graph);
+    if (ie != cudaSuccess) {
+      slot->exec = nullptr;
+      return fail(PBN_ERR_CUDA, "pbn_step_host: graph instantiation failed: %s", cudaGetErrorString(ie));
+    }
+    slot->launches = h->launches - launches_before;
+    PBN_CUDA(cudaGraphLaunch(slot->exec, h->s_origin));
+  } else {
+    const int rc = enqueue();
+    if (rc != PBN_OK) return rc;
+  }
+  slot->seen += 1;
+  return PBN_OK;
+}
+
 int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, void* stream_) {
   if (!h || !a || !io) return fail(PBN_ERR_INVALID, "null argument");
   if (a->n_envs < 0) return fail(PBN_ERR_INVALID, "n_envs=%lld", (long long)a->n_envs);
@@ -916,227 +986,112 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
   if (a->sel || a->pert_mask) return fail(PBN_ERR_INVALID, "pbn_step_host: sel/pert_mask must be null");
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  if (!h->s_h2d) {
-    PBN_CUDA(cudaStreamCreateWithFlags(&h->s_h2d, cudaStreamNonBlocking));
-    PBN_CUDA(cudaStreamCreateWithFlags(&h->s_d2h, cudaStreamNonBlocking));
-    PBN_CUDA(cudaEventCreateWithFlags(&h->ev_entry, cudaEventDisableTiming));
-    for (int i = 0; i < pbn_handle::kMaxChunks; ++i) {
-      PBN_CUDA(cudaEventCreateWithFlags(&h->ev_in[i], cudaEventDisableTiming));
-      PBN_CUDA(cudaEventCreateWithFlags(&h->ev_k[i], cudaEventDisableTiming));
-    }
-  }
-  // Outputs in page-locked host memory are written by an export kernel straight over PCIe (one launch
-  // per chunk); pageable outputs go through the copy engine (one cudaMemcpyAsync per array and chunk).
-  uint8_t* zc[4] = {nullptr, nullptr, nullptr, nullptr};
-  bool zero_copy = true;
+  // Results in page-locked host memory are written by the export kernel straight over PCIe, through the buffers' device
+  // aliases (one launch per lane); pageable full-width results go through the copy engine (one cudaMemcpyAsync per
+  // array and lane).  (Measured: letting the step kernel write the packed word straight into the mapped host buffer --
+  // 1024 CTAs posting 16-byte writes -- is slower over PCIe, 0.200 ms per 2^20 envs, than the 16-CTA export kernel,
+  // 0.176 ms.)
+  const int W = h->W, bins = h->net.bins;
+  ExportArgs all{};
+  bool zero_copy = true;   // every requested full-width output is page-locked
   {
-    void* hp[4] = {io->state, io->reward, io->terminated, io->truncated};
-    for (int k = 0; k < 4 && zero_copy; ++k) {
-      if (!hp[k]) continue;
-      void* dp = nullptr;
-      if (cudaHostGetDevicePointer(&dp, hp[k], 0) != cudaSuccess || !dp) {
-        cudaGetLastError();  // not page-locked: clear the sticky-less error and fall back to the copy engine
-        zero_copy = false;
-      }
-      zc[k] = static_cast<uint8_t*>(dp);
+    void* const host[4] = {io->state, io->reward, io->terminated, io->truncated};
+    const void* const dev[4] = {a->state, a->reward, a->terminated, a->truncated};
+    for (int k = 0; k < 4; ++k) {
+      all.src[k] = static_cast<const uint8_t*>(dev[k]);
+      all.dst[k] = static_cast<uint8_t*>(mapped(host[k]));
+      if (host[k] && !all.dst[k]) zero_copy = false;
     }
   }
-  uint32_t* zc_packed = nullptr;
+  all.state64 = a->state;
+  all.term = a->terminated;
+  all.trunc = a->truncated;
   if (io->packed) {
-    void* dp = nullptr;
     if (h->net.n_genes > 30 || !a->terminated || !a->truncated) return fail(PBN_ERR_INVALID, "pbn_step_host: packed needs N <= 30 and the terminated / truncated device arrays");
-    if (!zero_copy || cudaHostGetDevicePointer(&dp, io->packed, 0) != cudaSuccess || !(zc_packed = static_cast<uint32_t*>(dp))) {
-      cudaGetLastError();
+    if (!zero_copy || !(all.packed = static_cast<uint32_t*>(mapped(io->packed))))
       return fail(PBN_ERR_INVALID, "pbn_step_host: packed needs page-locked host memory for every output");
-    }
   }
-  uint32_t* zc_state32 = nullptr;
-  uint8_t* zc_done = nullptr;
   if (io->state32 || io->done) {
     if (io->state32 && h->net.n_genes > 32) return fail(PBN_ERR_INVALID, "pbn_step_host: state32 needs a network with N <= 32 (N=%d)", h->net.n_genes);
     if (io->done && (!a->terminated || !a->truncated)) return fail(PBN_ERR_INVALID, "pbn_step_host: done needs the terminated and truncated device arrays");
-    void* dp = nullptr;
-    if (!zero_copy || (io->state32 && (cudaHostGetDevicePointer(&dp, io->state32, 0) != cudaSuccess || !(zc_state32 = static_cast<uint32_t*>(dp)))) ||
-        (io->done && (cudaHostGetDevicePointer(&dp, io->done, 0) != cudaSuccess || !(zc_done = static_cast<uint8_t*>(dp))))) {
-      cudaGetLastError();
+    all.state32 = static_cast<uint32_t*>(mapped(io->state32));
+    all.done = static_cast<uint8_t*>(mapped(io->done));
+    if (!zero_copy || (io->state32 && !all.state32) || (io->done && !all.done))
       return fail(PBN_ERR_INVALID, "pbn_step_host: state32/done need page-locked host memory for every output");
-    }
   }
-  // only the packed word is wanted.  (Measured: letting the step kernel write it straight into the mapped host buffer
-  // -- 1024 CTAs posting 16-byte writes -- is slower over PCIe, 0.200 ms per 2^20 envs, than the 16-CTA export kernel,
-  // 0.176 ms.)
-  const bool packed_only = zc_packed && !io->state && !io->reward && !io->terminated && !io->truncated && !io->state32 && !io->done;
+  // Graph replay needs arguments that are the same from call to call -- a device step counter keeps the host part of
+  // the counter constant -- and only mapped outputs: a pageable copy cannot be captured.
+  const bool graphable = io->packed && io->actions16 && a->step_ctr_dev && !io->state && !io->reward && !io->terminated &&
+                         !io->truncated && !io->state32 && !io->done;
+  // Lanes: slices of whole tiles, each running upload -> step -> results in order on its own library stream, so nothing
+  // inside a lane needs an event and PCIe (full duplex) carries one lane's upload under another lane's results.  Envs are
+  // independent: the results do not depend on the number of lanes.  Measured on B200 / PCIe Gen5, packed form, 2^20
+  // envs: replayed graph 0.166 / 0.158 / 0.161 / 0.148 / 0.158 ms with 1 / 2 / 3 / 4 / 6 lanes; stream launches
+  // 0.175 / 0.169 / 0.167 / 0.173 / 0.189 ms.
   const int64_t E = a->n_envs, tiles = (E + 1023) / 1024;
-  // Lane form of the packed path: each lane (a slice of the batch) runs copy -> unpack -> step -> export in order on its
-  // own library stream, so nothing inside a lane needs an event, and PCIe (full duplex) carries one lane's upload under
-  // another lane's results.  The lanes' step kernels run concurrently, so they cannot each advance a device step
-  // counter: they share one counter value (see own_count below).
-  if (packed_only && io->actions16 && io->n_chunks <= 0 && E >= (1 << 18)) {
-    // graph replay needs call-invariant arguments: a device counter (the host part of the step counter constant)
-    const bool graphable = a->step_ctr_dev != nullptr;
-    // measured on B200 / PCIe Gen5, 2^20 envs: replayed graph 0.166 / 0.158 / 0.161 / 0.148 / 0.158 ms with
-    // 1 / 2 / 3 / 4 / 6 lanes; stream launches 0.175 / 0.169 / 0.167 / 0.173 / 0.189 ms
-    const int lanes = graphable ? 4 : 2;
-    const int64_t per = ((tiles + lanes - 1) / lanes) * 1024;   // envs per lane: whole tiles
-    // a device step counter that the steps themselves advance (no PDL sequence): the lanes share one counter value
-    // (PBN_STEP_NO_COUNT) and one small launch adds 1 after they have joined
-    const bool own_count = a->step_ctr_dev != nullptr && !(a->flags & PBN_STEP_PDL) && !(a->flags & PBN_STEP_NO_COUNT);
-    if (!h->s_origin) {
-      PBN_CUDA(cudaStreamCreateWithFlags(&h->s_origin, cudaStreamNonBlocking));
-      PBN_CUDA(cudaEventCreateWithFlags(&h->ev_done, cudaEventDisableTiming));
-      PBN_CUDA(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
-    }
-    for (int c = 2; c < lanes; ++c)
-      if (!h->s_lane[c]) PBN_CUDA(cudaStreamCreateWithFlags(&h->s_lane[c], cudaStreamNonBlocking));
-    // everything of one step on the library's streams, forked from and joined into s_origin
-    auto enqueue = [&]() -> int {
-      PBN_CUDA(cudaEventRecord(h->ev_fork, h->s_origin));
-      for (int c = 0; c < lanes; ++c) {
-        const int64_t e0 = c * per, n = (E - e0 < per) ? E - e0 : per;
-        if (n <= 0) continue;
-        cudaStream_t S = c == 0 ? h->s_h2d : (c == 1 ? h->s_d2h : h->s_lane[c]);
-        PBN_CUDA(cudaStreamWaitEvent(S, h->ev_fork, 0));
+  int64_t lanes = io->n_chunks > 0 ? io->n_chunks : (E < (1 << 18) ? 1 : (graphable ? 4 : 2));
+  lanes = std::min<int64_t>(std::min<int64_t>(lanes, pbn_handle::kMaxLanes), tiles);
+  const int64_t per = ((tiles + lanes - 1) / lanes) * 1024;
+  // The lanes' step kernels run concurrently, so they cannot each advance a device step counter: they share one counter
+  // value (PBN_STEP_NO_COUNT), and a counter the steps would advance themselves gets one launch that adds 1 after the join.
+  const bool own_count = a->step_ctr_dev && !(a->flags & (PBN_STEP_PDL | PBN_STEP_NO_COUNT));
+  if (!h->s_origin) PBN_CUDA(cudaStreamCreateWithFlags(&h->s_origin, cudaStreamNonBlocking));
+  for (cudaEvent_t* ev : {&h->ev_entry, &h->ev_fork, &h->ev_done})
+    if (!*ev) PBN_CUDA(cudaEventCreateWithFlags(ev, cudaEventDisableTiming));
+  for (int c = 0; c < lanes; ++c) {
+    if (!h->s_lane[c]) PBN_CUDA(cudaStreamCreateWithFlags(&h->s_lane[c], cudaStreamNonBlocking));
+    if (!h->ev_k[c]) PBN_CUDA(cudaEventCreateWithFlags(&h->ev_k[c], cudaEventDisableTiming));
+  }
+  const uint8_t* actions = (io->actions || io->actions16) ? io->actions_dev : nullptr;
+  auto enqueue = [&]() -> int {
+    PBN_CUDA(cudaEventRecord(h->ev_fork, h->s_origin));
+    for (int c = 0; c < lanes; ++c) {
+      const int64_t e0 = c * per, n = std::min(per, E - e0);
+      if (n <= 0) break;
+      cudaStream_t S = h->s_lane[c];
+      PBN_CUDA(cudaStreamWaitEvent(S, h->ev_fork, 0));
+      if (io->actions) {
+        PBN_CUDA(cudaMemcpyAsync(io->actions_dev + e0 * bins, io->actions + e0 * bins, (size_t)n * bins, cudaMemcpyHostToDevice, S));
+      } else if (io->actions16) {
         PBN_CUDA(cudaMemcpyAsync(io->actions16_dev + e0, io->actions16 + e0, (size_t)n * 2, cudaMemcpyHostToDevice, S));
-        unpack_actions16_kernel<<<grid_for(h, n / 4 + 1, 256, 4), 256, 0, S>>>(io->actions16_dev + e0, io->actions_dev + e0 * h->net.bins, n);
-        PBN_CUDA(cudaGetLastError());
-        pbn_step_args s = env_range(h, a, io->actions_dev, e0, n);
-        s.flags = (a->flags & ~PBN_STEP_PDL) | PBN_STEP_NO_COUNT;
-        const int rc = step_common(h, &s, S, false);
-        if (rc != PBN_OK) return rc;
-        ExportArgs x{};
-        x.state64 = a->state + e0;
-        x.term = a->terminated + e0;
-        x.trunc = a->truncated + e0;
-        x.packed = zc_packed + e0;
-        x.n_envs = n;
-        export_kernel<<<16, 256, 0, S>>>(x);
-        PBN_CUDA(cudaGetLastError());
-        h->launches += 2;   // (+ the step kernel, counted by step_common)
-        PBN_CUDA(cudaEventRecord(h->ev_k[c], S));
-        PBN_CUDA(cudaStreamWaitEvent(h->s_origin, h->ev_k[c], 0));
-      }
-      if (own_count) {
-        advance_counter_kernel<<<1, 1, 0, h->s_origin>>>(a->step_ctr_dev, 1ull);
+        unpack_actions16_kernel<<<grid_for(h, n / 4 + 1, 256, 4), 256, 0, S>>>(io->actions16_dev + e0, io->actions_dev + e0 * bins, n);
         PBN_CUDA(cudaGetLastError());
         h->launches += 1;
       }
-      return PBN_OK;
-    };
-    PBN_CUDA(cudaEventRecord(h->ev_entry, stream));
-    PBN_CUDA(cudaStreamWaitEvent(h->s_origin, h->ev_entry, 0));
-    pbn_handle::HostGraph* slot = nullptr;
-    if (graphable) {
-      pbn_handle::HostGraph* lru = &h->host_graph[0];
-      for (auto& g : h->host_graph) {
-        if (g.seen && memcmp(&g.a, a, sizeof(*a)) == 0 && memcmp(&g.io, io, sizeof(*io)) == 0) slot = &g;
-        if (g.last_use < lru->last_use) lru = &g;
-      }
-      if (!slot) {
-        slot = lru;
-        if (slot->exec) cudaGraphExecDestroy(slot->exec);
-        *slot = pbn_handle::HostGraph{};
-        memcpy(&slot->a, a, sizeof(*a));
-        memcpy(&slot->io, io, sizeof(*io));
-      }
-      slot->last_use = ++h->host_graph_clock;
-    }
-    const uint64_t launches_before = h->launches;
-    if (slot && slot->exec) {
-      PBN_CUDA(cudaGraphLaunch(slot->exec, h->s_origin));
-      h->launches += slot->launches;
-    } else if (slot && slot->seen >= 1) {
-      // second call with these arguments (the first ran eagerly, so every kernel it needs is loaded): capture
-      cudaGraph_t graph = nullptr;
-      PBN_CUDA(cudaStreamBeginCapture(h->s_origin, cudaStreamCaptureModeThreadLocal));
-      const int rc = enqueue();
-      const cudaError_t ce = cudaStreamEndCapture(h->s_origin, &graph);
-      if (rc != PBN_OK) {
-        if (graph) cudaGraphDestroy(graph);
-        return rc;
-      }
-      if (ce != cudaSuccess) return fail(PBN_ERR_CUDA, "pbn_step_host: graph capture failed: %s", cudaGetErrorString(ce));
-      const cudaError_t ie = cudaGraphInstantiate(&slot->exec, graph, 0);
-      cudaGraphDestroy(graph);
-      if (ie != cudaSuccess) {
-        slot->exec = nullptr;
-        return fail(PBN_ERR_CUDA, "pbn_step_host: graph instantiation failed: %s", cudaGetErrorString(ie));
-      }
-      slot->launches = h->launches - launches_before;
-      PBN_CUDA(cudaGraphLaunch(slot->exec, h->s_origin));
-    } else {
-      const int rc = enqueue();
+      // PDL only orders kernels, which the lane's stream already does
+      pbn_step_args s = env_range(h, a, actions, e0, n);
+      s.flags = (a->flags & ~PBN_STEP_PDL) | PBN_STEP_NO_COUNT;
+      const int rc = step_common(h, &s, S, false);
       if (rc != PBN_OK) return rc;
+      if (zero_copy) {
+        export_kernel<<<16, 256, 0, S>>>(export_range(all, W, e0, n));
+        PBN_CUDA(cudaGetLastError());
+        h->launches += 1;
+      } else {
+        if (io->state) PBN_CUDA(cudaMemcpyAsync(io->state + e0 * W, a->state + e0 * W, (size_t)n * W * 8, cudaMemcpyDeviceToHost, S));
+        if (io->reward) PBN_CUDA(cudaMemcpyAsync(io->reward + e0, a->reward + e0, (size_t)n * 4, cudaMemcpyDeviceToHost, S));
+        if (io->terminated) PBN_CUDA(cudaMemcpyAsync(io->terminated + e0, a->terminated + e0, (size_t)n, cudaMemcpyDeviceToHost, S));
+        if (io->truncated) PBN_CUDA(cudaMemcpyAsync(io->truncated + e0, a->truncated + e0, (size_t)n, cudaMemcpyDeviceToHost, S));
+      }
+      PBN_CUDA(cudaEventRecord(h->ev_k[c], S));
+      PBN_CUDA(cudaStreamWaitEvent(h->s_origin, h->ev_k[c], 0));
     }
-    if (slot) slot->seen += 1;
-    g_last_advance = own_count ? h : nullptr;
-    PBN_CUDA(cudaEventRecord(h->ev_done, h->s_origin));
-    PBN_CUDA(cudaStreamWaitEvent(stream, h->ev_done, 0));   // later work on the caller's stream sees the step
-    PBN_CUDA(cudaEventSynchronize(h->ev_done));
-    return PBN_OK;
-  }
-  int64_t nc = io->n_chunks > 0 ? io->n_chunks : (E >= (1 << 18) ? 2 : 1);  // measured best on B200 / PCIe Gen5 (scripts/host_path_probe.py)
-  if (nc > pbn_handle::kMaxChunks) nc = pbn_handle::kMaxChunks;
-  if (nc > tiles) nc = tiles;
-  const int64_t chunk = ((tiles + nc - 1) / nc) * 1024;  // envs per chunk: whole tiles
-  const int W = h->W, bins = h->net.bins;
-  // the staging buffer / device outputs may still be in use by earlier work on the caller's stream
-  PBN_CUDA(cudaEventRecord(h->ev_entry, stream));
-  PBN_CUDA(cudaStreamWaitEvent(h->s_h2d, h->ev_entry, 0));
-  int c = 0;
-  for (int64_t e0 = 0; e0 < E; e0 += chunk, ++c) {
-    const int64_t n = (E - e0 < chunk) ? (E - e0) : chunk;
-    const bool last = e0 + chunk >= E;
-    if (io->actions) {
-      PBN_CUDA(cudaMemcpyAsync(io->actions_dev + e0 * bins, io->actions + e0 * bins, (size_t)n * bins, cudaMemcpyHostToDevice, h->s_h2d));
-      PBN_CUDA(cudaEventRecord(h->ev_in[c], h->s_h2d));
-      PBN_CUDA(cudaStreamWaitEvent(stream, h->ev_in[c], 0));
-    } else if (io->actions16) {
-      PBN_CUDA(cudaMemcpyAsync(io->actions16_dev + e0, io->actions16 + e0, (size_t)n * 2, cudaMemcpyHostToDevice, h->s_h2d));
-      unpack_actions16_kernel<<<grid_for(h, n / 4 + 1, 256, 4), 256, 0, h->s_h2d>>>(io->actions16_dev + e0, io->actions_dev + e0 * bins, n);
+    if (own_count) {
+      advance_counter_kernel<<<1, 1, 0, h->s_origin>>>(a->step_ctr_dev, 1ull);
       PBN_CUDA(cudaGetLastError());
       h->launches += 1;
-      PBN_CUDA(cudaEventRecord(h->ev_in[c], h->s_h2d));
-      PBN_CUDA(cudaStreamWaitEvent(stream, h->ev_in[c], 0));
     }
-    pbn_step_args s = env_range(h, a, (io->actions || io->actions16) ? io->actions_dev : nullptr, e0, n);
-    // the chunks are one logical step: one counter value; PDL only orders kernels, which the event waits already do
-    s.flags = (a->flags & ~PBN_STEP_PDL) | ((last && !(a->flags & PBN_STEP_PDL)) ? 0u : PBN_STEP_NO_COUNT);
-    const int rc = step_common(h, &s, stream_, false);
-    if (rc != PBN_OK) return rc;
-    PBN_CUDA(cudaEventRecord(h->ev_k[c], stream));
-    PBN_CUDA(cudaStreamWaitEvent(h->s_d2h, h->ev_k[c], 0));
-    if (zero_copy) {
-      ExportArgs x{};
-      x.src[0] = reinterpret_cast<const uint8_t*>(a->state + e0 * W);
-      x.dst[0] = zc[0] ? zc[0] + (size_t)e0 * W * 8 : nullptr;
-      x.bytes[0] = (unsigned long long)n * W * 8;
-      x.src[1] = reinterpret_cast<const uint8_t*>(a->reward + e0);
-      x.dst[1] = zc[1] ? zc[1] + (size_t)e0 * 4 : nullptr;
-      x.bytes[1] = (unsigned long long)n * 4;
-      x.src[2] = a->terminated + e0;
-      x.dst[2] = zc[2] ? zc[2] + e0 : nullptr;
-      x.bytes[2] = (unsigned long long)n;
-      x.src[3] = a->truncated + e0;
-      x.dst[3] = zc[3] ? zc[3] + e0 : nullptr;
-      x.bytes[3] = (unsigned long long)n;
-      x.state64 = a->state + e0;
-      x.state32 = zc_state32 ? zc_state32 + e0 : nullptr;
-      x.term = a->terminated ? a->terminated + e0 : nullptr;
-      x.trunc = a->truncated ? a->truncated + e0 : nullptr;
-      x.done = zc_done ? zc_done + e0 : nullptr;
-      x.packed = zc_packed ? zc_packed + e0 : nullptr;
-      x.n_envs = n;
-      export_kernel<<<16, 256, 0, h->s_d2h>>>(x);
-      PBN_CUDA(cudaGetLastError());
-      h->launches += 1, g_last_advance = nullptr;
-      continue;
-    }
-    if (io->state) PBN_CUDA(cudaMemcpyAsync(io->state + e0 * W, a->state + e0 * W, (size_t)n * W * 8, cudaMemcpyDeviceToHost, h->s_d2h));
-    if (io->reward) PBN_CUDA(cudaMemcpyAsync(io->reward + e0, a->reward + e0, (size_t)n * 4, cudaMemcpyDeviceToHost, h->s_d2h));
-    if (io->terminated) PBN_CUDA(cudaMemcpyAsync(io->terminated + e0, a->terminated + e0, (size_t)n, cudaMemcpyDeviceToHost, h->s_d2h));
-    if (io->truncated) PBN_CUDA(cudaMemcpyAsync(io->truncated + e0, a->truncated + e0, (size_t)n, cudaMemcpyDeviceToHost, h->s_d2h));
-  }
-  PBN_CUDA(cudaStreamSynchronize(h->s_d2h));
+    return PBN_OK;
+  };
+  // the staging buffers and device arrays may still be in use by earlier work on the caller's stream
+  PBN_CUDA(cudaEventRecord(h->ev_entry, stream));
+  PBN_CUDA(cudaStreamWaitEvent(h->s_origin, h->ev_entry, 0));
+  const int rc = graphable ? run_host_graph(h, a, io, enqueue) : enqueue();
+  if (rc != PBN_OK) return rc;
+  g_last_advance = own_count ? h : nullptr;
+  PBN_CUDA(cudaEventRecord(h->ev_done, h->s_origin));
+  PBN_CUDA(cudaStreamWaitEvent(stream, h->ev_done, 0));   // later work on the caller's stream sees the step
+  PBN_CUDA(cudaEventSynchronize(h->ev_done));
   return PBN_OK;
 }
 int pbn_step_injected(pbn_handle* h, const pbn_step_args* a, void* stream) { return step_common(h, a, stream, true); }

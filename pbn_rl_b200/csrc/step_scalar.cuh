@@ -287,10 +287,10 @@ __global__ void __launch_bounds__(256) reset_kernel(const __grid_constant__ NetP
 
 __global__ void advance_counter_kernel(uint64_t* ctr, uint64_t n) { *ctr += n; }
 
-// pbn_step_host: stream one chunk's results from the device arrays into page-locked host memory that
+// pbn_step_host: stream one lane's results from the device arrays into page-locked host memory that
 // is mapped into the device address space (zero-copy posted writes over PCIe, 16 B per thread).
 // A few CTAs saturate the link (scripts/micro/zerocopy_rate.cu); the grid is kept small so that the
-// step kernel of the next chunk finds free SMs.
+// step kernels of the other lanes find free SMs.
 struct ExportArgs {
   const uint8_t* src[4];
   uint8_t* dst[4];

@@ -457,8 +457,8 @@ class VecPBNEnv:
         ``packed = state | terminated << 30 | truncated << 31`` -- the reward follows from the caller's own actions and
         the terminated bit through :meth:`reward_table`.  ``actions16`` (instead of ``actions_host``): a pinned int16
         ``[E]`` tensor of packed actions (:meth:`pack_actions16`), 2 instead of 3 bytes per env.  The batch is
-        processed in ``chunks`` ranges so that upload, kernel and download overlap (0 = library default); blocks
-        until the results are there."""
+        cut into ``chunks`` lanes, each of which uploads, steps and downloads its slice on its own stream, so that the
+        lanes' transfers and kernels overlap (0 = library default); blocks until the results are there."""
         hb = self._host_buffers()
         key = "io_packed" if compact == "packed" else ("io_compact" if compact else "io")
         if key not in hb:
@@ -514,24 +514,15 @@ class VecPBNEnv:
         a = hb.get("args")
         if a is None:
             a = hb["args"] = self._args(None, None, True, rows=True)
-        if compact == "packed" and actions16 is not None and self.step_ctr_dev is not None and int(chunks) <= 0 \
-                and self.num_envs >= (1 << 18):
-            # lane form with a device counter: the library advances the counter itself and, the arguments being the
-            # same from call to call, replays the whole step as one captured graph
-            if self._pos:
-                self.advance_counter()
+            # with a device counter the library advances it after the step, so the arguments stay the same from call
+            # to call (the packed form replays them as one captured graph)
             a.flags &= ~_cabi.STEP_PDL
-            a.step_ctr = self.step_ctr
-            check(self.lib.pbn_step_host(self._h, C.byref(a), C.byref(io), self._stream()))
-            if self.pdl:
-                a.flags |= _cabi.STEP_PDL
-        else:
-            a.step_ctr = self._pos if self.pdl else self.step_ctr
-            check(self.lib.pbn_step_host(self._h, C.byref(a), C.byref(io), self._stream()))
-            if self.step_ctr_dev is None:
-                self.step_ctr += 1
-            elif self.pdl:
-                self._pos += 1
+        if self._pos:
+            self.advance_counter()   # close the PDL sequence: the device counter then holds the whole count
+        a.step_ctr = self.step_ctr
+        check(self.lib.pbn_step_host(self._h, C.byref(a), C.byref(io), self._stream()))
+        if self.step_ctr_dev is None:
+            self.step_ctr += 1
         return hb["views_packed" if compact == "packed" else ("views_compact" if compact else "views")]
 
     @property

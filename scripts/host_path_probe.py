@@ -1,4 +1,5 @@
-"""PCIe copy rates and pbn_step_host timing for several chunk counts (tuning aid, not a bench)."""
+"""PCIe copy rates and pbn_step_host timing for several lane counts, every result form (tuning aid, not a bench).
+Lane count 0 is the library default."""
 import sys, time
 from pathlib import Path
 sys.path.insert(0, str(Path(__file__).resolve().parent.parent))
@@ -31,4 +32,4 @@ for compact in (False, True, "packed"):
             t = timeit(lambda: env.step_host(None, chunks=ch, compact="packed", actions16=a16))
         else:
             t = timeit(lambda: env.step_host(pa, chunks=ch, compact=compact))
-        print("step_host compact=%s chunks=%2d: %.3f ms  %.3e env-steps/s" % (compact, ch, t * 1e3, E / t))
+        print("step_host compact=%s lanes=%2d: %.3f ms  %.3e env-steps/s" % (compact, ch, t * 1e3, E / t))

@@ -1,5 +1,6 @@
-"""GPU: pbn_step_host (host buffers, chunk-pipelined upload / kernel / download) against pbn_step on the
-same inputs -- the result must not depend on the number of chunks, the counter mode or the kernel."""
+"""GPU: pbn_step_host (host buffers; the batch cut into lanes that each run upload / kernel / download on their own
+stream) against pbn_step on the same inputs -- the result must not depend on the number of lanes, the result form, the
+counter mode or the kernel."""
 import numpy as np
 import pytest
 
@@ -61,7 +62,7 @@ def test_step_host_equals_step(name, e, kernel, chunks):
 
 @pytest.mark.parametrize("mode", ["device_counter", "pdl"])
 def test_step_host_counter_modes(mode):
-    """Chunk launches of one logical step share one Philox step counter, whichever side keeps it."""
+    """The lanes of one logical step share one Philox step counter, whichever side keeps it."""
     import torch
     e, name = 6 * 1024 + 17, "pbn28"
     ref = _mk(name, e)                                    # host-side counter
@@ -225,14 +226,18 @@ def test_step_host_matches_oracle(name, e):
     env.close()
 
 
-@pytest.mark.parametrize("mode", ["host_counter", "device_counter", "pdl"])
-def test_packed_lane_form_and_graph_replay_equal_step(mode):
-    """Large batches take the lane form of the packed path (each lane: upload -> unpack -> step -> export on its own
-    stream); with a device step counter the whole step is captured on the second call with the same arguments and
-    replayed as one graph launch from the third on.  Seven steps alternating two pinned action buffers must equal
-    pbn_step on a twin env, step for step (eager, capture and replay calls all occur)."""
+_MODES = ["host_counter", "device_counter", "pdl"]
+
+
+@pytest.mark.parametrize("mode,e", [pytest.param(m, (1 << 18) + 1024 + 7, id=m) for m in _MODES] +
+                         [pytest.param(m, 5000, id=m + "-5000") for m in _MODES])
+def test_packed_lane_form_and_graph_replay_equal_step(mode, e):
+    """The packed form runs as lanes (each lane: upload -> unpack -> step -> export on its own stream); with a device
+    step counter the whole step is captured on the second call with the same arguments and replayed as one graph launch
+    from the third on.  Seven steps alternating two pinned action buffers must equal pbn_step on a twin env, step for
+    step (eager, capture and replay calls all occur)."""
     import torch
-    name, e = "pbn28", (1 << 18) + 1024 + 7
+    name = "pbn28"
     kw = dict(auto_reset=True)
     if mode != "host_counter":
         kw.update(device_counter=True, pdl=(mode == "pdl"))
@@ -260,9 +265,57 @@ def test_packed_lane_form_and_graph_replay_equal_step(mode):
         assert np.array_equal((packed >> np.uint32(30)) & np.uint32(1), ref.terminated.cpu().numpy().astype(np.uint32))
         assert np.array_equal(packed >> np.uint32(31), ref.truncated.cpu().numpy().astype(np.uint32))
     per_step = (dut.launches - launches0) / 7
-    # host counter: 2 lanes x (unpack, step, export); device counter: 4 lanes + the counter update
-    assert per_step == (13 if mode != "host_counter" else 6)
+    # lanes x (unpack, step, export), + the counter update with a device counter; from 2^18 envs on 2 lanes, 4 when the
+    # step is replayed as a graph (device counter): 13 / 6 launches per step at 2^18 + 1031 envs
+    lanes = 1 if e < (1 << 18) else (2 if mode == "host_counter" else 4)
+    assert per_step == lanes * 3 + (1 if mode != "host_counter" else 0)
     assert np.array_equal(dut.state.cpu().numpy(), ref.state.cpu().numpy())
+    ref.close(); dut.close()
+
+
+@pytest.mark.parametrize("compact", [False, True, "packed"])
+def test_step_host_between_pdl_steps(compact):
+    """On a pdl env, step_host closes the open PDL sequence and the library advances the device counter itself:
+    steps and host steps interleaved (two host steps in a row included) draw the random streams of a host-counter twin,
+    step for step."""
+    import torch
+    e, name = 3 * 1024 + 5, "pbn28"
+    ref = _mk(name, e, auto_reset=True)
+    dut = _mk(name, e, auto_reset=True, pdl=True)
+    for env in (ref, dut):
+        _seed_env(env, name, e, 13)
+    rng = np.random.default_rng(14)
+    a16 = dut.pinned_actions16()
+    for step in range(8):
+        act = rng.integers(0, 29, size=(e, 3), dtype=np.uint8)
+        ref.step(torch.from_numpy(act).cuda())
+        state, term, trunc = (x.cpu().numpy() for x in (ref.state, ref.terminated, ref.truncated))
+        reward = ref.reward.cpu().numpy()
+        if step not in (2, 3, 6):
+            dut.step(torch.from_numpy(act).cuda())
+            assert np.array_equal(dut.state.cpu().numpy(), state), f"state at step {step}"
+            assert np.array_equal(dut.reward.cpu().numpy(), reward), f"reward at step {step}"
+            continue
+        if compact == "packed":
+            a16.numpy().view(np.uint16)[...] = dut.pack_actions16(act)
+            out = dut.step_host(None, compact="packed", actions16=a16)
+            packed = out["packed"]
+            assert np.array_equal(packed & np.uint32((1 << 30) - 1), state[:, 0].astype(np.uint32)), f"state at step {step}"
+            assert np.array_equal((packed >> np.uint32(30)) & np.uint32(1), term.astype(np.uint32))
+            assert np.array_equal(packed >> np.uint32(31), trunc.astype(np.uint32))
+        elif compact:
+            out = dut.step_host(act, compact=True)
+            assert np.array_equal(out["state32"].astype(np.int64), state[:, 0]), f"state at step {step}"
+            assert np.array_equal(out["reward"], reward)
+            assert np.array_equal(out["done"], term | (trunc << 1))
+        else:
+            out = dut.step_host(act)
+            assert np.array_equal(out["state"], state), f"state at step {step}"
+            assert np.array_equal(out["reward"], reward)
+            assert np.array_equal(out["terminated"], term) and np.array_equal(out["truncated"], trunc)
+    dut.advance_counter()
+    assert int(dut.step_ctr_dev.item()) == 8
+    assert ref.stats() == dut.stats()
     ref.close(); dut.close()
 
 
