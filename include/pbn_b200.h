@@ -290,6 +290,25 @@ int pbn_resident_export(pbn_handle* h, const uint32_t* resident, uint64_t* state
 int pbn_rollout(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t step_ctr, int64_t env_offset,
                 int64_t n_envs, unsigned long long* stats, void* stream);
 
+/* ---- Steady-state statistics (compute_ssd_hist, train_pbn_28.py:257) ---------------------------------------
+ * A record ADDS into caller-owned DEVICE u64 accumulators and never overwrites them, so successive calls and shards
+ * of a batch can be summed:
+ *   gene_on [N] (may be NULL): gene_on[g] += the number of recorded env-states in which gene g is 1;
+ *   hist [2^n_proj] (may be NULL): the states projected onto the n_proj (0..12) distinct genes proj_genes[0..n_proj)
+ *     (a HOST array): bin b = sum_j bit(state, proj_genes[j]) << j (the packing of steady_state_histogram(genes=...));
+ *     with n_proj = 0, hist[0] counts every recorded state.
+ * Only real envs are counted, never the padding of a ragged last tile.  Invalid input (n_proj > 12, a repeated or
+ * out-of-range projection gene, stride < 1, the pbn_rollout checks) returns PBN_ERR_INVALID. */
+/* n_steps uncontrolled updates exactly as pbn_rollout (same streams, same final states, same stats), and after
+ * update s (s = 1..n_steps) the states are recorded iff s % stride == 0.  Sliced kernel only (PBN_ERR_UNSUPPORTED
+ * otherwise).  The recording kernel is a separate specialisation, compiled on the first call. */
+int pbn_rollout_record(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t step_ctr, int64_t env_offset,
+                       int64_t n_envs, int32_t stride, const int32_t* proj_genes, int32_t n_proj,
+                       unsigned long long* gene_on, unsigned long long* hist, unsigned long long* stats, void* stream);
+/* Record n_envs row-format states once (any kernel): after a pbn_step, for policy-in-the-loop statistics. */
+int pbn_record_states(pbn_handle* h, const uint64_t* state, int64_t n_envs, const int32_t* proj_genes,
+                      int32_t n_proj, unsigned long long* gene_on, unsigned long long* hist, void* stream);
+
 /* The same step with injected predictor choices / perturbation masks: the parity entry point
  * (deterministic core T of SURVEY.md 8a-4).  args->sel must be non-NULL. */
 int pbn_step_injected(pbn_handle* h, const pbn_step_args* args, void* stream);

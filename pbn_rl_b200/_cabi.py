@@ -33,7 +33,7 @@ EXPORTS = (
     "pbn_advance_counter", "pbn_step_host", "pbn_replay_observe", "pbn_replay_commit", "pbn_replay_sample",
     "pbn_observe", "pbn_in_target", "pbn_rollout_track", "pbn_rollout_reduce",
     "pbn_visit_count", "pbn_successor_sets", "pbn_closure_expand", "pbn_closure_reach",
-    "pbn_rollout",
+    "pbn_rollout", "pbn_rollout_record", "pbn_record_states",
     "pbn_resident_words", "pbn_resident_import", "pbn_resident_export", "pbn_reward_table", "pbn_attractor_hash_slots",
     "pbn_per_tree_floats", "pbn_per_init", "pbn_per_push", "pbn_per_update", "pbn_per_sample",
 )
@@ -213,6 +213,10 @@ def load_library(path: Optional[os.PathLike] = None) -> C.CDLL:
     lib.pbn_resident_export.restype = C.c_int
     lib.pbn_rollout.argtypes = [vp, vp, i64, u64, i64, i64, vp, vp]
     lib.pbn_rollout.restype = C.c_int
+    lib.pbn_rollout_record.argtypes = [vp, vp, i64, u64, i64, i64, i32, vp, i32, vp, vp, vp, vp]
+    lib.pbn_rollout_record.restype = C.c_int
+    lib.pbn_record_states.argtypes = [vp, vp, i64, vp, i32, vp, vp, vp]
+    lib.pbn_record_states.restype = C.c_int
     lib.pbn_step_injected.argtypes = [vp, C.POINTER(StepArgs), vp]
     lib.pbn_step_injected.restype = C.c_int
     lib.pbn_reset.argtypes = [vp, vp, vp, vp, vp, vp, u64, i64, i64, vp]

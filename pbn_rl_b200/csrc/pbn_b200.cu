@@ -20,6 +20,7 @@
 #include "discover.cuh"
 #include "resident.cuh"
 #include "per.cuh"
+#include "record.cuh"
 
 using namespace pbn;
 
@@ -126,8 +127,12 @@ struct pbn_handle {
   cudaKernel_t jit_kernel_gen[2] = {nullptr, nullptr};  // pbn_step_sliced_gen (hash set / global table / r_wrong)
   cudaKernel_t planes_kernel[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};  // [injected][0: 4 warps, 1: 8 warps] pbn_step_planes_w*
   uint32_t planes_smem_opt_in[2][2] = {{48u * 1024u, 48u * 1024u}, {48u * 1024u, 48u * 1024u}};
-  cudaKernel_t rollout_kernel = nullptr;  // pbn_rollout_sliced
+  cudaKernel_t rollout_kernel = nullptr;  // pbn_rollout_sliced<false>
   uint32_t rollout_smem_opt_in = 48u * 1024u;
+  cudaLibrary_t jit_lib_record = nullptr;  // the recording rollout's program, loaded on first use
+  std::string jit_key_record;
+  cudaKernel_t record_kernel = nullptr;   // pbn_rollout_sliced<true>
+  uint32_t record_smem_opt_in = 48u * 1024u;
   std::vector<uint32_t> surv_sliced_host;  // copied into every loaded specialisation's constant memory
   int sliced_threads = 128, sliced_min_blocks = 1;
   uint32_t jit_smem_opt_in[2][2] = {{48u * 1024u, 48u * 1024u}, {48u * 1024u, 48u * 1024u}};  // [injected][gen]
@@ -245,7 +250,7 @@ static int load_sliced(pbn_handle* h, int injected) {
   }
   PBN_CUDA(cudaLibraryGetKernel(&h->jit_kernel[injected], h->jit_lib[injected], "pbn_step_sliced"));
   PBN_CUDA(cudaLibraryGetKernel(&h->jit_kernel_gen[injected], h->jit_lib[injected], "pbn_step_sliced_gen"));
-  if (!injected) PBN_CUDA(cudaLibraryGetKernel(&h->rollout_kernel, h->jit_lib[0], "pbn_rollout_sliced"));
+  if (!injected) PBN_CUDA(cudaLibraryGetKernel(&h->rollout_kernel, h->jit_lib[0], jit::kRolloutKernel));
   h->sliced_threads = jit::sliced_threads(h->gen);
   h->sliced_min_blocks = jit::sliced_min_blocks(h->gen);
   return PBN_OK;
@@ -350,6 +355,20 @@ static int launch_sliced(pbn_handle* h, StepParams& p, bool injected, cudaStream
   } else {
     PBN_CUDA(cudaLaunchKernel(reinterpret_cast<const void*>(k), dim3((unsigned)grid), dim3((unsigned)h->sliced_threads), args, L.total, stream));
   }
+  return PBN_OK;
+}
+
+// The recording rollout's specialisation (own program, own-RNG only, compiled / loaded on first use).
+static int load_record(pbn_handle* h) {
+  if (h->record_kernel) return PBN_OK;
+  std::vector<char> cubin;
+  std::string err;
+  if (jit::compile(h->gen, false, 2, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());
+  {
+    const int rc = acquire_module(h, cubin, true, &h->jit_lib_record, &h->jit_key_record);
+    if (rc != PBN_OK) return rc;
+  }
+  PBN_CUDA(cudaLibraryGetKernel(&h->record_kernel, h->jit_lib_record, jit::kRecordKernel));
   return PBN_OK;
 }
 
@@ -467,6 +486,7 @@ void pbn_destroy(pbn_handle* h) {
       release_module(h->jit_key[i]);
       release_module(h->jit_key_planes[i]);
     }
+    release_module(h->jit_key_record);
     for (int c = 0; c < pbn_handle::kMaxLanes; ++c) {
       if (h->s_lane[c]) cudaStreamDestroy(h->s_lane[c]);
       if (h->ev_k[c]) cudaEventDestroy(h->ev_k[c]);
@@ -844,6 +864,7 @@ int pbn_jit_precompile(const pbn_net_desc* d) {
     std::string err;
     for (int part = 0; part < (jit::sel_bits(g) == 3 ? 1 : 2); ++part)   // (no plane-resident program with three selection planes)
       if (jit::compile(g, inj != 0, part, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());
+    if (!inj && jit::compile(g, false, 2, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());   // recording rollout
   }
   return PBN_OK;
 }
@@ -877,6 +898,88 @@ int pbn_rollout(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t step_c
   if (grid > cap) grid = cap;
   void* args[] = {&p};
   PBN_CUDA(cudaLaunchKernel(reinterpret_cast<const void*>(h->rollout_kernel), dim3((unsigned)grid), dim3((unsigned)h->sliced_threads), args, smem, stream));
+  h->launches += 1, g_last_advance = nullptr;
+  return PBN_OK;
+}
+
+// Checks the projection of a recording call and copies it into proj[12].
+static int record_projection(const pbn_handle* h, const char* who, const int32_t* proj_genes, int32_t n_proj, int32_t* proj) {
+  if (n_proj < 0 || n_proj > 12) return fail(PBN_ERR_INVALID, "%s: n_proj = %d, must be in [0, 12]", who, n_proj);
+  if (n_proj > 0 && !proj_genes) return fail(PBN_ERR_INVALID, "%s: proj_genes is NULL", who);
+  for (int j = 0; j < 12; ++j) proj[j] = 0;
+  for (int j = 0; j < n_proj; ++j) {
+    const int32_t g = proj_genes[j];
+    if (g < 0 || g >= h->net.n_genes) return fail(PBN_ERR_INVALID, "%s: projection gene %d outside [0, %d)", who, g, h->net.n_genes);
+    for (int i = 0; i < j; ++i)
+      if (proj[i] == g) return fail(PBN_ERR_INVALID, "%s: projection gene %d appears twice", who, g);
+    proj[j] = g;
+  }
+  return PBN_OK;
+}
+
+int pbn_rollout_record(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t step_ctr, int64_t env_offset,
+                       int64_t n_envs, int32_t stride, const int32_t* proj_genes, int32_t n_proj,
+                       unsigned long long* gene_on, unsigned long long* hist, unsigned long long* stats, void* stream_) {
+  if (!h || !state) return fail(PBN_ERR_INVALID, "null argument");
+  if (h->kernel != PBN_KERNEL_SLICED)
+    return fail(PBN_ERR_UNSUPPORTED, "pbn_rollout_record: the handle runs the scalar kernel (loop over pbn_step + pbn_record_states)");
+  if (n_envs < 0 || n_steps < 0 || n_steps > 0x7FFFFFFF || env_offset < 0 || (env_offset & 1023)) return fail(PBN_ERR_INVALID, "bad n_envs / n_steps / env_offset");
+  if (stride < 1) return fail(PBN_ERR_INVALID, "pbn_rollout_record: stride = %d, must be >= 1", stride);
+  RecordParams q;
+  int rc = record_projection(h, "pbn_rollout_record", proj_genes, n_proj, q.proj);
+  if (rc != PBN_OK) return rc;
+  if (n_envs == 0 || n_steps == 0) return PBN_OK;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  if ((rc = load_sliced(h, 0)) != PBN_OK || (rc = load_record(h)) != PBN_OK) return rc;
+  const int N = h->net.n_genes, NW = (N + 31) / 32, NSEL = jit::n_sel_slots(h->gen);
+  // the rollout's scratch (pbn_rollout), then the 2^n_proj histogram bins
+  const uint32_t smem = (uint32_t)(2 * NW * 1024 + jit::sel_bits(h->gen) * NSEL * 32 + 128 * (8 * N < 255 ? 1 : 2) + 32 + 8 + (1 << n_proj)) * 4u;
+  if (smem > 227u * 1024u) return fail(PBN_ERR_UNSUPPORTED, "pbn_rollout_record needs %u B of shared memory", smem);
+  if ((rc = ensure_dynamic_smem(h->record_kernel, smem, &h->record_smem_opt_in)) != PBN_OK) return rc;
+  q.r.n = h->net;
+  q.r.state = state;
+  q.r.stats = stats;
+  q.r.step_ctr = step_ctr;
+  q.r.env_offset = env_offset;
+  q.r.n_envs = n_envs;
+  q.r.n_steps = (int32_t)n_steps;
+  q.gene_on = gene_on;
+  q.hist = hist;
+  q.stride = stride;
+  q.n_proj = n_proj;
+  int64_t grid = (n_envs + 1023) / 1024;
+  const int64_t cap = (int64_t)h->num_sms * h->sliced_min_blocks * 8;
+  if (grid > cap) grid = cap;
+  void* args[] = {&q};
+  PBN_CUDA(cudaLaunchKernel(reinterpret_cast<const void*>(h->record_kernel), dim3((unsigned)grid), dim3((unsigned)h->sliced_threads), args, smem, stream));
+  h->launches += 1, g_last_advance = nullptr;
+  return PBN_OK;
+}
+
+int pbn_record_states(pbn_handle* h, const uint64_t* state, int64_t n_envs, const int32_t* proj_genes, int32_t n_proj,
+                      unsigned long long* gene_on, unsigned long long* hist, void* stream_) {
+  if (!h) return fail(PBN_ERR_INVALID, "null argument");
+  if (n_envs < 0) return fail(PBN_ERR_INVALID, "pbn_record_states: n_envs < 0");
+  if (n_envs > 0 && !state) return fail(PBN_ERR_INVALID, "pbn_record_states: state is NULL");
+  RecordStatesParams q;
+  int rc = record_projection(h, "pbn_record_states", proj_genes, n_proj, q.proj);
+  if (rc != PBN_OK) return rc;
+  if (n_envs == 0 || (!gene_on && !hist)) return PBN_OK;
+  DeviceGuard guard(h->device);
+  q.state = state;
+  q.gene_on = gene_on;
+  q.hist = hist;
+  q.n_envs = n_envs;
+  q.n_genes = h->net.n_genes;
+  q.W = h->W;
+  q.n_proj = n_proj;
+  const uint32_t smem = (uint32_t)((hist ? (1u << n_proj) : 0u) * 4u + 128u * 8u);
+  int64_t grid = (n_envs + kRecordThreads - 1) / kRecordThreads;
+  const int64_t cap = (int64_t)h->num_sms * 4;
+  if (grid > cap) grid = cap;
+  record_states_kernel<<<(unsigned)grid, kRecordThreads, smem, static_cast<cudaStream_t>(stream_)>>>(q);
+  PBN_CUDA(cudaGetLastError());
   h->launches += 1, g_last_advance = nullptr;
   return PBN_OK;
 }

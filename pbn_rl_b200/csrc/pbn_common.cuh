@@ -91,6 +91,16 @@ struct RolloutParams {
   int32_t n_steps;
 };
 
+// pbn_rollout_record: the rollout, and the states after every update s with s % stride == 0 counted into the caller's
+// u64 accumulators (include/pbn_b200.h).
+struct RecordParams {
+  RolloutParams r;
+  unsigned long long* gene_on;  // [N] or nullptr
+  unsigned long long* hist;     // [2^n_proj] or nullptr
+  int32_t stride, n_proj;
+  int32_t proj[12];             // bin bit j = gene proj[j]
+};
+
 // Effective Philox step counter of this launch (host part + optional device-resident part).
 __device__ __forceinline__ uint64_t effective_step(const pbn_step_args& a) {
   uint64_t step = a.step_ctr;

@@ -726,17 +726,22 @@ inline bool profile_build() {
   return env && env[0] && env[0] != '0';
 }
 
+// Mangled names of the two instances of the rollout kernel template (step_sliced.cuh: pbn_rollout_sliced<REC>).
+constexpr const char* kRolloutKernel = "_ZN3pbn18pbn_rollout_slicedILb0EEEvNS_8RollArgsIXT_EE1TE";
+constexpr const char* kRecordKernel = "_ZN3pbn18pbn_rollout_slicedILb1EEEvNS_8RollArgsIXT_EE1TE";
+
 // Compile (or fetch from the cache) the specialisation; returns 0 or PBN_ERR_JIT with *err set.
 // part 0: the row-format kernels (pbn_step_sliced, pbn_rollout_sliced); part 1: the plane-resident
-// kernels (pbn_step_planes_w4 / _w8), compiled and loaded on first use -- two programs, so that an env that never
-// uses one family never pays its compile time.
+// kernels (pbn_step_planes_w4 / _w8); part 2: the recording rollout (pbn_rollout_sliced<true>, own-RNG only).  Parts 1
+// and 2 are compiled and loaded on first use -- separate programs, so that an env that never uses one family never
+// pays its compile time.
 inline int compile(const GenNet& g, bool injected, int part, std::vector<char>* cubin, std::string* err) {
   std::string gen_h, upd;
   generate(g, injected, &gen_h, &upd);
   const std::string main_src = main_source();
   const bool profile = profile_build();
   const char* opts[] = {"--gpu-architecture=sm_100a", "-std=c++17", "-lineinfo", "-default-device",
-                        part ? "-DPBN_BUILD=1" : "-DPBN_BUILD=0", "-DPBN_PROFILE=1"};
+                        part == 2 ? "-DPBN_BUILD=2" : part ? "-DPBN_BUILD=1" : "-DPBN_BUILD=0", "-DPBN_PROFILE=1"};
   const int n_opts = profile ? 6 : 5;
   std::string key = gen_h + upd + main_src + kSrc_step_sliced + kSrc_step_planes + kSrc_pbn_common + kSrc_philox + kSrc_pbn_b200_h;
   for (int i = 0; i < n_opts; ++i) key += opts[i];

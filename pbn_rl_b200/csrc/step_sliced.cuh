@@ -1075,7 +1075,7 @@ pbn_step_sliced_gen(const __grid_constant__ StepParams p, const SlicedSmemLayout
 
 #endif  // PBN_BUILD == 0
 
-#if !PBN_INJECTED && PBN_BUILD == 0
+#if !PBN_INJECTED && (PBN_BUILD == 0 || PBN_BUILD == 2)
 // ---- pbn_rollout: S uncontrolled updates (env.step([]) S times, graph_classifier/__init__.py:148; the burn-in of
 // the attractor search; compute_ssd_hist's long runs) in ONE launch.  The tile's 1024 states are loaded and
 // bit-transposed once, then stay in shared memory as bit-planes: per update only the Philox selection
@@ -1089,10 +1089,30 @@ constexpr int kRollEv = kRollSel1 + (PBN_SELBITS - 1) * PBN_NSEL * 32;
 constexpr int kRollAny = kRollEv + 128 * kEvWords;              // mode A: rows of the column with an event [32]
 constexpr int kRollStat = kRollAny + 32;
 constexpr int kRollWords = kRollStat + 8;
+constexpr int kRollHist = kRollWords;                           // recording: 2^n_proj histogram bins (u32)
+constexpr int kGenesPerWarp = (PBN_N + kWarps - 1) / kWarps;    // recording: genes g = w, w + 4, ... of warp w
+// Recording: the shared-memory histogram bins and the per-thread gene counters are u32.  They are flushed into the u64
+// accumulators at the end of every tile and, within a tile, after every kRecordFlush recorded updates.  Between two
+// flushes a bin gains at most 1024 per recorded update (the tile's envs) and a gene counter at most 32 (its column),
+// so they stay below 2^21 * 1024 = 2^31; the warp sum of the 32 gene counters of a gene stays below 2^21 * 1024 too.
+constexpr int32_t kRecordFlush = 1 << 21;
 
-extern "C" __global__ void __launch_bounds__(PBN_THREADS, PBN_MIN_BLOCKS)
-pbn_rollout_sliced(const __grid_constant__ RolloutParams p) {
+template <bool REC> struct RollArgs { using T = RolloutParams; };
+template <> struct RollArgs<true> { using T = RecordParams; };
+__device__ __forceinline__ const RolloutParams& rollout_of(const RolloutParams& q) { return q; }
+__device__ __forceinline__ const RolloutParams& rollout_of(const RecordParams& q) { return q.r; }
+
+// The rollout: REC = false is the plain rollout (pbn_rollout, program 0); REC = true (pbn_rollout_record, program 2) also
+// records the states after every update s with s % stride == 0 into the caller's accumulators.  The two are instances of
+// one kernel template, looked up by their mangled names (sliced_host.cuh: kRolloutKernel, kRecordKernel): extern "C"
+// kernels that inline a shared body compile the plain rollout to different SASS (same instruction count, other
+// registers and schedule), a template kernel to the same SASS as before.
+template <bool REC>
+__global__ void __launch_bounds__(PBN_THREADS, PBN_MIN_BLOCKS) pbn_rollout_sliced(const __grid_constant__ typename RollArgs<REC>::T q) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
+  const RolloutParams& p = rollout_of(q);
+  const RecordParams* rec = nullptr;
+  if constexpr (REC) rec = &q;
   uint32_t* scr = reinterpret_cast<uint32_t*>(smem_raw);
   const NetParams& n = p.n;
   const uint32_t lane = threadIdx.x & 31u, w = threadIdx.x >> 5;
@@ -1105,12 +1125,84 @@ pbn_rollout_sliced(const __grid_constant__ RolloutParams p) {
   const int pert_mode = n.pert_rng ? n.pert_mode : PBN_PERT_NONE;  // block-uniform
   pbn_step_args dummy{};
   if (threadIdx.x < 8) s_stat[threadIdx.x] = 0u;
+  // recording (REC): histogram bins [2^n_proj] in shared memory, this thread's column counts of genes w + 4k
+  uint32_t* bins = scr + kRollHist;
+  uint32_t gcnt[kGenesPerWarp];
+  int32_t n_rec = 0;   // recorded updates since the last flush (block-uniform)
+  if constexpr (REC) {
+    for (int b = threadIdx.x; b < (1 << rec->n_proj); b += kWarps * 32) bins[b] = 0u;   // first added to after a barrier
+#pragma unroll
+    for (int k = 0; k < kGenesPerWarp; ++k) gcnt[k] = 0u;
+  }
+  // Record the planes of a completed update (all their writes are ordered before this by a barrier).  vm: the real envs
+  // of the column; valid: the real envs among this thread's 8 rows.
+  auto record = [&](const uint32_t* planes, uint32_t vm, uint32_t valid) {
+    if (rec->gene_on != nullptr) {
+#pragma unroll
+      for (int k = 0; k < kGenesPerWarp; ++k) {
+        const int g = (int)w + kWarps * k;
+        if (g < PBN_N) gcnt[k] += __popc(planes[g * 32 + lane] & vm);
+      }
+    }
+    if (rec->hist != nullptr) {
+      // bin of row i: bit j = gene proj[j] of the row's env (bit 8w + i of plane proj[j])
+      uint32_t idx[8];
+#pragma unroll
+      for (int i = 0; i < 8; ++i) idx[i] = 0u;
+#pragma unroll
+      for (int j = 0; j < 12; ++j) {
+        if (j < rec->n_proj) {
+          const uint32_t x = planes[rec->proj[j] * 32 + lane] >> (8u * w);
+#pragma unroll
+          for (int i = 0; i < 8; ++i) idx[i] |= ((x >> i) & 1u) << j;
+        }
+      }
+      // a steady state sits on few bins: the lanes of a row that share a bin add once, through their first lane
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        const bool ok = (valid >> i) & 1u;
+        const uint32_t peers = __match_any_sync(0xFFFFFFFFu, ok ? idx[i] : 0xFFFFFFFFu);
+        if (ok && __ffs(peers) - 1 == (int)lane) atomicAdd(&bins[idx[i]], (uint32_t)__popc(peers));
+      }
+    }
+  };
+  // add the u32 counters into the u64 accumulators and clear them (every thread, after a barrier)
+  auto flush = [&]() {
+    if (rec->hist != nullptr) {
+      for (int b = threadIdx.x; b < (1 << rec->n_proj); b += kWarps * 32) {
+        const uint32_t v = bins[b];
+        if (v != 0u) {
+          atomicAdd(&rec->hist[b], (unsigned long long)v);
+          bins[b] = 0u;
+        }
+      }
+    }
+    if (rec->gene_on != nullptr) {
+#pragma unroll
+      for (int k = 0; k < kGenesPerWarp; ++k) {
+        const int g = (int)w + kWarps * k;
+        const uint32_t sum = __reduce_add_sync(0xFFFFFFFFu, gcnt[k]);
+        if (g < PBN_N && lane == 0u && sum != 0u) atomicAdd(&rec->gene_on[g], (unsigned long long)sum);
+        gcnt[k] = 0u;
+      }
+    }
+    n_rec = 0;
+  };
   for (int64_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
     const int64_t e0 = tile * 1024 + 4 * (int64_t)lane;
     const uint64_t gid = (uint64_t)(((p.env_offset >> 10) + tile) * 32 + lane);
     uint32_t* cur = scr;                    // current planes
     uint32_t* nxt = scr + kRollPlanes;      // next planes (first: the rows, before the transpose)
     uint32_t valid = 0u;                    // which of this warp's 8 rows are real envs
+    uint32_t vm = 0xFFFFFFFFu;              // REC: which of the column's 32 envs are real (bit b: env e0 + 128 (b >> 2) + (b & 3))
+    int32_t phase = 0;                      // REC: updates since the last recorded one
+    if constexpr (REC) {
+      if ((tile + 1) * 1024 > E) {
+        vm = 0u;
+#pragma unroll
+        for (int b = 0; b < 32; ++b) vm |= (e0 + 128 * (b >> 2) + (b & 3) < E ? 1u : 0u) << b;
+      }
+    }
     // ---- rows of this warp's 8 envs -> scratch
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
@@ -1142,6 +1234,17 @@ pbn_rollout_sliced(const __grid_constant__ RolloutParams p) {
         if (pert_mode == PBN_PERT_A && w == 0u) anym[lane] = 0u;
       }
       __syncthreads();   // planes `cur` complete (transpose / previous update), selection planes drawn
+      if constexpr (REC) {
+        if (s != 0 && ++phase == rec->stride) {   // `cur` holds the state after update s
+          phase = 0;
+          record(cur, vm, valid);
+          if (++n_rec == kRecordFlush) {
+            __syncthreads();
+            flush();
+            __syncthreads();
+          }
+        }
+      }
       pbn_update_part(w, cur + lane, nxt + lane, sel0, sel1, PBN_SEL2_OF(sel1) 0u);
       if (pert_mode != PBN_PERT_NONE) {
         // this thread's events: (gene, row 8w + ib) of its column
@@ -1220,6 +1323,9 @@ pbn_rollout_sliced(const __grid_constant__ RolloutParams p) {
       uint32_t* t = cur; cur = nxt; nxt = t;
     }
     __syncthreads();         // the last update (and its flips) is complete
+    if constexpr (REC) {
+      if (++phase == rec->stride) record(cur, vm, valid);
+    }
     // ---- bit-planes -> this warp's 8 rows -> HBM
     uint32_t o[8][kNW];
 #pragma unroll
@@ -1247,12 +1353,19 @@ pbn_rollout_sliced(const __grid_constant__ RolloutParams p) {
       }
     }
     __syncthreads();         // scratch is reused by the next tile
+    if constexpr (REC) flush();   // (the next tile records after its first barrier)
   }
   if (p.stats != nullptr && threadIdx.x == 0) {
     atomicAdd(&p.stats[PBN_STAT_STEPS], (unsigned long long)s_stat[0] * (unsigned long long)p.n_steps);
     if (s_stat[1]) atomicAdd(&p.stats[PBN_STAT_PERTURBED], (unsigned long long)s_stat[1]);
   }
 }
+
+#if PBN_BUILD == 0
+template __global__ void pbn_rollout_sliced<false>(const __grid_constant__ RolloutParams q);
+#else   // the recording rollout's program (sliced_host.cuh: compile part 2)
+template __global__ void pbn_rollout_sliced<true>(const __grid_constant__ RecordParams q);
+#endif
 #endif
 
 }  // namespace pbn

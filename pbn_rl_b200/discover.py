@@ -14,10 +14,14 @@ Here:
   the whole STG, so every attractor returned is exact (closed and strongly connected); what is sampled is
   only *which* attractors are found (those with a basin the rollouts hit).
 * :func:`steady_state_histogram` -- visit counts of (projected) states over many perturbed steps.
+* :func:`steady_state_statistics` / :class:`StateRecorder` -- per-gene ON frequencies and the distribution of the
+  state projected onto up to 12 genes, counted on the device (``pbn_rollout_record`` inside the rollout kernel,
+  ``pbn_record_states`` after a step); full states of more than 12 genes go through :func:`steady_state_histogram`.
 """
 from __future__ import annotations
 
-from typing import Dict, List, Optional, Sequence, Tuple, Union
+import ctypes as C
+from typing import Callable, Dict, List, Optional, Sequence, Tuple, Union
 
 import numpy as np
 import torch
@@ -28,7 +32,7 @@ from .network import PBNNetwork
 from .vec_env import VecPBNEnv
 
 __all__ = ["VisitCounter", "find_attractors_rollout", "attractor_reached_from", "basin_labels", "steady_state_histogram", "successor_descriptors",
-           "forward_closure", "sink_sccs_of_closed_set"]
+           "forward_closure", "sink_sccs_of_closed_set", "StateRecorder", "steady_state_statistics"]
 
 
 def _words_to_int(words: Sequence[int]) -> int:
@@ -363,3 +367,81 @@ def steady_state_histogram(env: VecPBNEnv, steps: int, actions: Optional[torch.T
             table.add(proj)
     states, counts = table.items()
     return {_words_to_int(states[k]): int(counts[k]) for k in range(len(counts))}
+
+
+class StateRecorder:
+    """Device accumulators of steady-state statistics for the states of ``env``: per-gene ON counts
+    (``marginals=True``) and the histogram of the states projected onto ``genes`` (at most 12 distinct genes; bin
+    bit j = gene ``genes[j]``, the packing of :func:`steady_state_histogram`; ``genes=None`` keeps no histogram,
+    ``genes=[]`` one bin counting every state).  Counts only ever grow: :meth:`add` and
+    ``env.rollout(n, recorder=...)`` add to them."""
+
+    def __init__(self, env: VecPBNEnv, genes: Optional[Sequence[int]] = None, marginals: bool = True):
+        self.env = env
+        self.genes = None if genes is None else [int(g) for g in genes]
+        if self.genes is not None:
+            if len(self.genes) > 12:
+                raise ValueError("at most 12 genes in a projection (full states: steady_state_histogram)")
+            if len(set(self.genes)) != len(self.genes) or any(g < 0 or g >= env.n_genes for g in self.genes):
+                raise ValueError("projection genes must be distinct and in [0, %d)" % env.n_genes)
+        self.k = 0 if self.genes is None else len(self.genes)
+        self._proj = (C.c_int32 * 12)(*(self.genes or []))
+        self._proj_ptr = C.addressof(self._proj)
+        dev = env.device
+        self.gene_on = torch.zeros((env.n_genes,), dtype=torch.int64, device=dev) if marginals else None
+        self.hist = torch.zeros((1 << self.k,), dtype=torch.int64, device=dev) if self.genes is not None else None
+        self.n = 0   # recorded env-states
+
+    def add(self, states: Optional[torch.Tensor] = None) -> None:
+        """Record ``states`` (row-format ``[E, W]`` words; default: the env's current states) once."""
+        env = self.env
+        states = env.state if states is None else states.to(device=env.device, dtype=torch.int64).contiguous()
+        if states.dim() != 2 or states.shape[1] != env.n_words:
+            raise ValueError("states must be [E, %d] int64 words" % env.n_words)
+        check(env.lib.pbn_record_states(env._h, states.data_ptr(), states.shape[0], self._proj_ptr, self.k,
+                                        None if self.gene_on is None else self.gene_on.data_ptr(),
+                                        None if self.hist is None else self.hist.data_ptr(), env._stream()))
+        self.n += int(states.shape[0])
+
+    def counts(self) -> Tuple[Optional[np.ndarray], Optional[np.ndarray]]:
+        """The raw accumulators ``(gene_on [N], hist [2^k])`` as uint64 arrays (``None`` where not kept)."""
+        f = (lambda t: None if t is None else t.cpu().numpy().astype(np.uint64))
+        return f(self.gene_on), f(self.hist)
+
+    def marginals(self) -> np.ndarray:
+        """P(gene g is ON) over the recorded states, float64 ``[N]``."""
+        if self.gene_on is None:
+            raise ValueError("this recorder keeps no per-gene counts (marginals=False)")
+        return self.gene_on.cpu().numpy().astype(np.float64) / max(self.n, 1)
+
+    def distribution(self) -> np.ndarray:
+        """Frequency of every projected state over the recorded states, float64 ``[2^k]``."""
+        if self.hist is None:
+            raise ValueError("this recorder keeps no histogram (genes=None)")
+        return self.hist.cpu().numpy().astype(np.float64) / max(self.n, 1)
+
+
+def steady_state_statistics(env: VecPBNEnv, steps: int, burn_in: int = 0, genes: Optional[Sequence[int]] = None,
+                            stride: int = 1, policy: Optional[Callable[[torch.Tensor], torch.Tensor]] = None,
+                            marginals: bool = True) -> StateRecorder:
+    """Steady-state statistics of ``env``'s network (``compute_ssd_hist``, train_pbn_28.py:257): ``burn_in`` steps,
+    then ``steps`` more, recording every instance's state after each step ``s`` (``s = 1..steps``) with
+    ``s % stride == 0``.  Returns the :class:`StateRecorder` (``marginals()``, ``distribution()`` over ``genes``).
+
+    Without ``policy`` the network runs uncontrolled: ``env.rollout(burn_in)`` and ``env.rollout(steps,
+    recorder=..., stride=stride)``, the recording fused into the rollout kernel on the sliced kernel.  With
+    ``policy(obs) -> actions`` the agent acts at every step: ``observe -> policy -> step -> record``, the
+    controlled steady state ``compute_ssd_hist(env, model)`` estimates.  Actions are uint8 ``[E, bins]`` as
+    :meth:`VecPBNEnv.step` takes them; the env's horizon, targets and auto-reset apply as in any other step."""
+    rec = StateRecorder(env, genes=genes, marginals=marginals)
+    if policy is None:
+        env.rollout(int(burn_in), stats=False)
+        env.rollout(int(steps), stats=False, recorder=rec, stride=int(stride))
+        return rec
+    if int(stride) < 1:
+        raise ValueError("stride must be >= 1")
+    for s in range(1, int(burn_in) + int(steps) + 1):
+        env.step(policy(env.observe()), stats=False)
+        if s > int(burn_in) and (s - int(burn_in)) % int(stride) == 0:
+            rec.add()
+    return rec

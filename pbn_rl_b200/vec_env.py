@@ -374,13 +374,24 @@ class VecPBNEnv:
             self.step_ctr += 1
         return (None if a.resident else self._state), self.reward, self.terminated, self.truncated
 
-    def rollout(self, n_steps: int, stats: bool = True) -> torch.Tensor:
+    def rollout(self, n_steps: int, stats: bool = True, recorder=None, stride: int = 1) -> torch.Tensor:
         """``n_steps`` uncontrolled updates of every instance (``env.step([])`` ``n_steps`` times,
         graph_classifier/__init__.py:148) in one launch: the states stay on chip as bit-planes between the
         updates (``pbn_rollout``).  Only ``state`` changes -- bit-identical to ``n_steps`` calls of
         ``step(None)`` -- counters, targets, rewards and flags are left alone and nothing is reset.  Networks
-        the sliced kernel does not take fall back to a loop of steps."""
+        the sliced kernel does not take fall back to a loop of steps.
+
+        ``recorder`` (a :class:`pbn_rl_b200.discover.StateRecorder` of this env): the states after every update
+        ``s`` (``s = 1..n_steps``) with ``s % stride == 0`` are also counted into it, inside the same launch
+        (``pbn_rollout_record``); the updates themselves are the same.  The step-loop fallback calls
+        ``recorder.add()`` after every ``stride``-th step instead."""
         n_steps = int(n_steps)
+        stride = int(stride)
+        if recorder is not None:
+            if stride < 1:
+                raise ValueError("stride must be >= 1")
+            if recorder.env is not self:
+                raise ValueError("the recorder belongs to another env")
         if n_steps <= 0:
             return self.state
         if self.step_ctr_dev is not None:
@@ -388,14 +399,23 @@ class VecPBNEnv:
         if self.kernel != "sliced":
             saved = (self.t.clone(), self.target_id.clone(), self.auto_reset)
             self.auto_reset = False
-            for _ in range(n_steps):
+            for s in range(1, n_steps + 1):
                 self.step(None, stats=stats)
+                if recorder is not None and s % stride == 0:
+                    recorder.add()
             self.t.copy_(saved[0])
             self.target_id.copy_(saved[1])
             self.auto_reset = saved[2]
             return self.state
-        check(self.lib.pbn_rollout(self._h, _ptr(self.state), n_steps, self.step_ctr, self.env_offset, self.num_envs,
-                                   _ptr(self.stats_buf) if stats else None, self._stream()))
+        st = _ptr(self.stats_buf) if stats else None
+        if recorder is None:
+            check(self.lib.pbn_rollout(self._h, _ptr(self.state), n_steps, self.step_ctr, self.env_offset, self.num_envs,
+                                       st, self._stream()))
+        else:
+            check(self.lib.pbn_rollout_record(self._h, _ptr(self.state), n_steps, self.step_ctr, self.env_offset,
+                                              self.num_envs, stride, recorder._proj_ptr, recorder.k,
+                                              _ptr(recorder.gene_on), _ptr(recorder.hist), st, self._stream()))
+            recorder.n += self.num_envs * (n_steps // stride)
         self.step_ctr += n_steps
         return self.state
 

@@ -13,7 +13,7 @@ import torch
 
 from helpers import GOLD, attractor_set, product_net
 from pbn_rl_b200 import PBNNetwork, VecPBNEnv
-from pbn_rl_b200.discover import VisitCounter, find_attractors_rollout, steady_state_histogram
+from pbn_rl_b200.discover import StateRecorder, VisitCounter, find_attractors_rollout, steady_state_histogram
 from pbn_rl_b200.evaluate import evaluate_all_pairs, hamming_policy
 from pbn_rl_b200.replay import DeviceReplay
 
@@ -79,6 +79,9 @@ assert env.kernel == "sliced"
 for _ in range(3):
     env.step(torch.from_numpy(rng.integers(0, 10, size=(1500, 3), dtype=np.uint8)).cuda())
 env.rollout(5)
+rec = StateRecorder(env, genes=[8, 0, 5])     # pbn_rollout_record (ragged last tile) and pbn_record_states
+env.rollout(5, recorder=rec, stride=2)
+rec.add()
 env.close()
 if "--host-lanes" in sys.argv:   # 2^18 envs: slow under the sanitizer's racecheck
     e = 1 << 18
