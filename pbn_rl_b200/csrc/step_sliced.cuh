@@ -1096,6 +1096,11 @@ constexpr int kGenesPerWarp = (PBN_N + kWarps - 1) / kWarps;    // recording: ge
 // flushes a bin gains at most 1024 per recorded update (the tile's envs) and a gene counter at most 32 (its column),
 // so they stay below 2^21 * 1024 = 2^31; the warp sum of the 32 gene counters of a gene stays below 2^21 * 1024 too.
 constexpr int32_t kRecordFlush = 1 << 21;
+// The perturbation count: a thread's u32 count covers at most kPertFold updates of its 8 rows (< 8 * 96 * 2^16 = 3 * 2^24
+// events, < 3 * 2^29 for the warp) before it is folded into the block's u64 counter; the count of a call is exact for
+// any n_steps and any number of tiles per block.
+constexpr int32_t kPertFold = 1 << 16;
+static_assert(kRollStat % 2 == 0, "the u64 perturbation counter at kRollStat + 2 must be 8-byte aligned");
 
 template <bool REC> struct RollArgs { using T = RolloutParams; };
 template <> struct RollArgs<true> { using T = RecordParams; };
@@ -1121,7 +1126,8 @@ __global__ void __launch_bounds__(PBN_THREADS, PBN_MIN_BLOCKS) pbn_rollout_slice
   uint32_t* sel0 = scr + kRollSel0 + lane;
   uint32_t* sel1 = scr + kRollSel1 + lane;
   uint32_t* anym = scr + kRollAny;
-  uint32_t* s_stat = scr + kRollStat;
+  uint32_t* s_stat = scr + kRollStat;   // [0]: the block's real envs; [2..3]: its perturbation count (u64)
+  unsigned long long* const s_pert = reinterpret_cast<unsigned long long*>(s_stat + 2);
   const int pert_mode = n.pert_rng ? n.pert_mode : PBN_PERT_NONE;  // block-uniform
   pbn_step_args dummy{};
   if (threadIdx.x < 8) s_stat[threadIdx.x] = 0u;
@@ -1224,7 +1230,7 @@ __global__ void __launch_bounds__(PBN_THREADS, PBN_MIN_BLOCKS) pbn_rollout_slice
 #pragma unroll
       for (int i = 0; i < 8; ++i) cur[(wd * 32 + 8 * (int)w + i) * 32 + lane] = q8[i];
     }
-    uint32_t npert = 0u;
+    uint32_t npert = 0u;   // this thread's perturbations since the last fold into s_pert
 #pragma unroll 1
     for (int s = 0; s < p.n_steps; ++s) {
       const uint64_t step_ctr = p.step_ctr + (uint64_t)s;
@@ -1321,6 +1327,11 @@ __global__ void __launch_bounds__(PBN_THREADS, PBN_MIN_BLOCKS) pbn_rollout_slice
         }
       }
       uint32_t* t = cur; cur = nxt; nxt = t;
+      if ((s & (kPertFold - 1)) == kPertFold - 1) {   // fold the count every kPertFold updates (unused without stats)
+        const uint32_t np = __reduce_add_sync(0xFFFFFFFFu, npert);
+        if (lane == 0u && np) atomicAdd(s_pert, (unsigned long long)np);
+        npert = 0u;
+      }
     }
     __syncthreads();         // the last update (and its flips) is complete
     if constexpr (REC) {
@@ -1349,7 +1360,7 @@ __global__ void __launch_bounds__(PBN_THREADS, PBN_MIN_BLOCKS) pbn_rollout_slice
       const uint32_t np = __reduce_add_sync(0xFFFFFFFFu, npert);
       if (lane == 0u) {
         atomicAdd(&s_stat[0], nv);
-        if (np) atomicAdd(&s_stat[1], np);
+        if (np) atomicAdd(s_pert, (unsigned long long)np);
       }
     }
     __syncthreads();         // scratch is reused by the next tile
@@ -1357,7 +1368,7 @@ __global__ void __launch_bounds__(PBN_THREADS, PBN_MIN_BLOCKS) pbn_rollout_slice
   }
   if (p.stats != nullptr && threadIdx.x == 0) {
     atomicAdd(&p.stats[PBN_STAT_STEPS], (unsigned long long)s_stat[0] * (unsigned long long)p.n_steps);
-    if (s_stat[1]) atomicAdd(&p.stats[PBN_STAT_PERTURBED], (unsigned long long)s_stat[1]);
+    if (*s_pert) atomicAdd(&p.stats[PBN_STAT_PERTURBED], *s_pert);
   }
 }
 

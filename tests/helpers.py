@@ -88,3 +88,76 @@ def random_case(name, e, seed, pert_density=0.05, sel_max=3):
     target = rng.integers(0, n_attr, size=e, dtype=np.int32)
     t = rng.integers(0, 25, size=e).astype(np.uint16)
     return dict(state=state, actions=actions, sel=sel, pert=pert, target=target, t=t)
+
+
+# ---- random networks at the edges of what the ABI admits (test_gpu_synthetic.py, test_gpu_edges.py)
+def _sop(names, table):
+    """Sum-of-products expression string for a truth table over `names` (bit j of the row index = names[j])."""
+    k = len(names)
+    rows = [a for a in range(1 << k) if (table >> a) & 1]
+    if k == 0 or not rows:
+        return "( %s & ~ %s )" % (names[0] if names else "x0", names[0] if names else "x0") if not rows else "( x0 | ~ x0 )"
+    if len(rows) == 1 << k:
+        return "( %s | ~ %s )" % (names[0], names[0])
+    terms = []
+    for a in rows:
+        terms.append("( " + " & ".join(("%s" if (a >> j) & 1 else "~ %s") % names[j] for j in range(k)) + " )")
+    return " | ".join(terms)
+
+
+def make_network(n, kmax, amax, seed, uniform=True):
+    rng = np.random.default_rng(seed)
+    genes = ["x%d" % i for i in range(n)]
+    exprs = []
+    for i in range(n):
+        k = int(rng.integers(1, kmax + 1))
+        row = []
+        weights = np.ones(k) if uniform else rng.integers(1, 6, size=k).astype(float)
+        for f in range(k):
+            ar = int(rng.integers(0, min(amax, n) + 1))
+            ins = sorted(rng.choice(n, size=ar, replace=False).tolist())
+            table = int(rng.integers(0, 1 << min(1 << ar, 62))) | (int(rng.integers(0, 1 << 62)) << 62 if ar > 5 else 0)
+            table &= (1 << (1 << ar)) - 1
+            if ar >= 7:   # keep the expression strings of wide predictors short: few minterms
+                table = 0
+                for a in rng.integers(0, 1 << ar, size=5):
+                    table |= 1 << int(a)
+            row.append((_sop([genes[j] for j in ins], table), float(weights[f] / weights.sum())))
+        exprs.append(row)
+    return genes, exprs
+
+
+def make_attractors(n, count, seed):
+    rng = np.random.default_rng(seed)
+    out = []
+    for a in range(count):
+        states = []
+        for _ in range(int(rng.integers(1, 4))):
+            s = [int(v) for v in rng.integers(0, 2, size=n)]
+            if a % 2 and n > 2:
+                for j in rng.choice(n, size=min(2, n), replace=False):
+                    s[int(j)] = "*"
+            states.append(tuple(s))
+        out.append(states)
+    return out
+
+
+CASES = [
+    # n, kmax, amax, bins, uniform, kernels
+    (1, 3, 1, 1, True, ("sliced", "scalar")),
+    (2, 4, 2, 3, True, ("sliced", "scalar")),
+    (31, 3, 4, 3, True, ("sliced", "scalar")),
+    (32, 4, 5, 8, True, ("sliced", "scalar")),
+    (33, 2, 6, 2, True, ("sliced", "scalar")),
+    (64, 3, 4, 3, True, ("sliced", "scalar")),
+    (65, 3, 4, 3, True, ("sliced", "scalar")),
+    (96, 2, 3, 4, True, ("sliced", "scalar")),
+    (97, 3, 3, 3, True, ("scalar",)),           # more than 96 genes: general kernel only
+    (128, 2, 4, 5, True, ("scalar",)),
+    (20, 5, 3, 3, False, ("sliced", "scalar")),  # five predictors, real selection probabilities: third selection plane
+    (26, 8, 4, 3, True, ("sliced", "scalar")),   # up to eight predictors, uniform
+    (12, 9, 3, 3, True, ("scalar",)),            # more than eight predictors: general kernel only
+    (24, 2, 9, 3, False, ("sliced", "scalar")),  # wide predictors (7..9 inputs), weighted selection
+    (40, 3, 12, 3, True, ("sliced", "scalar")),  # up to 12 inputs, two-word states
+    (20, 2, 14, 3, True, ("scalar",)),           # more than 12 inputs: general kernel only
+]

@@ -162,3 +162,29 @@ def test_per_instance_env_protocol():
     assert env.in_target(env.render())  # wildcard positions 4,5
     s2, r, term, trunc, _ = env.step([])  # uncontrolled step inside the wildcard attractor stays inside
     assert term and r == 5.0
+
+
+@pytest.mark.parametrize("name", ["pbn28", "pbn70"])
+@pytest.mark.parametrize("bins", [1, 3, 8])
+def test_batched_step_ignores_action_bytes_above_n(name, bins):
+    """The batched flip mask equals the per-instance one for action bytes 0..255: 0 and bytes above N are no-ops,
+    repeats flip once, and only the flipped genes are charged r_action."""
+    onet = oracle_net(name)
+    n, w, e = onet.n, onet.words, 512
+    rng = np.random.default_rng(bins)
+    acts = rng.integers(0, 256, size=(e, bins)).astype(np.uint8)
+    acts[::4] = rng.integers(0, n + 2, size=(len(acts[::4]), bins))
+    acts[1::4, 0] = n
+    acts[2::4] = acts[2::4, :1]
+    words = k4_inputs(n)[:e]
+    sel = np.zeros((e, n), dtype=np.uint8)
+    nxt, _, rew, _, _ = O.batched_step(onet, O.attractor_tables([], n), words, acts, np.full(e, -1), np.zeros(e),
+                                       horizon=0, mode=0, sel=sel, pert=np.zeros((e, w), dtype=np.uint64),
+                                       r_success=0.0, r_step=0.0, r_action=-1.0)
+    flip = np.zeros((e, w), dtype=np.uint64)
+    for i, row in enumerate(acts):
+        m = O.flip_mask_from_actions(row, n)
+        for wd in range(w):
+            flip[i, wd] = (m >> (64 * wd)) & 0xFFFFFFFFFFFFFFFF
+        assert rew[i] == -bin(m).count("1"), (i, row)
+    assert np.array_equal(nxt, onet.transition_batch(words, flip, sel, np.zeros_like(flip), 0))
