@@ -466,6 +466,36 @@ int pbn_closure_reach(pbn_handle* h, const uint64_t* list, int64_t count, uint8_
                       const unsigned long long* tags, const uint64_t* slot_state,
                       const unsigned long long* slot_index, int64_t capacity, int32_t* changed, void* stream);
 
+/* ---- Exact optimal control: finite-horizon dynamic programming over every state (N <= PBN_DP_MAX_GENES) ----------
+ * The env is a finite Markov decision process, so for networks whose 2^N states fit on the GPU the best possible policy
+ * of a target can be computed exactly by backward induction -- the yardstick an agent's strategy lengths and returns are
+ * compared against.  States are indices s in [0, 2^N) (bit i = gene i); a flip mask m is a subset of the controllable
+ * genes with popcount(m) <= max_flips; one env step from s with mask m starts from u = s ^ m and draws t ~ P(u -> .),
+ * P = items 2-4 of "One env step" above with the handle's perturbation model and perturb_p.  A backup is
+ *   W = P U (pbn_dp_expect),   V(s) = max_m fl(r_action |m|) + W[s ^ m] (pbn_dp_improve),
+ * the rest (rewards, discount, target and wrong-attractor terms) is elementwise work of the caller
+ * (pbn_rl_b200/control.py).  Perturbation: NONE: P = F (the selection step); B: P = F K_p; A: P = (1-p)^N F +
+ * K_p - (1-p)^N I, K_p = the per-gene binary symmetric channel (a perturbed step skips the update and lands on
+ * u ^ pert, pert != 0); model C with p > 0 makes nearly every gene free in every state (a backup of O(4^N)) and is
+ * refused; any model with p = 0 is NONE.
+ * Both calls run on the caller's stream without synchronising or allocating, in launches of at most 2^22 states, and
+ * are deterministic: the same inputs give bit-identical outputs (no floating-point atomics). */
+#define PBN_DP_MAX_GENES 28
+/* Bytes of caller-owned DEVICE workspace the two calls below need for this handle (24 * 2^N), or a negative status:
+ * PBN_ERR_UNSUPPORTED when N > PBN_DP_MAX_GENES or the perturbation model is C with p > 0. */
+int64_t pbn_dp_workspace_bytes(const pbn_handle* h);
+/* w[u] = sum_t P(u -> t) u_in[t] for every u in [0, 2^N)  (fp64, DEVICE arrays of 2^N; w must not alias u_in).  P: one
+ * step of the handle's dynamics without interventions -- predictor selection with probabilities func_prob (DEVICE fp64
+ * [F], the network's selection probabilities in func_offset order; not validated), then the handle's perturbation model
+ * at perturb_p.  workspace: pbn_dp_workspace_bytes (may be NULL when p = 0). */
+int pbn_dp_expect(pbn_handle* h, const double* func_prob, const double* u_in, double* w, void* workspace, void* stream);
+/* v[s] = max over masks m with m subset of flip_genes and popcount(m) <= max_flips of  fl(r_action * popcount(m)) +
+ * w[s ^ m] (no FMA); policy[s] = that m (may be NULL).  Ties: fewer flips, then larger w[s ^ m], then smaller s ^ m.
+ * r_action <= 0, 0 <= max_flips <= PBN_MAX_BINS, flip_genes within the N genes, else PBN_ERR_INVALID.  v must not alias
+ * w; workspace (pbn_dp_workspace_bytes) may be NULL when max_flips <= 1. */
+int pbn_dp_improve(pbn_handle* h, const double* w, uint64_t flip_genes, int32_t max_flips, double r_action,
+                   double* v, uint32_t* policy, void* workspace, void* stream);
+
 /* *step_ctr_dev += n on the stream (fully serialised): closes a sequence of PBN_STEP_PDL launches. */
 int pbn_advance_counter(pbn_handle* h, uint64_t* step_ctr_dev, uint64_t n, void* stream);
 

@@ -13,7 +13,10 @@ __all__ = [
     "AttractorSet", "find_attractors_stg", "load_attractor_pickle", "save_attractor_pickle",
     "sorted_id_permutation", "BoolFunction", "IsplError", "compile_expression", "logic_functions_from_ispl",
     "parse_ispl", "render_ispl", "PBNNetwork", "pack_states", "unpack_states", "VecPBNEnv",
+    "solve_control", "ControlSolution", "TabularPolicy", "policy_values", "tabulate_policy", "expected_all_pairs",
 ]
+
+_CONTROL = ("solve_control", "ControlSolution", "TabularPolicy", "policy_values", "tabulate_policy", "expected_all_pairs")
 
 
 def __getattr__(name):
@@ -24,4 +27,7 @@ def __getattr__(name):
     if name in ("PBNEnv", "ControlPBNEnv", "make", "register_gym_ids"):
         from . import gym_env
         return getattr(gym_env, name)
+    if name in _CONTROL:
+        from . import control
+        return getattr(control, name)
     raise AttributeError(name)

@@ -15,6 +15,9 @@ __all__ = ["lib", "load_library", "PbnError", "NetDesc", "StepArgs", "HostIO", "
 LIB_PATH = Path(__file__).resolve().parent / "libpbn_b200.so"
 
 PBN_OK = 0
+PBN_ERR_INVALID = -1
+PBN_ERR_UNSUPPORTED = -3
+DP_MAX_GENES = 28  # PBN_DP_MAX_GENES
 PERT_MODES = {"none": 0, "A": 1, "B": 2, "C": 3}
 KERNEL_KINDS = {"auto": 0, "scalar": 1, "sliced": 2}
 STEP_AUTORESET = 1
@@ -36,6 +39,7 @@ EXPORTS = (
     "pbn_rollout", "pbn_rollout_record", "pbn_record_states",
     "pbn_resident_words", "pbn_resident_import", "pbn_resident_export", "pbn_reward_table", "pbn_attractor_hash_slots",
     "pbn_per_tree_floats", "pbn_per_init", "pbn_per_push", "pbn_per_update", "pbn_per_sample",
+    "pbn_dp_workspace_bytes", "pbn_dp_expect", "pbn_dp_improve",
 )
 
 
@@ -185,6 +189,12 @@ def load_library(path: Optional[os.PathLike] = None) -> C.CDLL:
     lib.pbn_per_update.restype = C.c_int
     lib.pbn_per_sample.argtypes = [vp, C.POINTER(Per), vp, i64, C.c_float, vp, vp, vp]
     lib.pbn_per_sample.restype = C.c_int
+    lib.pbn_dp_workspace_bytes.argtypes = [vp]
+    lib.pbn_dp_workspace_bytes.restype = i64
+    lib.pbn_dp_expect.argtypes = [vp, vp, vp, vp, vp, vp]
+    lib.pbn_dp_expect.restype = C.c_int
+    lib.pbn_dp_improve.argtypes = [vp, vp, u64, i32, C.c_double, vp, vp, vp, vp]
+    lib.pbn_dp_improve.restype = C.c_int
     lib.pbn_observe.argtypes = [vp, vp, vp, vp, i64, vp]
     lib.pbn_observe.restype = C.c_int
     lib.pbn_in_target.argtypes = [vp, vp, vp, vp, i64, vp]

@@ -99,6 +99,27 @@ __global__ void __launch_bounds__(256) visit_count_kernel(const uint64_t* __rest
   }
 }
 
+// Value (0 or 1) of predictor function f in state s: the narrow 64-bit truth table or a wide one.  Shared by the
+// successor descriptor below and the exact backup of control.cuh, so both see the same predictor values.
+template <int W>
+__device__ __forceinline__ uint64_t eval_func(const NetParams& n, int f, const uint64_t (&s)[W]) {
+  const FuncDesc d = n.funcs[f];
+  uint64_t v;
+  if (d.in47 == kWideMarker) {
+    v = eval_wide<W>(n, d.lut_lo, s);
+  } else {
+    uint32_t idx = 0;
+#pragma unroll
+    for (int j = 0; j < 6; ++j) {
+      const uint32_t in = ((j < 4 ? d.in03 >> (8 * j) : d.in47 >> (8 * (j - 4))) & 0xFFu);
+      idx |= (uint32_t)((s[W == 1 ? 0 : (in >> 6)] >> (in & 63u)) & 1ull) << j;
+    }
+    const uint64_t lut = ((uint64_t)d.lut_hi << 32) | d.lut_lo;   // replicated over unused inputs
+    v = (lut >> idx) & 1ull;
+  }
+  return v;
+}
+
 // (can1, can0) of one state: which genes some predictor can set to 1 / to 0 in one perturbation-free update.
 template <int W>
 __device__ __forceinline__ void successor_descriptor(const NetParams& n, const uint64_t (&s)[W], uint64_t (&c1)[W],
@@ -107,20 +128,7 @@ __device__ __forceinline__ void successor_descriptor(const NetParams& n, const u
   for (int w = 0; w < W; ++w) { c1[w] = 0; c0[w] = 0; }
   for (int g = 0; g < n.n_genes; ++g) {
     for (int f = n.func_offset[g]; f < n.func_offset[g + 1]; ++f) {
-      const FuncDesc d = n.funcs[f];
-      uint64_t v;
-      if (d.in47 == kWideMarker) {
-        v = eval_wide<W>(n, d.lut_lo, s);
-      } else {
-        uint32_t idx = 0;
-#pragma unroll
-        for (int j = 0; j < 6; ++j) {
-          const uint32_t in = ((j < 4 ? d.in03 >> (8 * j) : d.in47 >> (8 * (j - 4))) & 0xFFu);
-          idx |= (uint32_t)((s[W == 1 ? 0 : (in >> 6)] >> (in & 63u)) & 1ull) << j;
-        }
-        const uint64_t lut = ((uint64_t)d.lut_hi << 32) | d.lut_lo;   // replicated over unused inputs
-        v = (lut >> idx) & 1ull;
-      }
+      const uint64_t v = eval_func<W>(n, f, s);
       c1[g >> 6] |= v << (g & 63);
       c0[g >> 6] |= (v ^ 1ull) << (g & 63);
     }

@@ -21,6 +21,7 @@
 #include "resident.cuh"
 #include "per.cuh"
 #include "record.cuh"
+#include "control.cuh"
 
 using namespace pbn;
 
@@ -96,6 +97,7 @@ struct pbn_handle {
   int W = 1;
   int kernel = PBN_KERNEL_SCALAR;
   int num_sms = 148;
+  double perturb_p = 0.0;   // the perturbation probability as given (exact control needs it in fp64)
   NetParams net{};
   // owned device tables
   int32_t* d_func_offset = nullptr;
@@ -592,6 +594,7 @@ int pbn_create(const pbn_net_desc* d, pbn_handle** out) {
   h->device = d->device;
   h->W = N <= 64 ? 1 : 2;
   h->kernel = kernel;
+  h->perturb_p = d->perturb_p;
   cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, d->device);
 
   int rc;
@@ -1610,6 +1613,110 @@ int pbn_attractor_id(pbn_handle* h, const uint64_t* state, int32_t* attr_id, int
     attractor_id_kernel<2><<<grid, 256, 0, stream>>>(h->net, state, attr_id, n_envs);
   PBN_CUDA(cudaGetLastError());
   h->launches += 1, g_last_advance = nullptr;
+  return PBN_OK;
+}
+
+// ---- exact optimal control (control.cuh) ----
+static constexpr uint32_t kDpSliceStates = 1u << 22;   // states (or state pairs) per launch
+
+// The perturbation model a backup applies: PBN_PERT_NONE whenever p = 0; model C with p > 0 is refused.
+static int dp_model(const pbn_handle* h, const char* who, int* model) {
+  if (!h) return fail(PBN_ERR_INVALID, "%s: null handle", who);
+  if (h->net.n_genes > PBN_DP_MAX_GENES)
+    return fail(PBN_ERR_UNSUPPORTED, "%s: %d genes, exact control covers at most %d", who, h->net.n_genes, PBN_DP_MAX_GENES);
+  *model = h->perturb_p > 0.0 ? h->net.pert_mode : PBN_PERT_NONE;
+  if (*model == PBN_PERT_C)
+    return fail(PBN_ERR_UNSUPPORTED, "%s: perturbation model C with p > 0 makes every gene free (a backup of O(4^N))", who);
+  return PBN_OK;
+}
+
+int64_t pbn_dp_workspace_bytes(const pbn_handle* h) {
+  int model, rc;
+  if ((rc = dp_model(h, "pbn_dp_workspace_bytes", &model)) != PBN_OK) return rc;
+  return (int64_t)24 << h->net.n_genes;   // two (fp64 value, u32 endpoint) buffers of the relaxation; expect uses the first
+}
+
+int pbn_dp_expect(pbn_handle* h, const double* func_prob, const double* u_in, double* w, void* workspace, void* stream_) {
+  int model, rc;
+  if ((rc = dp_model(h, "pbn_dp_expect", &model)) != PBN_OK) return rc;
+  if (!func_prob || !u_in || !w) return fail(PBN_ERR_INVALID, "pbn_dp_expect: null array");
+  if (u_in == w) return fail(PBN_ERR_INVALID, "pbn_dp_expect: w must not alias u_in");
+  if (model != PBN_PERT_NONE && !workspace) return fail(PBN_ERR_INVALID, "pbn_dp_expect: perturbation needs the workspace");
+  const int N = h->net.n_genes;
+  const uint32_t S = 1u << N;
+  const double p = h->perturb_p;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  double* kpu = static_cast<double*>(workspace);
+  if (model != PBN_PERT_NONE) {   // kpu = K_p u_in: low genes tile by tile in shared memory, then one pass per higher gene
+    const int tb = N < kKpTileBits ? N : kKpTileBits;
+    const uint32_t tiles = S >> tb, per = kDpSliceStates >> tb;
+    for (uint32_t t0 = 0; t0 < tiles; t0 += per) {
+      const uint32_t nt = tiles - t0 < per ? tiles - t0 : per;
+      dp_kp_low_kernel<<<grid_for(h, (int64_t)nt * 256, 256, 8), 256, 0, stream>>>(u_in, kpu, tb, t0, nt, p);
+      PBN_CUDA(cudaGetLastError());
+      h->launches += 1;
+    }
+    for (int b = tb; b < N; ++b)
+      for (uint32_t j0 = 0; j0 < S / 2; j0 += kDpSliceStates) {
+        const uint32_t cnt = S / 2 - j0 < kDpSliceStates ? S / 2 - j0 : kDpSliceStates;
+        dp_kp_bit_kernel<<<grid_for(h, cnt, 256, 8), 256, 0, stream>>>(kpu, b, j0, cnt, p);
+        PBN_CUDA(cudaGetLastError());
+        h->launches += 1;
+      }
+  }
+  const double c = std::pow(1.0 - p, (double)N);
+  for (uint32_t s0 = 0; s0 < S; s0 += kDpSliceStates) {
+    const uint32_t cnt = S - s0 < kDpSliceStates ? S - s0 : kDpSliceStates;
+    dp_expect_kernel<<<grid_for(h, (int64_t)cnt * 32, kDpWarps * 32, 8), kDpWarps * 32, 0, stream>>>(
+        h->net, func_prob, model == PBN_PERT_B ? kpu : u_in, w, s0, cnt);
+    PBN_CUDA(cudaGetLastError());
+    h->launches += 1;
+    if (model == PBN_PERT_A) {
+      dp_mix_kernel<<<grid_for(h, cnt, 256, 8), 256, 0, stream>>>(w, kpu, u_in, c, s0, cnt);
+      PBN_CUDA(cudaGetLastError());
+      h->launches += 1;
+    }
+  }
+  g_last_advance = nullptr;
+  return PBN_OK;
+}
+
+int pbn_dp_improve(pbn_handle* h, const double* w, uint64_t flip_genes, int32_t max_flips, double r_action, double* v,
+                   uint32_t* policy, void* workspace, void* stream_) {
+  if (!h) return fail(PBN_ERR_INVALID, "pbn_dp_improve: null handle");
+  const int N = h->net.n_genes;
+  if (N > PBN_DP_MAX_GENES)
+    return fail(PBN_ERR_UNSUPPORTED, "pbn_dp_improve: %d genes, exact control covers at most %d", N, PBN_DP_MAX_GENES);
+  if (!w || !v) return fail(PBN_ERR_INVALID, "pbn_dp_improve: null array");
+  if (w == v) return fail(PBN_ERR_INVALID, "pbn_dp_improve: v must not alias w");
+  if (!(r_action <= 0.0)) return fail(PBN_ERR_INVALID, "pbn_dp_improve: r_action=%g must be <= 0", r_action);
+  if (max_flips < 0 || max_flips > PBN_MAX_BINS) return fail(PBN_ERR_INVALID, "pbn_dp_improve: max_flips=%d outside 0..%d", max_flips, PBN_MAX_BINS);
+  if (flip_genes >> N) return fail(PBN_ERR_INVALID, "pbn_dp_improve: flip_genes has genes beyond the %d of the network", N);
+  if (max_flips >= 2 && !workspace) return fail(PBN_ERR_INVALID, "pbn_dp_improve: max_flips >= 2 needs the workspace");
+  const uint32_t S = 1u << N;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  // ping-pong buffers of the relaxation: values [2][S] fp64, then endpoints [2][S] u32
+  double* bv[2] = {static_cast<double*>(workspace), workspace ? static_cast<double*>(workspace) + S : nullptr};
+  uint32_t* be[2] = {workspace ? reinterpret_cast<uint32_t*>(static_cast<double*>(workspace) + 2 * (size_t)S) : nullptr,
+                     workspace ? reinterpret_cast<uint32_t*>(static_cast<double*>(workspace) + 2 * (size_t)S) + S : nullptr};
+  const double cost0 = r_action * 0.0;
+  for (int k = max_flips == 0 ? 0 : 1; k <= max_flips; ++k) {
+    const double* ival = k >= 2 ? bv[k & 1] : nullptr;        // B_{k-1}: w itself for k = 1
+    const uint32_t* iend = k >= 2 ? be[k & 1] : nullptr;
+    double* oval = k < max_flips ? bv[(k + 1) & 1] : nullptr;  // B_k, unless this is the last pass
+    uint32_t* oend = k < max_flips ? be[(k + 1) & 1] : nullptr;
+    const double cost_k = r_action * (double)k;
+    for (uint32_t s0 = 0; s0 < S; s0 += kDpSliceStates) {
+      const uint32_t cnt = S - s0 < kDpSliceStates ? S - s0 : kDpSliceStates;
+      dp_improve_kernel<<<grid_for(h, cnt, 256, 8), 256, 0, stream>>>(w, ival, iend, oval, oend, v, policy,
+                                                                      (uint32_t)flip_genes, k, cost0, cost_k, s0, cnt);
+      PBN_CUDA(cudaGetLastError());
+      h->launches += 1;
+    }
+  }
+  g_last_advance = nullptr;
   return PBN_OK;
 }
 

@@ -157,6 +157,8 @@ class VecPBNEnv:
         self.step_ctr = 0
         self.perturb_p = float(perturb_p)
         self.perturb_mode = perturb_mode
+        self.r_success, self.r_step, self.r_action = float(r_success), float(r_step), float(r_action)
+        self.r_wrong = float(r_wrong)
 
         d, self._keep = make_desc(network, bins=self.bins, horizon=self.horizon, perturb_p=self.perturb_p,
                                   perturb_mode=perturb_mode, r_success=r_success, r_step=r_step,
