@@ -8,7 +8,10 @@ pbn_rl_b200/control.py) for small networks, written from the step contract rathe
 - the maximum over flip sets by brute-force enumeration of every allowed mask with the contract's tie order (fewer
   flips, then larger w[s ^ m], then smaller s ^ m);
 - the finite-horizon recursion of both objectives ("return", "steps").
-Test infrastructure only; N <= 12 for the dense forms.
+Test infrastructure only; N <= 12 for the dense forms.  The sampled forms scale to N = 28: sparse_expect enumerates
+a state's successor set in chunks and gathers u through a formula (u_hash, w_ties, w_rounding) where no 2^N vector
+is wanted, kp_tensor applies the perturbation channel gene by gene (N <= 24), and improve_brute_states /
+classify_states evaluate the brute force and the classification at listed states only.
 """
 import itertools
 
@@ -106,22 +109,125 @@ def expect(onet, u, mode="none", p=0.0, f=None):
     return f @ ku
 
 
-def sparse_expect(onet, u, states):
-    """(F u)(x) for the listed states by enumerating each state's successor set (p = 0; any N up to ~20)."""
-    q = gene_probabilities(onet, states)
-    u = np.asarray(u, dtype=np.float64)
+def gene_split(net, states):
+    """(q1, q0) [len(states), N]: the summed selection probabilities of gene i's predictors that yield 1 / yield 0 in
+    each listed state.  Gene i is free where both are > 0, fixed to 1 where q0 = 0 and fixed to 0 where q1 = 0."""
+    n = n_genes(net)
+    xs = np.asarray(states, dtype=np.int64)
+    q1 = np.zeros((xs.size, n), dtype=np.float64)
+    q0 = np.zeros((xs.size, n), dtype=np.float64)
+    if hasattr(net, "np_code"):
+        ns = {g: ((xs >> i) & 1).astype(bool) for i, g in enumerate(net.genes)}
+        for i in range(n):
+            for code, p in zip(net.np_code[i], net.probs[i]):
+                v = np.broadcast_to(np.asarray(eval(code, {}, ns), dtype=bool), xs.shape)
+                q1[:, i] += np.where(v, p, 0.0)
+                q0[:, i] += np.where(v, 0.0, p)
+        return q1, q0
+    for i, (fs, ps) in enumerate(zip(net.functions, net.probabilities)):
+        for f, p in zip(fs, ps):
+            idx = np.zeros(xs.size, dtype=np.int64)
+            for j, g in enumerate(f.inputs):
+                idx |= ((xs >> g) & 1) << j
+            tab = np.array([(f.lut >> a) & 1 for a in range(1 << f.arity)], dtype=bool)
+            v = tab[idx]
+            q1[:, i] += np.where(v, p, 0.0)
+            q0[:, i] += np.where(v, 0.0, p)
+    return q1, q0
+
+
+def free_counts(net, states):
+    """Number of free genes (predictors yielding both values) of each listed state: log2 of its successor count."""
+    q1, q0 = gene_split(net, states)
+    return ((q1 > 0.0) & (q0 > 0.0)).sum(axis=1)
+
+
+def _gather(u, idx):
+    return u(idx) if callable(u) else np.asarray(u, dtype=np.float64)[idx]
+
+
+def _successors(genes, q1, q0, base):
+    """Indices and weights of every assignment of ``genes`` (lowest gene = lowest bit of the enumeration order)."""
+    t = np.full(1, base, dtype=np.int64)
+    wt = np.ones(1)
+    for i in genes:
+        t = np.concatenate([t, t | (1 << int(i))])
+        wt = np.concatenate([wt * q0[i], wt * q1[i]])
+    return t, wt
+
+
+def sparse_expect(onet, u, states, chunk_bits=20):
+    """(F u)(x) for the listed states by enumerating each state's successor set (p = 0).  ``u``: an array over all
+    states or a callable ``u(indices int64) -> float64``, so that nothing of size 2^N is built.  The lowest
+    ``chunk_bits`` free genes of a state are enumerated as one vector of at most 2^chunk_bits successors; the higher
+    free genes run in an outer loop, so a state of 28 free genes is 2^(28 - chunk_bits) gathers of 2^chunk_bits."""
+    q1, q0 = gene_split(onet, states)
+    n = n_genes(onet)
     out = np.zeros(len(states))
     for r in range(len(states)):
-        n = n_genes(onet)
-        free = [i for i in range(n) if 0.0 < q[r, i] < 1.0]
-        fixed = sum(1 << i for i in range(n) if q[r, i] >= 1.0)
-        t = np.full(1, fixed, dtype=np.int64)
-        wt = np.ones(1)
-        for i in free:
-            t = np.concatenate([t, t | (1 << i)])
-            wt = np.concatenate([wt * (1.0 - q[r, i]), wt * q[r, i]])
-        out[r] = float(np.dot(wt, u[t]))
+        free = [i for i in range(n) if q1[r, i] > 0.0 and q0[r, i] > 0.0]
+        fixed = sum(1 << i for i in range(n) if q0[r, i] == 0.0)
+        lo, hi = free[:chunk_bits], free[chunk_bits:]
+        t_lo, w_lo = _successors(lo, q1[r], q0[r], fixed)
+        t_hi, w_hi = _successors(hi, q1[r], q0[r], 0)
+        acc = 0.0
+        for th, wh in zip(t_hi, w_hi):
+            acc += wh * float(np.dot(w_lo, _gather(u, t_lo | th)))
+        out[r] = acc
     return out
+
+
+# ---- formula inputs: exact integer formulas evaluated where they are gathered (torch on the device, numpy here) ----
+_GOLD32 = 0x9E3779B1
+
+
+def hash32(t):
+    """(t * 0x9E3779B1) mod 2^32 for int64 indices t < 2^31 (exact: the product stays below 2^63)."""
+    return (t * _GOLD32) & 0xFFFFFFFF
+
+
+def u_hash(t):
+    """u(t) = hash32(t) 2^-32 - 0.5: fp64-exact values in [-0.5, 0.5) (numpy int64 array or torch int64 tensor)."""
+    h = hash32(t)
+    return (h.astype(np.float64) if isinstance(h, np.ndarray) else h.double()) * 2.0 ** -32 - 0.5
+
+
+def w_ties(t):
+    """hash mod 4: values 0..3 with many exact ties."""
+    h = hash32(t) % 4
+    return h.astype(np.float64) if isinstance(h, np.ndarray) else h.double()
+
+
+def w_rounding(t):
+    """1e16 + 2 (hash mod 3): r_action k of order 1 is lost in the rounding of fl(r_action k) + w."""
+    h = hash32(t) % 3
+    return 1e16 + 2.0 * (h.astype(np.float64) if isinstance(h, np.ndarray) else h.double())
+
+
+# ---- the perturbation channel over all states, for N <= 24 ----------------------------------------------------------
+def kp_tensor(u, p):
+    """(K_p u) over all 2^N states as a tensor product: one 2x2 contraction [[1-p, p], [p, 1-p]] per gene axis."""
+    v = np.array(u, dtype=np.float64)
+    n = v.size.bit_length() - 1
+    q = 1.0 - p
+    for i in range(n):
+        x = v.reshape(-1, 2, 1 << i)
+        a, z = x[:, 0, :].copy(), x[:, 1, :].copy()
+        x[:, 0, :] = q * a + p * z
+        x[:, 1, :] = q * z + p * a
+    return v
+
+
+def kp_direct(u, states, p):
+    """(K_p u)(x) = sum over every perturbation mask m of p^|m| (1-p)^(N-|m|) u[x ^ m], at the listed states."""
+    u = np.asarray(u, dtype=np.float64)
+    n = u.size.bit_length() - 1
+    m = np.arange(1 << n, dtype=np.int64)
+    pc = np.zeros(m.size, dtype=np.int64)
+    for i in range(n):
+        pc += (m >> i) & 1
+    pm = (p ** pc) * ((1.0 - p) ** (n - pc))
+    return np.array([float(np.dot(pm, u[int(x) ^ m])) for x in states])
 
 
 def masks_of(flip_genes, max_flips):
@@ -157,6 +263,30 @@ def improve_brute(w, flip_genes, max_flips, r_action):
     return best_v, (best_e ^ s).astype(np.int64)
 
 
+def improve_brute_states(w, states, flip_genes, max_flips, r_action):
+    """improve_brute evaluated only at the listed states: each state's allowed masks enumerated, ``w`` an array over
+    all states or a callable on int64 indices.  Returns (v, policy) at those states."""
+    s = np.asarray(states, dtype=np.int64)
+    masks = np.asarray(masks_of(flip_genes, max_flips), dtype=np.int64)
+    ends = s[:, None] ^ masks[None, :]
+    wall = _gather(w, ends.ravel()).reshape(ends.shape)
+    best_v = np.full(s.size, -np.inf)
+    best_k = np.zeros(s.size, dtype=np.int64)
+    best_w = np.full(s.size, -np.inf)
+    best_e = np.zeros(s.size, dtype=np.int64)
+    for j, m in enumerate(masks):
+        k = bin(int(m)).count("1")
+        e, we = ends[:, j], wall[:, j]
+        val = np.float64(r_action) * np.float64(k) + we
+        better = (val > best_v) | ((val == best_v) & ((k < best_k) | ((k == best_k) & ((we > best_w) |
+                                                                                        ((we == best_w) & (e < best_e))))))
+        best_v = np.where(better, val, best_v)
+        best_k = np.where(better, k, best_k)
+        best_w = np.where(better, we, best_w)
+        best_e = np.where(better, e, best_e)
+    return best_v, best_e ^ s
+
+
 def improve_ball(w, flip_genes, max_flips, r_action):
     """The device's rule restated: B_0 = (w[s], s), B_k = best of B_{k-1} over s and its one-flip neighbours (larger
     value, then smaller endpoint); the candidate fl(r_action k) + B_k replaces the incumbent only when strictly larger."""
@@ -183,8 +313,13 @@ def improve_ball(w, flip_genes, max_flips, r_action):
 
 def classify(onet_n, attractors, target):
     """(hit, wrong) over all states: in the target attractor; in another attractor and not in the target."""
+    return classify_states(onet_n, attractors, target, np.arange(1 << onet_n))
+
+
+def classify_states(onet_n, attractors, target, states):
+    """classify restricted to the listed states."""
     offs, care, val = O.attractor_tables(attractors, onet_n)
-    s = np.arange(1 << onet_n, dtype=np.uint64)
+    s = np.asarray(states, dtype=np.int64).astype(np.uint64)
     inside = []
     for a in range(len(offs) - 1):
         h = np.zeros(s.size, dtype=bool)

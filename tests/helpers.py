@@ -127,6 +127,34 @@ def make_network(n, kmax, amax, seed, uniform=True):
     return genes, exprs
 
 
+def window_network(n, k, seed):
+    """A network whose free-gene count per state is set by the state: gene i has the copy predictor x_i and
+    x_i XOR (x_{i+1} & ... & x_{i+k}) (indices mod n), with seeded unequal selection probabilities.  Gene i is free
+    exactly when its window of k genes is all ones; otherwise both predictors keep x_i.  So a state whose ones form one
+    cyclic run of length L >= k (L < n) has L - k + 1 free genes, the all-ones state has n, and the total successor
+    count sum_x 2^free(x) is the trace of the n-th power of a 2^k-state transfer matrix.  k = 6 makes 7-input
+    (wide) predictors."""
+    rng = np.random.default_rng(seed)
+    genes = ["x%d" % i for i in range(n)]
+    exprs = []
+    for i in range(n):
+        win = " & ".join(genes[(i + j) % n] for j in range(1, k + 1))
+        xor = "( %s & ~ ( %s ) ) | ( ~ %s & ( %s ) )" % (genes[i], win, genes[i], win)
+        p = float(rng.uniform(0.15, 0.85))
+        while abs(p - 0.5) < 0.05:
+            p = float(rng.uniform(0.15, 0.85))
+        exprs.append([(genes[i], p), (xor, 1.0 - p)])
+    return genes, exprs
+
+
+def run_state(n, start, length):
+    """The state whose ones are the cyclic run of ``length`` genes from gene ``start`` (indices mod n)."""
+    s = 0
+    for j in range(length):
+        s |= 1 << ((start + j) % n)
+    return s
+
+
 def make_attractors(n, count, seed):
     rng = np.random.default_rng(seed)
     out = []
