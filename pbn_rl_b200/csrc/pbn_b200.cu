@@ -120,26 +120,23 @@ struct pbn_handle {
   uint32_t* d_surv_sliced = nullptr;
   WideDesc* d_wide = nullptr;
   uint64_t* d_wide_lut = nullptr;
-  // sliced kernel: [0] = own-RNG specialisation, [1] = injected-randomness one (compiled on first use)
+  // sliced kernel: the network's JIT programs (kJitParts), [part][0 = own-RNG, 1 = injected randomness], each loaded
+  // on first use
   jit::GenNet gen;
-  cudaLibrary_t jit_lib[2] = {nullptr, nullptr};
-  cudaLibrary_t jit_lib_planes[2] = {nullptr, nullptr};   // the plane-resident kernels' program, loaded on first use
-  std::string jit_key[2], jit_key_planes[2];               // shared-module registry keys (release_module)
-  cudaKernel_t jit_kernel[2] = {nullptr, nullptr};      // pbn_step_sliced (attractor table in shared memory)
-  cudaKernel_t jit_kernel_gen[2] = {nullptr, nullptr};  // pbn_step_sliced_gen (hash set / global table / r_wrong)
-  cudaKernel_t planes_kernel[2][2] = {{nullptr, nullptr}, {nullptr, nullptr}};  // [injected][0: 4 warps, 1: 8 warps] pbn_step_planes_w*
-  uint32_t planes_smem_opt_in[2][2] = {{48u * 1024u, 48u * 1024u}, {48u * 1024u, 48u * 1024u}};
-  cudaKernel_t rollout_kernel = nullptr;  // pbn_rollout_sliced<false>
-  uint32_t rollout_smem_opt_in = 48u * 1024u;
-  cudaLibrary_t jit_lib_record = nullptr;  // the recording rollout's program, loaded on first use
-  std::string jit_key_record;
-  cudaKernel_t record_kernel = nullptr;   // pbn_rollout_sliced<true>
-  uint32_t record_smem_opt_in = 48u * 1024u;
+  struct JitKernel {
+    cudaKernel_t k = nullptr;
+    uint32_t smem_opt_in = 48u * 1024u;   // ensure_dynamic_smem's cache
+  };
+  struct JitProgram {
+    cudaLibrary_t lib = nullptr;
+    std::string key;         // shared-module registry key (release_module)
+    JitKernel kernel[3];     // in the order of kJitParts[part].kernels
+  };
+  JitProgram jit[3][2];
   std::vector<uint32_t> surv_sliced_host;  // copied into every loaded specialisation's constant memory
   int sliced_threads = 128, sliced_min_blocks = 1;
-  uint32_t jit_smem_opt_in[2][2] = {{48u * 1024u, 48u * 1024u}, {48u * 1024u, 48u * 1024u}};  // [injected][gen]
+  uint32_t scalar_smem_opt_in = 48u * 1024u;   // step_scalar_kernel (one instance per handle)
   uint64_t launches = 0;
-  bool scalar_smem_opted = false;
   // pbn_step_host: one stream and one join event per lane (created on first use)
   static constexpr int kMaxLanes = 16;
   cudaStream_t s_lane[kMaxLanes] = {};
@@ -226,54 +223,126 @@ static void release_module(const std::string& key) {
 
 // Dynamic shared memory above 48 KB must be opted into per kernel -- and the kernels are shared between handles, so the
 // handle's cached value is only a shortcut: the kernel's own attribute decides, and it is only ever raised.
-static int ensure_dynamic_smem(cudaKernel_t k, uint32_t bytes, uint32_t* cached) {
+static int ensure_dynamic_smem(const void* k, uint32_t bytes, uint32_t* cached) {
   if (bytes <= *cached) return PBN_OK;
   cudaFuncAttributes fa{};
-  PBN_CUDA(cudaFuncGetAttributes(&fa, reinterpret_cast<const void*>(k)));
+  PBN_CUDA(cudaFuncGetAttributes(&fa, k));
   uint32_t cur = fa.maxDynamicSharedSizeBytes > 0 ? (uint32_t)fa.maxDynamicSharedSizeBytes : 0u;
   if (cur < 48u * 1024u) cur = 48u * 1024u;
   if (bytes > cur) {
-    PBN_CUDA(cudaFuncSetAttribute(reinterpret_cast<const void*>(k), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
+    PBN_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes));
     cur = bytes;
   }
   *cached = cur;
   return PBN_OK;
 }
 
-// Compile (or fetch from the cubin cache) and load one specialisation of the sliced kernel.
-static int load_sliced(pbn_handle* h, int injected) {
-  if (h->jit_kernel[injected]) return PBN_OK;
-  std::vector<char> cubin;
-  std::string err;
-  if (jit::compile(h->gen, injected != 0, 0, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());
-  {
-    const int rc = acquire_module(h, cubin, !injected, &h->jit_lib[injected], &h->jit_key[injected]);
-    if (rc != PBN_OK) return rc;
+// Every kernel launch of the library goes through launch(), which counts it (pbn_launch_count) and applies the PDL
+// rule: a step launched with PBN_STEP_PDL reads *step_ctr_dev before its griddepcontrol.wait, and a primary grid's
+// writes are only guaranteed visible after the wait, so when the launch right before it is this handle's own
+// pbn_advance_counter, the step is launched fully serialised instead.
+template <typename Go>
+static int launch_with(pbn_handle* h, const void* k, unsigned grid, unsigned block, uint32_t smem, cudaStream_t stream,
+                       bool pdl, Go go) {
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(grid);
+  cfg.blockDim = dim3(block);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = stream;
+  cudaLaunchAttribute attr[1];
+  if (pdl && g_last_advance != h) {
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
   }
-  PBN_CUDA(cudaLibraryGetKernel(&h->jit_kernel[injected], h->jit_lib[injected], "pbn_step_sliced"));
-  PBN_CUDA(cudaLibraryGetKernel(&h->jit_kernel_gen[injected], h->jit_lib[injected], "pbn_step_sliced_gen"));
-  if (!injected) PBN_CUDA(cudaLibraryGetKernel(&h->rollout_kernel, h->jit_lib[0], jit::kRolloutKernel));
-  h->sliced_threads = jit::sliced_threads(h->gen);
-  h->sliced_min_blocks = jit::sliced_min_blocks(h->gen);
+  const cudaError_t e = go(&cfg);
+  if (e != cudaSuccess) {
+    const char* name = nullptr;
+    if (cudaFuncGetName(&name, k) != cudaSuccess || !name) name = "kernel";
+    cudaGetLastError();   // the error is returned here; a later check must not see it again
+    return fail(PBN_ERR_CUDA, "launch of %s (grid %u, block %u, %u B shared memory) failed: %s", name, grid, block, smem,
+                cudaGetErrorString(e));
+  }
+  h->launches += 1;
+  g_last_advance = nullptr;
   return PBN_OK;
 }
 
-// The plane-resident kernels' specialisation (own program, compiled / loaded on first use).
-static int load_planes(pbn_handle* h, int injected) {
-  if (h->planes_kernel[injected][0]) return PBN_OK;
+// A kernel of this library: the arguments are converted to the kernel's parameter types.
+template <typename... P, typename... A>
+static int launch(pbn_handle* h, void (*k)(P...), unsigned grid, unsigned block, uint32_t smem, cudaStream_t stream,
+                  bool pdl, A&&... args) {
+  return launch_with(h, reinterpret_cast<const void*>(k), grid, block, smem, stream, pdl,
+                     [&](const cudaLaunchConfig_t* cfg) { return cudaLaunchKernelEx(cfg, k, std::forward<A>(args)...); });
+}
+
+// A kernel of a JIT program.
+static int launch(pbn_handle* h, cudaKernel_t k, unsigned grid, unsigned block, uint32_t smem, cudaStream_t stream,
+                  bool pdl, void** args) {
+  const void* f = reinterpret_cast<const void*>(k);
+  return launch_with(h, f, grid, block, smem, stream, pdl,
+                     [&](const cudaLaunchConfig_t* cfg) { return cudaLaunchKernelExC(cfg, f, args); });
+}
+
+// The JIT programs of a network (jit::compile's `part`) and the kernels each one holds: [0] the own-RNG build, [1] the
+// injected-randomness one, each a list of kernel names ended by a null; an empty list means that build does not exist.
+// Parts 1 and 2 are separate programs so that an env that never uses one family never pays its compile time.
+enum { kPartRow = 0, kPartPlanes = 1, kPartRecord = 2, kParts = 3 };
+struct JitPart {
+  const char* kernels[2][3];
+  bool two_sel_planes;   // not built for networks with a third selection plane (genes with more than 4 predictors)
+};
+static const JitPart kJitParts[kParts] = {
+    // kPartRow: the row-format step (attractor table in shared memory / hash set, global table or r_wrong), pbn_rollout
+    {{{"pbn_step_sliced", "pbn_step_sliced_gen", jit::kRolloutKernel}, {"pbn_step_sliced", "pbn_step_sliced_gen"}}, false},
+    // kPartPlanes: the plane-resident step, 4 and 8 warps per tile
+    {{{"pbn_step_planes_w4", "pbn_step_planes_w8"}, {"pbn_step_planes_w4", "pbn_step_planes_w8"}}, true},
+    // kPartRecord: pbn_rollout_record
+    {{{jit::kRecordKernel}, {}}, false},
+};
+
+static bool part_exists(const jit::GenNet& g, int part, int injected) {
+  return kJitParts[part].kernels[injected][0] && !(kJitParts[part].two_sel_planes && jit::sel_bits(g) == 3);
+}
+
+// Compile (or fetch from the cubin cache) and load one program of the handle's network.
+static int load_program(pbn_handle* h, int part, int injected) {
+  pbn_handle::JitProgram& m = h->jit[part][injected];
+  if (m.lib) return PBN_OK;
   std::vector<char> cubin;
-  std::string err;
-  if (jit::compile(h->gen, injected != 0, 1, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());
-  {
-    const int rc = acquire_module(h, cubin, !injected, &h->jit_lib_planes[injected], &h->jit_key_planes[injected]);
-    if (rc != PBN_OK) return rc;
+  std::string err, key;
+  if (jit::compile(h->gen, injected != 0, part, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());
+  cudaLibrary_t lib = nullptr;
+  const int rc = acquire_module(h, cubin, !injected, &lib, &key);
+  if (rc != PBN_OK) return rc;
+  const char* const* names = kJitParts[part].kernels[injected];
+  for (int i = 0; i < 3 && names[i]; ++i) {
+    const cudaError_t e = cudaLibraryGetKernel(&m.kernel[i].k, lib, names[i]);
+    if (e != cudaSuccess) {
+      release_module(key);
+      return fail(PBN_ERR_CUDA, "cudaLibraryGetKernel(%s): %s", names[i], cudaGetErrorString(e));
+    }
   }
-  PBN_CUDA(cudaLibraryGetKernel(&h->planes_kernel[injected][1], h->jit_lib_planes[injected], "pbn_step_planes_w8"));
-  PBN_CUDA(cudaLibraryGetKernel(&h->planes_kernel[injected][0], h->jit_lib_planes[injected], "pbn_step_planes_w4"));
+  m.lib = lib;
+  m.key = key;
+  if (part == kPartRow) {
+    h->sliced_threads = jit::sliced_threads(h->gen);
+    h->sliced_min_blocks = jit::sliced_min_blocks(h->gen);
+  }
   return PBN_OK;
 }
 
-static SlicedSmemLayout sliced_smem_layout(const NetParams& n, int W, int warps, int scratch_words) {
+// Blocks of `block` threads (or tiles of `block` envs) over n, at most per_sm of them per SM.
+static int grid_for(const pbn_handle* h, int64_t n, int block, int per_sm) {
+  int64_t g = (n + block - 1) / block;
+  const int64_t cap = (int64_t)h->num_sms * per_sm;
+  if (g > cap) g = cap;
+  if (g < 1) g = 1;
+  return (int)g;
+}
+
+static SlicedSmemLayout sliced_smem_layout(const NetParams& n, int W, int scratch_words) {
   const uint32_t stage_state_bytes = 1024u * 8u * (uint32_t)W;
   const uint32_t stage_act_bytes = (1024u * (uint32_t)n.bins + 127u) & ~127u;
   SlicedSmemLayout L{};
@@ -306,7 +375,6 @@ static SlicedSmemLayout sliced_smem_layout(const NetParams& n, int W, int warps,
     o = (o + 15u) & ~15u;
   }
   L.scratch_off = o;
-  (void)warps;
   o += (uint32_t)scratch_words * 4u;  // one scratch per CTA (= per tile)
   o = (o + 127u) & ~127u;
   L.stage_state_off = o;
@@ -327,51 +395,16 @@ static int launch_sliced(pbn_handle* h, StepParams& p, bool injected, cudaStream
       !aligned_to(a.reward, 16) || !aligned_to(a.t, 8) || !aligned_to(a.actions, 16) ||
       !aligned_to(a.terminated, 4) || !aligned_to(a.truncated, 4))
     return fail(PBN_ERR_INVALID, "sliced kernel needs 16-byte aligned state/actions/target_id/reward, 8-byte t, 4-byte flags");
-  int rc = load_sliced(h, injected ? 1 : 0);
+  int rc = load_program(h, kPartRow, injected);
   if (rc != PBN_OK) return rc;
-  SlicedSmemLayout L = sliced_smem_layout(h->net, h->W, h->sliced_threads / 32, jit::scratch_words(h->gen));
+  SlicedSmemLayout L = sliced_smem_layout(h->net, h->W, jit::scratch_words(h->gen));
   if (L.total > 227u * 1024u) return fail(PBN_ERR_UNSUPPORTED, "sliced kernel needs %u B of shared memory", L.total);
-  const int gen = L.attractors_in_smem ? 0 : 1;
-  cudaKernel_t k = gen ? h->jit_kernel_gen[injected ? 1 : 0] : h->jit_kernel[injected ? 1 : 0];
-  if ((rc = ensure_dynamic_smem(k, L.total, &h->jit_smem_opt_in[injected ? 1 : 0][gen])) != PBN_OK) return rc;
+  pbn_handle::JitKernel& k = h->jit[kPartRow][injected].kernel[L.attractors_in_smem ? 0 : 1];
+  if ((rc = ensure_dynamic_smem(reinterpret_cast<const void*>(k.k), L.total, &k.smem_opt_in)) != PBN_OK) return rc;
   // one CTA per 1024-env tile; beyond a few waves the CTAs loop over tiles
-  int64_t grid = (a.n_envs + 1023) / 1024;
-  const int64_t cap = (int64_t)h->num_sms * h->sliced_min_blocks * 8;
-  if (grid > cap) grid = cap;
   void* args[] = {&p, &L};
-  // A PDL step reads *step_ctr_dev before its griddepcontrol.wait, and a primary grid's writes are only guaranteed
-  // visible after the wait: when the launch right before this one is this handle's own pbn_advance_counter, the step
-  // is launched fully serialised instead.
-  if ((a.flags & PBN_STEP_PDL) && g_last_advance != h) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3((unsigned)h->sliced_threads);
-    cfg.dynamicSmemBytes = L.total;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    PBN_CUDA(cudaLaunchKernelExC(&cfg, reinterpret_cast<const void*>(k), args));
-  } else {
-    PBN_CUDA(cudaLaunchKernel(reinterpret_cast<const void*>(k), dim3((unsigned)grid), dim3((unsigned)h->sliced_threads), args, L.total, stream));
-  }
-  return PBN_OK;
-}
-
-// The recording rollout's specialisation (own program, own-RNG only, compiled / loaded on first use).
-static int load_record(pbn_handle* h) {
-  if (h->record_kernel) return PBN_OK;
-  std::vector<char> cubin;
-  std::string err;
-  if (jit::compile(h->gen, false, 2, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());
-  {
-    const int rc = acquire_module(h, cubin, true, &h->jit_lib_record, &h->jit_key_record);
-    if (rc != PBN_OK) return rc;
-  }
-  PBN_CUDA(cudaLibraryGetKernel(&h->record_kernel, h->jit_lib_record, jit::kRecordKernel));
-  return PBN_OK;
+  return launch(h, k.k, grid_for(h, a.n_envs, 1024, h->sliced_min_blocks * 8), h->sliced_threads, L.total, stream,
+                a.flags & PBN_STEP_PDL, args);
 }
 
 // Which networks / attractor tables the plane-resident kernel takes (include/pbn_b200.h "Plane-resident env state").
@@ -392,16 +425,14 @@ static int launch_planes(pbn_handle* h, StepParams& p, bool injected, cudaStream
   if (rc != PBN_OK) return rc;
   if (!aligned_to(a.resident, 128) || !aligned_to(a.reward, 16) || !aligned_to(a.actions, 4) || !aligned_to(a.terminated, 4) || !aligned_to(a.truncated, 4))
     return fail(PBN_ERR_INVALID, "plane-resident step needs a 128-byte aligned block, 16-byte aligned reward, 4-byte aligned actions / flags");
-  if ((rc = load_planes(h, injected ? 1 : 0)) != PBN_OK) return rc;
+  if ((rc = load_program(h, kPartPlanes, injected)) != PBN_OK) return rc;
   const NetParams& n = h->net;
   const int N = n.n_genes, NW = (N + 31) / 32;
-  const int64_t tiles = (a.n_envs + 1023) / 1024;
   // 4 warps per tile (the selection planes stay in registers) for one-word states; 8 warps per tile where the
   // planes of a group would not fit the register file (N > 32: they are handed over through shared memory).  Both draw
   // the same streams.  (Measured with one shared code module per process, chained sequences: 3.69 vs 3.81 us per
   // 2^17-env step and 5.70 vs 6.51 us per 2^18-env step for 4 vs 8 warps.)
   int v = N > 32 ? 1 : 0;
-  (void)tiles;
   if (const char* env = getenv("PBN_B200_PLANES_WARPS")) v = atoi(env) == 8 ? 1 : 0;
   const int maxs4 = (jit::n_sel_slots(h->gen) + 3) / 4 > 0 ? (jit::n_sel_slots(h->gen) + 3) / 4 : 1;
   PlanesLayout L{};
@@ -422,32 +453,13 @@ static int launch_planes(pbn_handle* h, StepParams& p, bool injected, cudaStream
   }
   L.total = o;
   if (L.total > 227u * 1024u) return fail(PBN_ERR_UNSUPPORTED, "plane-resident kernel needs %u B of shared memory", L.total);
-  cudaKernel_t k = h->planes_kernel[injected ? 1 : 0][v];
-  if ((rc = ensure_dynamic_smem(k, L.total, &h->planes_smem_opt_in[injected ? 1 : 0][v])) != PBN_OK) return rc;
+  pbn_handle::JitKernel& k = h->jit[kPartPlanes][injected].kernel[v];
+  if ((rc = ensure_dynamic_smem(reinterpret_cast<const void*>(k.k), L.total, &k.smem_opt_in)) != PBN_OK) return rc;
   // One tile per CTA.  (CTAs that walk two tiles were the better form for tile-chained sequences while every handle ran
   // its own copy of the kernel code -- 7.1 vs 7.6 us per 2^17-env step; with the shared module one tile per CTA wins,
   // 3.8 vs 4.25 us.)
-  int64_t grid = tiles;
-  const int64_t cap = (int64_t)h->num_sms * 64;
-  if (grid > cap) grid = cap;
-  const unsigned threads = v ? 256u : 128u;
   void* args[] = {&p, &L};
-  if ((a.flags & PBN_STEP_PDL) && g_last_advance != h) {
-    cudaLaunchConfig_t cfg{};
-    cfg.gridDim = dim3((unsigned)grid);
-    cfg.blockDim = dim3(threads);
-    cfg.dynamicSmemBytes = L.total;
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    PBN_CUDA(cudaLaunchKernelExC(&cfg, reinterpret_cast<const void*>(k), args));
-  } else {
-    PBN_CUDA(cudaLaunchKernel(reinterpret_cast<const void*>(k), dim3((unsigned)grid), dim3(threads), args, L.total, stream));
-  }
-  return PBN_OK;
+  return launch(h, k.k, grid_for(h, a.n_envs, 1024, 64), v ? 256u : 128u, L.total, stream, a.flags & PBN_STEP_PDL, args);
 }
 
 extern "C" {
@@ -484,11 +496,8 @@ void pbn_destroy(pbn_handle* h) {
     cudaFree(h->d_surv_sliced);
     cudaFree(h->d_wide);
     cudaFree(h->d_wide_lut);
-    for (int i = 0; i < 2; ++i) {
-      release_module(h->jit_key[i]);
-      release_module(h->jit_key_planes[i]);
-    }
-    release_module(h->jit_key_record);
+    for (auto& part : h->jit)
+      for (auto& m : part) release_module(m.key);
     for (int c = 0; c < pbn_handle::kMaxLanes; ++c) {
       if (h->s_lane[c]) cudaStreamDestroy(h->s_lane[c]);
       if (h->ev_k[c]) cudaEventDestroy(h->ev_k[c]);
@@ -623,7 +632,7 @@ int pbn_create(const pbn_net_desc* d, pbn_handle** out) {
     h->gen = jit::gen_net_from_desc(d);
     const std::vector<uint32_t> ss = jit::sliced_survival(d->perturb_p, N);
     h->surv_sliced_host = ss;
-    if ((rc = upload(&h->d_surv_sliced, ss.data(), ss.size())) != PBN_OK || (rc = load_sliced(h, 0)) != PBN_OK) {
+    if ((rc = upload(&h->d_surv_sliced, ss.data(), ss.size())) != PBN_OK || (rc = load_program(h, kPartRow, 0)) != PBN_OK) {
       pbn_destroy(h);
       return rc;
     }
@@ -773,14 +782,6 @@ int pbn_update_attractors(pbn_handle* h, const int32_t* attr_offset, const uint6
 
 int pbn_attractor_hash_slots(const pbn_handle* h) { return h ? (h->net.ahash_tags ? (int)h->net.ahash_mask + 1 : 0) : PBN_ERR_INVALID; }
 
-static int grid_for(const pbn_handle* h, int64_t n, int block, int per_sm) {
-  int64_t g = (n + block - 1) / block;
-  const int64_t cap = (int64_t)h->num_sms * per_sm;
-  if (g > cap) g = cap;
-  if (g < 1) g = 1;
-  return (int)g;
-}
-
 static int step_common(pbn_handle* h, const pbn_step_args* a, void* stream_, bool injected) {
   if (!h || !a) return fail(PBN_ERR_INVALID, "null argument");
   if (a->n_envs < 0) return fail(PBN_ERR_INVALID, "n_envs=%lld", (long long)a->n_envs);
@@ -813,33 +814,18 @@ static int step_common(pbn_handle* h, const pbn_step_args* a, void* stream_, boo
   p.a = *a;
   p.n = h->net;
   p.ticket = h->d_ticket;
-  if (h->kernel == PBN_KERNEL_SLICED) {
-    const int rc = a->resident ? launch_planes(h, p, injected, stream) : launch_sliced(h, p, injected, stream);
-    if (rc == PBN_OK) h->launches += 1, g_last_advance = nullptr;
-    return rc;
-  }
+  if (h->kernel == PBN_KERNEL_SLICED)
+    return a->resident ? launch_planes(h, p, injected, stream) : launch_sliced(h, p, injected, stream);
   const ScalarSmemLayout L = scalar_smem_layout(h->net, h->W);
   if (L.total > 200u * 1024u) return fail(PBN_ERR_UNSUPPORTED, "network tables need %u B of shared memory", L.total);
-  const int block = 256;
-  const int grid = grid_for(h, a->n_envs, block, 8);
-  const bool wide = h->net.max_arity > 4;
-  const bool xwide = h->net.max_arity > PBN_MAX_ARITY;
-#define PBN_LAUNCH_SCALAR(WW, MA)                                                                          \
-  do {                                                                                                     \
-    if (L.total > 48u * 1024u && !h->scalar_smem_opted) {                                                  \
-      PBN_CUDA(cudaFuncSetAttribute(step_scalar_kernel<WW, MA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)L.total)); \
-    }                                                                                                      \
-    step_scalar_kernel<WW, MA><<<grid, block, L.total, stream>>>(p, L);                                    \
-  } while (0)
-  if (h->W == 1) {
-    if (xwide) PBN_LAUNCH_SCALAR(1, 16); else if (wide) PBN_LAUNCH_SCALAR(1, 6); else PBN_LAUNCH_SCALAR(1, 4);
-  } else {
-    if (xwide) PBN_LAUNCH_SCALAR(2, 16); else if (wide) PBN_LAUNCH_SCALAR(2, 6); else PBN_LAUNCH_SCALAR(2, 4);
-  }
-#undef PBN_LAUNCH_SCALAR
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  // [W - 1][predictor arity: up to 4, up to 6, wider]
+  static const decltype(&step_scalar_kernel<1, 4>) scalar_kernel[2][3] = {
+      {step_scalar_kernel<1, 4>, step_scalar_kernel<1, 6>, step_scalar_kernel<1, 16>},
+      {step_scalar_kernel<2, 4>, step_scalar_kernel<2, 6>, step_scalar_kernel<2, 16>}};
+  const auto k = scalar_kernel[h->W - 1][h->net.max_arity > PBN_MAX_ARITY ? 2 : h->net.max_arity > 4 ? 1 : 0];
+  const int rc = ensure_dynamic_smem(reinterpret_cast<const void*>(k), L.total, &h->scalar_smem_opt_in);
+  if (rc != PBN_OK) return rc;
+  return launch(h, k, grid_for(h, a->n_envs, 256, 8), 256, L.total, stream, false, p, L);
 }
 
 int64_t pbn_jit_source(const pbn_net_desc* d, int injected, char* buf, int64_t len) {
@@ -865,45 +851,13 @@ int pbn_jit_precompile(const pbn_net_desc* d) {
   for (int inj = 0; inj < 2; ++inj) {
     std::vector<char> cubin;
     std::string err;
-    for (int part = 0; part < (jit::sel_bits(g) == 3 ? 1 : 2); ++part)   // (no plane-resident program with three selection planes)
-      if (jit::compile(g, inj != 0, part, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());
-    if (!inj && jit::compile(g, false, 2, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());   // recording rollout
+    for (int part = 0; part < kParts; ++part)
+      if (part_exists(g, part, inj) && jit::compile(g, inj != 0, part, &cubin, &err) != 0) return fail(PBN_ERR_JIT, "%s", err.c_str());
   }
   return PBN_OK;
 }
 
 int pbn_step(pbn_handle* h, const pbn_step_args* a, void* stream) { return step_common(h, a, stream, false); }
-
-int pbn_rollout(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t step_ctr, int64_t env_offset, int64_t n_envs,
-                unsigned long long* stats, void* stream_) {
-  if (!h || !state) return fail(PBN_ERR_INVALID, "null argument");
-  if (h->kernel != PBN_KERNEL_SLICED) return fail(PBN_ERR_UNSUPPORTED, "pbn_rollout: the handle runs the scalar kernel (loop over pbn_step)");
-  if (n_envs < 0 || n_steps < 0 || n_steps > 0x7FFFFFFF || env_offset < 0 || (env_offset & 1023)) return fail(PBN_ERR_INVALID, "bad n_envs / n_steps / env_offset");
-  if (n_envs == 0 || n_steps == 0) return PBN_OK;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
-  DeviceGuard guard(h->device);
-  int rc = load_sliced(h, 0);
-  if (rc != PBN_OK) return rc;
-  const int N = h->net.n_genes, NW = (N + 31) / 32, NSEL = jit::n_sel_slots(h->gen);
-  const uint32_t smem = (uint32_t)(2 * NW * 1024 + jit::sel_bits(h->gen) * NSEL * 32 + 128 * (8 * N < 255 ? 1 : 2) + 32 + 8) * 4u;
-  if (smem > 227u * 1024u) return fail(PBN_ERR_UNSUPPORTED, "pbn_rollout needs %u B of shared memory", smem);
-  if ((rc = ensure_dynamic_smem(h->rollout_kernel, smem, &h->rollout_smem_opt_in)) != PBN_OK) return rc;
-  RolloutParams p;
-  p.n = h->net;
-  p.state = state;
-  p.stats = stats;
-  p.step_ctr = step_ctr;
-  p.env_offset = env_offset;
-  p.n_envs = n_envs;
-  p.n_steps = (int32_t)n_steps;
-  int64_t grid = (n_envs + 1023) / 1024;
-  const int64_t cap = (int64_t)h->num_sms * h->sliced_min_blocks * 8;
-  if (grid > cap) grid = cap;
-  void* args[] = {&p};
-  PBN_CUDA(cudaLaunchKernel(reinterpret_cast<const void*>(h->rollout_kernel), dim3((unsigned)grid), dim3((unsigned)h->sliced_threads), args, smem, stream));
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
-}
 
 // Checks the projection of a recording call and copies it into proj[12].
 static int record_projection(const pbn_handle* h, const char* who, const int32_t* proj_genes, int32_t n_proj, int32_t* proj) {
@@ -920,26 +874,33 @@ static int record_projection(const pbn_handle* h, const char* who, const int32_t
   return PBN_OK;
 }
 
-int pbn_rollout_record(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t step_ctr, int64_t env_offset,
-                       int64_t n_envs, int32_t stride, const int32_t* proj_genes, int32_t n_proj,
-                       unsigned long long* gene_on, unsigned long long* hist, unsigned long long* stats, void* stream_) {
+// pbn_rollout (rec = false: the rollout kernel of program kPartRow) and pbn_rollout_record (rec = true: program
+// kPartRecord, which also takes the recording arguments).
+static int rollout(pbn_handle* h, bool rec, uint64_t* state, int64_t n_steps, uint64_t step_ctr, int64_t env_offset,
+                   int64_t n_envs, int32_t stride, const int32_t* proj_genes, int32_t n_proj, unsigned long long* gene_on,
+                   unsigned long long* hist, unsigned long long* stats, void* stream_) {
+  const char* who = rec ? "pbn_rollout_record" : "pbn_rollout";
   if (!h || !state) return fail(PBN_ERR_INVALID, "null argument");
   if (h->kernel != PBN_KERNEL_SLICED)
-    return fail(PBN_ERR_UNSUPPORTED, "pbn_rollout_record: the handle runs the scalar kernel (loop over pbn_step + pbn_record_states)");
+    return fail(PBN_ERR_UNSUPPORTED, "%s: the handle runs the scalar kernel (loop over %s)", who, rec ? "pbn_step + pbn_record_states" : "pbn_step");
   if (n_envs < 0 || n_steps < 0 || n_steps > 0x7FFFFFFF || env_offset < 0 || (env_offset & 1023)) return fail(PBN_ERR_INVALID, "bad n_envs / n_steps / env_offset");
-  if (stride < 1) return fail(PBN_ERR_INVALID, "pbn_rollout_record: stride = %d, must be >= 1", stride);
   RecordParams q;
-  int rc = record_projection(h, "pbn_rollout_record", proj_genes, n_proj, q.proj);
-  if (rc != PBN_OK) return rc;
+  if (rec) {
+    if (stride < 1) return fail(PBN_ERR_INVALID, "%s: stride = %d, must be >= 1", who, stride);
+    const int rc = record_projection(h, who, proj_genes, n_proj, q.proj);
+    if (rc != PBN_OK) return rc;
+  }
   if (n_envs == 0 || n_steps == 0) return PBN_OK;
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  if ((rc = load_sliced(h, 0)) != PBN_OK || (rc = load_record(h)) != PBN_OK) return rc;
+  int rc = load_program(h, kPartRow, 0);
+  if (rc == PBN_OK && rec) rc = load_program(h, kPartRecord, 0);
+  if (rc != PBN_OK) return rc;
   const int N = h->net.n_genes, NW = (N + 31) / 32, NSEL = jit::n_sel_slots(h->gen);
-  // the rollout's scratch (pbn_rollout), then the 2^n_proj histogram bins
-  const uint32_t smem = (uint32_t)(2 * NW * 1024 + jit::sel_bits(h->gen) * NSEL * 32 + 128 * (8 * N < 255 ? 1 : 2) + 32 + 8 + (1 << n_proj)) * 4u;
-  if (smem > 227u * 1024u) return fail(PBN_ERR_UNSUPPORTED, "pbn_rollout_record needs %u B of shared memory", smem);
-  if ((rc = ensure_dynamic_smem(h->record_kernel, smem, &h->record_smem_opt_in)) != PBN_OK) return rc;
+  // the rollout's scratch, then the 2^n_proj histogram bins of the recording form
+  const uint32_t smem = (uint32_t)(2 * NW * 1024 + jit::sel_bits(h->gen) * NSEL * 32 + 128 * (8 * N < 255 ? 1 : 2) + 32 + 8 + (rec ? 1 << n_proj : 0)) * 4u;
+  if (smem > 227u * 1024u) return fail(PBN_ERR_UNSUPPORTED, "%s needs %u B of shared memory", who, smem);
+  pbn_handle::JitKernel& k = rec ? h->jit[kPartRecord][0].kernel[0] : h->jit[kPartRow][0].kernel[2];
+  if ((rc = ensure_dynamic_smem(reinterpret_cast<const void*>(k.k), smem, &k.smem_opt_in)) != PBN_OK) return rc;
   q.r.n = h->net;
   q.r.state = state;
   q.r.stats = stats;
@@ -951,13 +912,21 @@ int pbn_rollout_record(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t
   q.hist = hist;
   q.stride = stride;
   q.n_proj = n_proj;
-  int64_t grid = (n_envs + 1023) / 1024;
-  const int64_t cap = (int64_t)h->num_sms * h->sliced_min_blocks * 8;
-  if (grid > cap) grid = cap;
-  void* args[] = {&q};
-  PBN_CUDA(cudaLaunchKernel(reinterpret_cast<const void*>(h->record_kernel), dim3((unsigned)grid), dim3((unsigned)h->sliced_threads), args, smem, stream));
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  void* args[] = {rec ? static_cast<void*>(&q) : static_cast<void*>(&q.r)};
+  return launch(h, k.k, grid_for(h, n_envs, 1024, h->sliced_min_blocks * 8), h->sliced_threads, smem,
+                static_cast<cudaStream_t>(stream_), false, args);
+}
+
+int pbn_rollout(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t step_ctr, int64_t env_offset, int64_t n_envs,
+                unsigned long long* stats, void* stream) {
+  return rollout(h, false, state, n_steps, step_ctr, env_offset, n_envs, 1, nullptr, 0, nullptr, nullptr, stats, stream);
+}
+
+int pbn_rollout_record(pbn_handle* h, uint64_t* state, int64_t n_steps, uint64_t step_ctr, int64_t env_offset,
+                       int64_t n_envs, int32_t stride, const int32_t* proj_genes, int32_t n_proj,
+                       unsigned long long* gene_on, unsigned long long* hist, unsigned long long* stats, void* stream) {
+  return rollout(h, true, state, n_steps, step_ctr, env_offset, n_envs, stride, proj_genes, n_proj, gene_on, hist, stats,
+                 stream);
 }
 
 int pbn_record_states(pbn_handle* h, const uint64_t* state, int64_t n_envs, const int32_t* proj_genes, int32_t n_proj,
@@ -978,13 +947,8 @@ int pbn_record_states(pbn_handle* h, const uint64_t* state, int64_t n_envs, cons
   q.W = h->W;
   q.n_proj = n_proj;
   const uint32_t smem = (uint32_t)((hist ? (1u << n_proj) : 0u) * 4u + 128u * 8u);
-  int64_t grid = (n_envs + kRecordThreads - 1) / kRecordThreads;
-  const int64_t cap = (int64_t)h->num_sms * 4;
-  if (grid > cap) grid = cap;
-  record_states_kernel<<<(unsigned)grid, kRecordThreads, smem, static_cast<cudaStream_t>(stream_)>>>(q);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, record_states_kernel, grid_for(h, n_envs, kRecordThreads, 4), kRecordThreads, smem,
+                static_cast<cudaStream_t>(stream_), false, q);
 }
 
 // The step arguments of envs [e0, e0 + n) of a row-format batch; actions: the device actions of the whole batch or null.
@@ -1160,19 +1124,17 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
         PBN_CUDA(cudaMemcpyAsync(io->actions_dev + e0 * bins, io->actions + e0 * bins, (size_t)n * bins, cudaMemcpyHostToDevice, S));
       } else if (io->actions16) {
         PBN_CUDA(cudaMemcpyAsync(io->actions16_dev + e0, io->actions16 + e0, (size_t)n * 2, cudaMemcpyHostToDevice, S));
-        unpack_actions16_kernel<<<grid_for(h, n / 4 + 1, 256, 4), 256, 0, S>>>(io->actions16_dev + e0, io->actions_dev + e0 * bins, n);
-        PBN_CUDA(cudaGetLastError());
-        h->launches += 1;
+        const int rc = launch(h, unpack_actions16_kernel, grid_for(h, n / 4 + 1, 256, 4), 256, 0, S, false,
+                              io->actions16_dev + e0, io->actions_dev + e0 * bins, n);
+        if (rc != PBN_OK) return rc;
       }
       // PDL only orders kernels, which the lane's stream already does
       pbn_step_args s = env_range(h, a, actions, e0, n);
       s.flags = (a->flags & ~PBN_STEP_PDL) | PBN_STEP_NO_COUNT;
-      const int rc = step_common(h, &s, S, false);
+      int rc = step_common(h, &s, S, false);
       if (rc != PBN_OK) return rc;
       if (zero_copy) {
-        export_kernel<<<16, 256, 0, S>>>(export_range(all, W, e0, n));
-        PBN_CUDA(cudaGetLastError());
-        h->launches += 1;
+        if ((rc = launch(h, export_kernel, 16, 256, 0, S, false, export_range(all, W, e0, n))) != PBN_OK) return rc;
       } else {
         if (io->state) PBN_CUDA(cudaMemcpyAsync(io->state + e0 * W, a->state + e0 * W, (size_t)n * W * 8, cudaMemcpyDeviceToHost, S));
         if (io->reward) PBN_CUDA(cudaMemcpyAsync(io->reward + e0, a->reward + e0, (size_t)n * 4, cudaMemcpyDeviceToHost, S));
@@ -1182,12 +1144,7 @@ int pbn_step_host(pbn_handle* h, const pbn_step_args* a, const pbn_host_io* io, 
       PBN_CUDA(cudaEventRecord(h->ev_k[c], S));
       PBN_CUDA(cudaStreamWaitEvent(h->s_origin, h->ev_k[c], 0));
     }
-    if (own_count) {
-      advance_counter_kernel<<<1, 1, 0, h->s_origin>>>(a->step_ctr_dev, 1ull);
-      PBN_CUDA(cudaGetLastError());
-      h->launches += 1;
-    }
-    return PBN_OK;
+    return own_count ? launch(h, advance_counter_kernel, 1, 1, 0, h->s_origin, false, a->step_ctr_dev, 1ull) : PBN_OK;
   };
   // the staging buffers and device arrays may still be in use by earlier work on the caller's stream
   PBN_CUDA(cudaEventRecord(h->ev_entry, stream));
@@ -1225,14 +1182,8 @@ int pbn_reset(pbn_handle* h, uint64_t* state, int32_t* target_id, int32_t* sourc
   if (env_offset < 0 || (env_offset & 1023)) return fail(PBN_ERR_INVALID, "env_offset must be a non-negative multiple of 1024");
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, n_envs, 256, 8);
-  if (h->W == 1)
-    reset_kernel<1><<<grid, 256, 0, stream>>>(h->net, state, target_id, source_id, t, done_mask, step_ctr, env_offset, n_envs);
-  else
-    reset_kernel<2><<<grid, 256, 0, stream>>>(h->net, state, target_id, source_id, t, done_mask, step_ctr, env_offset, n_envs);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, h->W == 1 ? reset_kernel<1> : reset_kernel<2>, grid_for(h, n_envs, 256, 8), 256, 0, stream, false,
+                h->net, state, target_id, source_id, t, done_mask, step_ctr, env_offset, n_envs);
 }
 
 int pbn_unpack(pbn_handle* h, const uint64_t* state, void* out, int32_t out_kind, int64_t n_envs, void* stream_) {
@@ -1242,25 +1193,18 @@ int pbn_unpack(pbn_handle* h, const uint64_t* state, void* out, int32_t out_kind
   DeviceGuard guard(h->device);
   const int grid = grid_for(h, n_envs * h->net.n_genes, 256, 8);
   if (out_kind == PBN_UNPACK_U8)
-    unpack_kernel<uint8_t><<<grid, 256, 0, stream>>>(state, static_cast<uint8_t*>(out), h->net.n_genes, h->W, n_envs);
-  else if (out_kind == PBN_UNPACK_F32)
-    unpack_kernel<float><<<grid, 256, 0, stream>>>(state, static_cast<float*>(out), h->net.n_genes, h->W, n_envs);
-  else
-    return fail(PBN_ERR_INVALID, "out_kind=%d unknown", out_kind);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+    return launch(h, unpack_kernel<uint8_t>, grid, 256, 0, stream, false, state, static_cast<uint8_t*>(out), h->net.n_genes, h->W, n_envs);
+  if (out_kind == PBN_UNPACK_F32)
+    return launch(h, unpack_kernel<float>, grid, 256, 0, stream, false, state, static_cast<float*>(out), h->net.n_genes, h->W, n_envs);
+  return fail(PBN_ERR_INVALID, "out_kind=%d unknown", out_kind);
 }
 
 int pbn_advance_counter(pbn_handle* h, uint64_t* step_ctr_dev, uint64_t n, void* stream_) {
   if (!h || !step_ctr_dev) return fail(PBN_ERR_INVALID, "bad arguments");
-  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  advance_counter_kernel<<<1, 1, 0, stream>>>(step_ctr_dev, n);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1;
-  g_last_advance = h;
-  return PBN_OK;
+  const int rc = launch(h, advance_counter_kernel, 1, 1, 0, static_cast<cudaStream_t>(stream_), false, step_ctr_dev, n);
+  if (rc == PBN_OK) g_last_advance = h;
+  return rc;
 }
 
 static int check_replay(const pbn_replay* r) {
@@ -1278,10 +1222,8 @@ int pbn_replay_observe(pbn_handle* h, const pbn_replay* r, int64_t head, const u
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  replay_observe_kernel<<<grid_for(h, n_envs * h->W, 256, 8), 256, 0, stream>>>(*r, head, state, target_id, h->W, n_envs);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, replay_observe_kernel, grid_for(h, n_envs * h->W, 256, 8), 256, 0, stream, false, *r, head, state,
+                target_id, h->W, n_envs);
 }
 
 int pbn_replay_commit(pbn_handle* h, const pbn_replay* r, int64_t head, const uint8_t* actions, const float* reward,
@@ -1294,11 +1236,8 @@ int pbn_replay_commit(pbn_handle* h, const pbn_replay* r, int64_t head, const ui
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  replay_commit_kernel<<<grid_for(h, n_envs * h->net.bins, 256, 8), 256, 0, stream>>>(*r, head, actions, reward, terminated, truncated,
-                                                                                 next_state, h->W, h->net.bins, n_envs);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, replay_commit_kernel, grid_for(h, n_envs * h->net.bins, 256, 8), 256, 0, stream, false, *r, head,
+                actions, reward, terminated, truncated, next_state, h->W, h->net.bins, n_envs);
 }
 
 int pbn_replay_sample(pbn_handle* h, const pbn_replay* r, const int64_t* index, int64_t batch, float* obs, float* next_obs,
@@ -1309,17 +1248,13 @@ int pbn_replay_sample(pbn_handle* h, const pbn_replay* r, const int64_t* index, 
   if (batch == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  if (obs || next_obs) {
-    gather_unpack_kernel<<<grid_for(h, batch * h->net.n_genes, 256, 8), 256, 0, stream>>>(h->net, r->state, r->next_state, r->target_id, index,
-                                                                                      h->W, batch, obs, next_obs);
-    PBN_CUDA(cudaGetLastError());
-    h->launches += 1, g_last_advance = nullptr;
-  }
-  if (actions || reward || done) {
-    gather_scalars_kernel<<<grid_for(h, batch * h->net.bins, 256, 8), 256, 0, stream>>>(*r, index, h->net.bins, batch, actions, reward, done);
-    PBN_CUDA(cudaGetLastError());
-    h->launches += 1, g_last_advance = nullptr;
-  }
+  if ((obs || next_obs) &&
+      (rc = launch(h, gather_unpack_kernel, grid_for(h, batch * h->net.n_genes, 256, 8), 256, 0, stream, false, h->net,
+                   r->state, r->next_state, r->target_id, index, h->W, batch, obs, next_obs)) != PBN_OK)
+    return rc;
+  if (actions || reward || done)
+    return launch(h, gather_scalars_kernel, grid_for(h, batch * h->net.bins, 256, 8), 256, 0, stream, false, *r, index,
+                  h->net.bins, batch, actions, reward, done);
   return PBN_OK;
 }
 
@@ -1364,10 +1299,8 @@ static int per_rebuild(pbn_handle* h, const PerView& v, int64_t a0, int64_t b0, 
   r.t1 = a1 >> r.lt;
   if (t1_end > r.t0) t1_end = r.t0;   // a tile the first range already covers
   const int64_t n1 = std::max<int64_t>(0, t1_end - r.t1);
-  per_rebuild_kernel<<<(unsigned)(r.n0 + n1), kPerRebuildThreads, 0, stream>>>(v, r, reset_index, reset_n);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, per_rebuild_kernel, (unsigned)(r.n0 + n1), kPerRebuildThreads, 0, stream, false, v, r, reset_index,
+                reset_n);
 }
 
 int pbn_per_init(pbn_handle* h, const pbn_per* p, void* stream_) {
@@ -1376,10 +1309,7 @@ int pbn_per_init(pbn_handle* h, const pbn_per* p, void* stream_) {
   if (rc != PBN_OK) return rc;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  per_init_kernel<<<grid_for(h, 2 * v.L, 256, 8), 256, 0, stream>>>(v);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, per_init_kernel, grid_for(h, 2 * v.L, 256, 8), 256, 0, stream, false, v);
 }
 
 int pbn_per_push(pbn_handle* h, const pbn_per* p, int64_t head, int64_t n, void* stream_) {
@@ -1405,17 +1335,12 @@ int pbn_per_update(pbn_handle* h, const pbn_per* p, const int64_t* index, const 
   if (batch == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  if (batch <= kPerUpdateOneCta) {
-    per_update_cta_kernel<<<1, kPerUpdateThreads, 0, stream>>>(v, index, td_error, (int)batch, eps);
-    PBN_CUDA(cudaGetLastError());
-    h->launches += 1, g_last_advance = nullptr;
-    return PBN_OK;
-  }
-  per_update_claim_kernel<<<grid_for(h, batch, 256, 8), 256, 0, stream>>>(v, index, batch);
-  PBN_CUDA(cudaGetLastError());
-  per_update_write_kernel<<<grid_for(h, batch, 256, 8), 256, 0, stream>>>(v, index, td_error, batch, eps);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 2, g_last_advance = nullptr;
+  if (batch <= kPerUpdateOneCta)
+    return launch(h, per_update_cta_kernel, 1, kPerUpdateThreads, 0, stream, false, v, index, td_error, (int)batch, eps);
+  const int grid = grid_for(h, batch, 256, 8);
+  if ((rc = launch(h, per_update_claim_kernel, grid, 256, 0, stream, false, v, index, batch)) != PBN_OK ||
+      (rc = launch(h, per_update_write_kernel, grid, 256, 0, stream, false, v, index, td_error, batch, eps)) != PBN_OK)
+    return rc;
   return per_rebuild(h, v, 0, v.L, 0, 0, 0, index, batch, stream);
 }
 
@@ -1429,10 +1354,8 @@ int pbn_per_sample(pbn_handle* h, const pbn_per* p, const float* u, int64_t batc
   if (batch == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  per_sample_kernel<<<grid_for(h, batch * 32, 256, 8), 256, 0, stream>>>(v, u, batch, beta, index, weight);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, per_sample_kernel, grid_for(h, batch * 32, 256, 8), 256, 0, stream, false, v, u, batch, beta, index,
+                weight);
 }
 
 int pbn_observe(pbn_handle* h, const uint64_t* state, const int32_t* target_id, float* obs, int64_t n_envs, void* stream_) {
@@ -1440,11 +1363,8 @@ int pbn_observe(pbn_handle* h, const uint64_t* state, const int32_t* target_id, 
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  gather_unpack_kernel<<<grid_for(h, n_envs * h->net.n_genes, 256, 8), 256, 0, stream>>>(h->net, state, nullptr, target_id, nullptr, h->W,
-                                                                                     n_envs, obs, nullptr);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, gather_unpack_kernel, grid_for(h, n_envs * h->net.n_genes, 256, 8), 256, 0, stream, false, h->net,
+                state, nullptr, target_id, nullptr, h->W, n_envs, obs, nullptr);
 }
 
 int pbn_in_target(pbn_handle* h, const uint64_t* state, const int32_t* target_id, uint8_t* out, int64_t n_envs, void* stream_) {
@@ -1452,12 +1372,8 @@ int pbn_in_target(pbn_handle* h, const uint64_t* state, const int32_t* target_id
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, n_envs, 256, 8);
-  if (h->W == 1) in_target_kernel<1><<<grid, 256, 0, stream>>>(h->net, state, target_id, out, n_envs);
-  else in_target_kernel<2><<<grid, 256, 0, stream>>>(h->net, state, target_id, out, n_envs);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, h->W == 1 ? in_target_kernel<1> : in_target_kernel<2>, grid_for(h, n_envs, 256, 8), 256, 0, stream,
+                false, h->net, state, target_id, out, n_envs);
 }
 
 int pbn_rollout_track(pbn_handle* h, const uint8_t* terminated, uint8_t* active, int32_t* count, int32_t max_steps,
@@ -1466,10 +1382,8 @@ int pbn_rollout_track(pbn_handle* h, const uint8_t* terminated, uint8_t* active,
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  rollout_track_kernel<<<grid_for(h, n_envs, 256, 8), 256, 0, stream>>>(terminated, active, count, max_steps, n_envs, n_active);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, rollout_track_kernel, grid_for(h, n_envs, 256, 8), 256, 0, stream, false, terminated, active, count,
+                max_steps, n_envs, n_active);
 }
 
 int pbn_rollout_reduce(pbn_handle* h, const int32_t* count, const int32_t* pair_id, int64_t n_envs, int32_t n_pairs,
@@ -1479,10 +1393,8 @@ int pbn_rollout_reduce(pbn_handle* h, const int32_t* count, const int32_t* pair_
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  rollout_reduce_kernel<<<grid_for(h, n_envs, 256, 8), 256, 0, stream>>>(count, pair_id, n_envs, n_pairs, max_steps, matrix, hist);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, rollout_reduce_kernel, grid_for(h, n_envs, 256, 8), 256, 0, stream, false, count, pair_id, n_envs,
+                n_pairs, max_steps, matrix, hist);
 }
 
 int pbn_visit_count(pbn_handle* h, const uint64_t* state, const uint8_t* mask, int64_t n_envs, unsigned long long* tags,
@@ -1492,12 +1404,9 @@ int pbn_visit_count(pbn_handle* h, const uint64_t* state, const uint8_t* mask, i
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, n_envs, 256, 8);
-  if (h->W == 1) visit_count_kernel<1><<<grid, 256, 0, stream>>>(state, mask, n_envs, tags, slot_state, counts, (uint64_t)capacity - 1, h->net.n_genes <= 63, overflow);
-  else visit_count_kernel<2><<<grid, 256, 0, stream>>>(state, mask, n_envs, tags, slot_state, counts, (uint64_t)capacity - 1, false, overflow);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, h->W == 1 ? visit_count_kernel<1> : visit_count_kernel<2>, grid_for(h, n_envs, 256, 8), 256, 0, stream,
+                false, state, mask, n_envs, tags, slot_state, counts, (uint64_t)capacity - 1,
+                h->W == 1 && h->net.n_genes <= 63, overflow);
 }
 
 int pbn_successor_sets(pbn_handle* h, const uint64_t* state, int64_t n_states, uint64_t* can1, uint64_t* can0, void* stream_) {
@@ -1505,12 +1414,8 @@ int pbn_successor_sets(pbn_handle* h, const uint64_t* state, int64_t n_states, u
   if (n_states == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, n_states, 256, 8);
-  if (h->W == 1) successor_sets_kernel<1><<<grid, 256, 0, stream>>>(h->net, state, n_states, can1, can0);
-  else successor_sets_kernel<2><<<grid, 256, 0, stream>>>(h->net, state, n_states, can1, can0);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, h->W == 1 ? successor_sets_kernel<1> : successor_sets_kernel<2>, grid_for(h, n_states, 256, 8), 256, 0,
+                stream, false, h->net, state, n_states, can1, can0);
 }
 
 int pbn_closure_expand(pbn_handle* h, uint64_t* list, int64_t begin, int64_t end, int64_t list_cap, unsigned long long* list_count,
@@ -1523,12 +1428,9 @@ int pbn_closure_expand(pbn_handle* h, uint64_t* list, int64_t begin, int64_t end
   if (end == begin) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, (end - begin) * 128, 128, 16);
-  if (h->W == 1) closure_expand_kernel<1><<<grid, 128, 0, stream>>>(h->net, list, begin, end, list_cap, list_count, tags, slot_state, slot_index, (uint64_t)capacity - 1, max_free, status);
-  else closure_expand_kernel<2><<<grid, 128, 0, stream>>>(h->net, list, begin, end, list_cap, list_count, tags, slot_state, slot_index, (uint64_t)capacity - 1, max_free, status);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, h->W == 1 ? closure_expand_kernel<1> : closure_expand_kernel<2>, grid_for(h, (end - begin) * 128, 128, 16),
+                128, 0, stream, false, h->net, list, begin, end, list_cap, list_count, tags, slot_state, slot_index,
+                (uint64_t)capacity - 1, max_free, status);
 }
 
 int pbn_closure_reach(pbn_handle* h, const uint64_t* list, int64_t count, uint8_t* flags, const unsigned long long* tags,
@@ -1539,12 +1441,8 @@ int pbn_closure_reach(pbn_handle* h, const uint64_t* list, int64_t count, uint8_
   if (count == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, count * 128, 128, 16);
-  if (h->W == 1) closure_reach_kernel<1><<<grid, 128, 0, stream>>>(h->net, list, count, flags, tags, slot_state, slot_index, (uint64_t)capacity - 1, changed);
-  else closure_reach_kernel<2><<<grid, 128, 0, stream>>>(h->net, list, count, flags, tags, slot_state, slot_index, (uint64_t)capacity - 1, changed);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, h->W == 1 ? closure_reach_kernel<1> : closure_reach_kernel<2>, grid_for(h, count * 128, 128, 16), 128, 0,
+                stream, false, h->net, list, count, flags, tags, slot_state, slot_index, (uint64_t)capacity - 1, changed);
 }
 
 int64_t pbn_resident_words(const pbn_handle* h, int64_t n_envs) {
@@ -1563,15 +1461,11 @@ int pbn_resident_import(pbn_handle* h, uint32_t* resident, const uint64_t* state
   if (target_id && h->net.n_attr == 0) return fail(PBN_ERR_NO_ATTRACTORS, "target_id given but no attractor table uploaded");
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, ((n_envs + 1023) / 1024) * 1024, 256, 8);
-  if (h->W == 1) resident_import_kernel<1><<<grid, 256, 0, stream>>>(h->net, resident, state, target_id, t, n_envs);
-  else resident_import_kernel<2><<<grid, 256, 0, stream>>>(h->net, resident, state, target_id, t, n_envs);
-  {
-    const int64_t nt = (n_envs + 1023) / 1024;
-    PBN_CUDA(cudaMemsetAsync(resident + nt * 32 * (int64_t)resident_rows(h->net.n_genes), 0, (size_t)((nt + 31) / 32) * 32 * 4, stream));
-  }
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
+  const int64_t nt = (n_envs + 1023) / 1024;
+  if ((rc = launch(h, h->W == 1 ? resident_import_kernel<1> : resident_import_kernel<2>, grid_for(h, nt * 1024, 256, 8), 256,
+                   0, stream, false, h->net, resident, state, target_id, t, n_envs)) != PBN_OK)
+    return rc;
+  PBN_CUDA(cudaMemsetAsync(resident + nt * 32 * (int64_t)resident_rows(h->net.n_genes), 0, (size_t)((nt + 31) / 32) * 32 * 4, stream));
   return PBN_OK;
 }
 
@@ -1581,12 +1475,9 @@ int pbn_resident_export(pbn_handle* h, const uint32_t* resident, uint64_t* state
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, ((n_envs + 1023) / 1024) * 1024, 256, 8);
-  if (h->W == 1) resident_export_kernel<1><<<grid, 256, 0, stream>>>(h->net, resident, state, target_id, t, n_envs);
-  else resident_export_kernel<2><<<grid, 256, 0, stream>>>(h->net, resident, state, target_id, t, n_envs);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, h->W == 1 ? resident_export_kernel<1> : resident_export_kernel<2>,
+                grid_for(h, ((n_envs + 1023) / 1024) * 1024, 256, 8), 256, 0, stream, false, h->net, resident, state, target_id,
+                t, n_envs);
 }
 
 int pbn_pack(pbn_handle* h, const uint8_t* bits, uint64_t* state, int64_t n_envs, void* stream_) {
@@ -1594,11 +1485,8 @@ int pbn_pack(pbn_handle* h, const uint8_t* bits, uint64_t* state, int64_t n_envs
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, n_envs * h->W, 256, 8);
-  pack_kernel<<<grid, 256, 0, stream>>>(bits, state, h->net.n_genes, h->W, n_envs);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, pack_kernel, grid_for(h, n_envs * h->W, 256, 8), 256, 0, stream, false, bits, state, h->net.n_genes,
+                h->W, n_envs);
 }
 
 int pbn_attractor_id(pbn_handle* h, const uint64_t* state, int32_t* attr_id, int64_t n_envs, void* stream_) {
@@ -1606,14 +1494,8 @@ int pbn_attractor_id(pbn_handle* h, const uint64_t* state, int32_t* attr_id, int
   if (n_envs == 0) return PBN_OK;
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
-  const int grid = grid_for(h, n_envs, 256, 8);
-  if (h->W == 1)
-    attractor_id_kernel<1><<<grid, 256, 0, stream>>>(h->net, state, attr_id, n_envs);
-  else
-    attractor_id_kernel<2><<<grid, 256, 0, stream>>>(h->net, state, attr_id, n_envs);
-  PBN_CUDA(cudaGetLastError());
-  h->launches += 1, g_last_advance = nullptr;
-  return PBN_OK;
+  return launch(h, h->W == 1 ? attractor_id_kernel<1> : attractor_id_kernel<2>, grid_for(h, n_envs, 256, 8), 256, 0, stream,
+                false, h->net, state, attr_id, n_envs);
 }
 
 // ---- exact optimal control (control.cuh) ----
@@ -1653,32 +1535,27 @@ int pbn_dp_expect(pbn_handle* h, const double* func_prob, const double* u_in, do
     const uint32_t tiles = S >> tb, per = kDpSliceStates >> tb;
     for (uint32_t t0 = 0; t0 < tiles; t0 += per) {
       const uint32_t nt = tiles - t0 < per ? tiles - t0 : per;
-      dp_kp_low_kernel<<<grid_for(h, (int64_t)nt * 256, 256, 8), 256, 0, stream>>>(u_in, kpu, tb, t0, nt, p);
-      PBN_CUDA(cudaGetLastError());
-      h->launches += 1;
+      if ((rc = launch(h, dp_kp_low_kernel, grid_for(h, (int64_t)nt * 256, 256, 8), 256, 0, stream, false, u_in, kpu, tb,
+                       t0, nt, p)) != PBN_OK)
+        return rc;
     }
     for (int b = tb; b < N; ++b)
       for (uint32_t j0 = 0; j0 < S / 2; j0 += kDpSliceStates) {
         const uint32_t cnt = S / 2 - j0 < kDpSliceStates ? S / 2 - j0 : kDpSliceStates;
-        dp_kp_bit_kernel<<<grid_for(h, cnt, 256, 8), 256, 0, stream>>>(kpu, b, j0, cnt, p);
-        PBN_CUDA(cudaGetLastError());
-        h->launches += 1;
+        if ((rc = launch(h, dp_kp_bit_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, kpu, b, j0, cnt, p)) != PBN_OK)
+          return rc;
       }
   }
   const double c = std::pow(1.0 - p, (double)N);
   for (uint32_t s0 = 0; s0 < S; s0 += kDpSliceStates) {
     const uint32_t cnt = S - s0 < kDpSliceStates ? S - s0 : kDpSliceStates;
-    dp_expect_kernel<<<grid_for(h, (int64_t)cnt * 32, kDpWarps * 32, 8), kDpWarps * 32, 0, stream>>>(
-        h->net, func_prob, model == PBN_PERT_B ? kpu : u_in, w, s0, cnt);
-    PBN_CUDA(cudaGetLastError());
-    h->launches += 1;
-    if (model == PBN_PERT_A) {
-      dp_mix_kernel<<<grid_for(h, cnt, 256, 8), 256, 0, stream>>>(w, kpu, u_in, c, s0, cnt);
-      PBN_CUDA(cudaGetLastError());
-      h->launches += 1;
-    }
+    if ((rc = launch(h, dp_expect_kernel, grid_for(h, (int64_t)cnt * 32, kDpWarps * 32, 8), kDpWarps * 32, 0, stream, false,
+                     h->net, func_prob, model == PBN_PERT_B ? kpu : u_in, w, s0, cnt)) != PBN_OK)
+      return rc;
+    if (model == PBN_PERT_A &&
+        (rc = launch(h, dp_mix_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, w, kpu, u_in, c, s0, cnt)) != PBN_OK)
+      return rc;
   }
-  g_last_advance = nullptr;
   return PBN_OK;
 }
 
@@ -1710,13 +1587,11 @@ int pbn_dp_improve(pbn_handle* h, const double* w, uint64_t flip_genes, int32_t 
     const double cost_k = r_action * (double)k;
     for (uint32_t s0 = 0; s0 < S; s0 += kDpSliceStates) {
       const uint32_t cnt = S - s0 < kDpSliceStates ? S - s0 : kDpSliceStates;
-      dp_improve_kernel<<<grid_for(h, cnt, 256, 8), 256, 0, stream>>>(w, ival, iend, oval, oend, v, policy,
-                                                                      (uint32_t)flip_genes, k, cost0, cost_k, s0, cnt);
-      PBN_CUDA(cudaGetLastError());
-      h->launches += 1;
+      const int rc = launch(h, dp_improve_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, w, ival, iend, oval, oend,
+                            v, policy, (uint32_t)flip_genes, k, cost0, cost_k, s0, cnt);
+      if (rc != PBN_OK) return rc;
     }
   }
-  g_last_advance = nullptr;
   return PBN_OK;
 }
 
