@@ -478,10 +478,11 @@ int pbn_closure_reach(pbn_handle* h, const uint64_t* list, int64_t count, uint8_
  * K_p - (1-p)^N I, K_p = the per-gene binary symmetric channel (a perturbed step skips the update and lands on
  * u ^ pert, pert != 0); model C with p > 0 makes nearly every gene free in every state (a backup of O(4^N)) and is
  * refused; any model with p = 0 is NONE.
- * Both calls run on the caller's stream without synchronising or allocating, in launches of at most 2^22 states, and
- * are deterministic: the same inputs give bit-identical outputs (no floating-point atomics). */
+ * The exact state distribution after a step, x P, is pbn_dp_push.  All three calls run on the caller's stream without
+ * synchronising or allocating, in launches of at most 2^22 states, and are deterministic: the same inputs give
+ * bit-identical outputs (no floating-point atomics). */
 #define PBN_DP_MAX_GENES 28
-/* Bytes of caller-owned DEVICE workspace the two calls below need for this handle (24 * 2^N), or a negative status:
+/* Bytes of caller-owned DEVICE workspace the three calls below need for this handle (24 * 2^N), or a negative status:
  * PBN_ERR_UNSUPPORTED when N > PBN_DP_MAX_GENES or the perturbation model is C with p > 0. */
 int64_t pbn_dp_workspace_bytes(const pbn_handle* h);
 /* w[u] = sum_t P(u -> t) u_in[t] for every u in [0, 2^N)  (fp64, DEVICE arrays of 2^N; w must not alias u_in).  P: one
@@ -495,6 +496,17 @@ int pbn_dp_expect(pbn_handle* h, const double* func_prob, const double* u_in, do
  * w; workspace (pbn_dp_workspace_bytes) may be NULL when max_flips <= 1. */
 int pbn_dp_improve(pbn_handle* h, const double* w, uint64_t flip_genes, int32_t max_flips, double r_action,
                    double* v, uint32_t* policy, void* workspace, void* stream);
+/* y = x P (masks == NULL) or x P_mu, P_mu(s, .) = P(s ^ masks[s], .) -- the forward operator of pbn_dp_expect, for
+ * state distributions: y[t] = sum_s x_in[s] P_mu(s -> t), one env step from distribution x_in with the flips
+ * masks[s] (DEVICE uint32 [2^N], bits at gene N and above ignored; NULL: no interventions) applied first.  x_in, y:
+ * DEVICE fp64 [2^N], y must not alias x_in; func_prob as for pbn_dp_expect; workspace: pbn_dp_workspace_bytes (may be
+ * NULL when p = 0 and masks == NULL).  The sums are exact integer sums in fixed point: every term x_in[s] P(s -> t) of
+ * the selection step (and x_in[s] of the interventions) is rounded to the nearest multiple of 2^-63, losing at most
+ * 2^-64, so y is bit-identical from call to call whatever the order of the additions.  This needs x_in >= 0 and
+ * sum x_in <= 1 (a probability or sub-probability vector; not validated).  Perturbation is applied in fp64 after the
+ * selection step (model B) or mixed in with c = (1-p)^N (model A: y = c x F + x K_p - c x). */
+int pbn_dp_push(pbn_handle* h, const double* func_prob, const double* x_in, const uint32_t* masks, double* y,
+                void* workspace, void* stream);
 
 /* *step_ctr_dev += n on the stream (fully serialised): closes a sequence of PBN_STEP_PDL launches. */
 int pbn_advance_counter(pbn_handle* h, uint64_t* step_ctr_dev, uint64_t n, void* stream);

@@ -14,9 +14,11 @@ __all__ = [
     "sorted_id_permutation", "BoolFunction", "IsplError", "compile_expression", "logic_functions_from_ispl",
     "parse_ispl", "render_ispl", "PBNNetwork", "pack_states", "unpack_states", "VecPBNEnv",
     "solve_control", "ControlSolution", "TabularPolicy", "policy_values", "tabulate_policy", "expected_all_pairs",
+    "StateDistribution", "propagate", "stationary_distribution",
 ]
 
 _CONTROL = ("solve_control", "ControlSolution", "TabularPolicy", "policy_values", "tabulate_policy", "expected_all_pairs")
+_STEADY_STATE = ("StateDistribution", "propagate", "stationary_distribution")
 
 
 def __getattr__(name):
@@ -30,4 +32,7 @@ def __getattr__(name):
     if name in _CONTROL:
         from . import control
         return getattr(control, name)
+    if name in _STEADY_STATE:
+        from . import steady_state
+        return getattr(steady_state, name)
     raise AttributeError(name)

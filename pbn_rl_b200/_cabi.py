@@ -39,7 +39,7 @@ EXPORTS = (
     "pbn_rollout", "pbn_rollout_record", "pbn_record_states",
     "pbn_resident_words", "pbn_resident_import", "pbn_resident_export", "pbn_reward_table", "pbn_attractor_hash_slots",
     "pbn_per_tree_floats", "pbn_per_init", "pbn_per_push", "pbn_per_update", "pbn_per_sample",
-    "pbn_dp_workspace_bytes", "pbn_dp_expect", "pbn_dp_improve",
+    "pbn_dp_workspace_bytes", "pbn_dp_expect", "pbn_dp_improve", "pbn_dp_push",
 )
 
 
@@ -195,6 +195,8 @@ def load_library(path: Optional[os.PathLike] = None) -> C.CDLL:
     lib.pbn_dp_expect.restype = C.c_int
     lib.pbn_dp_improve.argtypes = [vp, vp, u64, i32, C.c_double, vp, vp, vp, vp]
     lib.pbn_dp_improve.restype = C.c_int
+    lib.pbn_dp_push.argtypes = [vp, vp, vp, vp, vp, vp, vp]
+    lib.pbn_dp_push.restype = C.c_int
     lib.pbn_observe.argtypes = [vp, vp, vp, vp, i64, vp]
     lib.pbn_observe.restype = C.c_int
     lib.pbn_in_target.argtypes = [vp, vp, vp, vp, i64, vp]

@@ -122,6 +122,16 @@ class _Backup:
                                      self.vec._stream()))
         return w
 
+    def push(self, x: torch.Tensor, masks: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """y = x P, the forward operator of :meth:`expect` (x P_mu with flip masks ``masks`` [2^N] applied first).
+        ``x`` must be a probability or sub-probability vector (pbn_dp_push's fixed point)."""
+        x = x.to(torch.float64).contiguous()
+        y = torch.empty_like(x)
+        m = None if masks is None else masks.to(torch.int32).contiguous()
+        check(self.lib.pbn_dp_push(self.h, self.func_prob.data_ptr(), x.data_ptr(), None if m is None else m.data_ptr(),
+                                   y.data_ptr(), self.ws.data_ptr(), self.vec._stream()))
+        return y
+
     def improve(self, w: torch.Tensor, flip_genes: int, max_flips: int, r_action: float):
         v = torch.empty_like(w)
         pol = torch.empty((self.S,), dtype=torch.int32, device=self.dev)

@@ -2,9 +2,11 @@
 // backward-induction backup over all 2^N states of a network with N <= PBN_DP_MAX_GENES genes.
 //   expect : w = P u, P = one step of the handle's dynamics without interventions (selection, then perturbation)
 //   improve: v[s] = max over flip masks m of fl(r_action * |m|) + w[s ^ m], policy[s] = the maximising m
+// and the forward operator of expect, for state distributions:
+//   push   : y = x P (x P_mu with interventions), the same successor enumeration as a fixed-point scatter
 // Generic kernels over the handle's NetParams (like discover.cuh): states are one 32-bit index (bit i = gene i),
-// every launch covers a bounded slice of the state space, and no floating-point sum uses atomics, so the results are
-// bit-identical from call to call.
+// every launch covers a bounded slice of the state space, and no floating-point sum uses atomics (push adds integers),
+// so the results are bit-identical from call to call.
 #pragma once
 #include "pbn_common.cuh"
 #include "discover.cuh"
@@ -155,6 +157,123 @@ __global__ void __launch_bounds__(256) dp_mix_kernel(double* __restrict__ w, con
   for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < count; i += gridDim.x * blockDim.x) {
     const uint32_t x = s0 + i;
     w[x] = (c * w[x] + kpu[x]) - c * u[x];
+  }
+}
+
+// ---- push: y = x F, the transpose of expect -------------------------------------------------------------------------
+// A scatter, made deterministic by fixed point: every term x[s] F(s -> t) is rounded to the nearest multiple of 2^-63
+// and added to y[t] as an unsigned 64-bit integer.  Integer addition is associative, so the sum does not depend on the
+// order in which the atomics land; dp_fix_kernel converts each total to fp64 once.  For x >= 0 with sum x <= 1 the
+// totals stay below 2^64 units.  A term loses at most 2^-64 to the rounding (terms below 2^-64 vanish).
+constexpr double kDpFixOne = 9223372036854775808.0;   // 2^63: fixed-point units per 1.0
+
+__device__ __forceinline__ void dp_fix_add(unsigned long long* __restrict__ acc, uint32_t t, double v) {
+  const unsigned long long q = __double2ull_rn(v * kDpFixOne);
+  if (q != 0ull) atomicAdd(acc + t, q);
+}
+
+// One warp per source state s, enumerating its successors with dp_expect_kernel's code (lane genes, ballots, digit
+// tables; repeated here so that expect compiles as before); each term x[s] * weight is added to y[t] instead of
+// gathering u[t].  A state with x[s] = 0 is skipped, so a push from a point mass or a sparse distribution costs one pass
+// over x plus its terms.
+__global__ void __launch_bounds__(kDpWarps * 32) dp_push_kernel(const __grid_constant__ NetParams n,
+                                                               const double* __restrict__ func_prob,
+                                                               const double* __restrict__ x,
+                                                               unsigned long long* __restrict__ y, uint32_t s0,
+                                                               uint32_t count) {
+  __shared__ ExpectWarpTables tabs[kDpWarps];
+  const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31u;
+  ExpectWarpTables& tb = tabs[warp];
+  for (uint32_t i = blockIdx.x * kDpWarps + warp; i < count; i += gridDim.x * kDpWarps) {
+    const uint32_t s = s0 + i;
+    const double xs = x[s];
+    if (xs == 0.0) continue;   // the same for every lane of the warp
+    double q1 = 0.0, q0 = 0.0;
+    bool can1 = false, can0 = false;
+    if ((int)lane < n.n_genes) {
+      const uint64_t st[1] = {s};
+      for (int f = n.func_offset[lane]; f < n.func_offset[lane + 1]; ++f) {
+        const double p = func_prob[f];
+        if (eval_func<1>(n, f, st)) { q1 += p; can1 = true; } else { q0 += p; can0 = true; }
+      }
+    }
+    const uint32_t one = __ballot_sync(0xFFFFFFFFu, can1), zero = __ballot_sync(0xFFFFFFFFu, can0);
+    uint32_t fr = one & zero;
+    const uint32_t fixed = one & ~zero;
+    const int nf = __popc(fr);
+    const int nlo = nf < 5 ? nf : 5;
+    // lane part: the lowest nlo free genes
+    double wlo = 1.0;
+    uint32_t tlo = 0;
+    for (int j = 0; j < nlo; ++j) {
+      const int g = __ffs(fr) - 1;
+      fr &= fr - 1;
+      const double a1 = __shfl_sync(0xFFFFFFFFu, q1, g), a0 = __shfl_sync(0xFFFFFFFFu, q0, g);
+      const bool b = (lane >> j) & 1u;
+      wlo *= b ? a1 : a0;
+      tlo |= (uint32_t)b << g;
+    }
+    // digit tables of the remaining free genes: digit k holds genes 4k..4k+3 of them
+    const int nhi = nf - nlo;
+    double dw = 1.0;
+    uint32_t db = 0;
+    for (int j = 0; j < nhi; ++j) {
+      const int g = __ffs(fr) - 1;
+      fr &= fr - 1;
+      const double a1 = __shfl_sync(0xFFFFFFFFu, q1, g), a0 = __shfl_sync(0xFFFFFFFFu, q0, g);
+      const bool b = (lane >> (j & 3)) & 1u;
+      dw *= b ? a1 : a0;
+      db |= (uint32_t)b << g;
+      if ((j & 3) == 3 || j == nhi - 1) {
+        if (lane < 16u) { tb.wt[j >> 2][lane] = dw; tb.bits[j >> 2][lane] = db; }
+        dw = 1.0;
+        db = 0;
+      }
+    }
+    __syncwarp();
+    if (lane < (1u << nlo)) {
+      const int b0 = nhi < 4 ? nhi : 4;
+      const int nd = (nhi + 3) >> 2;
+      const uint32_t outer = 1u << (nhi - b0), inner = 1u << b0;
+      const uint32_t base = fixed | tlo;
+      for (uint32_t xo = 0; xo < outer; ++xo) {
+        double wo = xs * wlo;
+        uint32_t to = base;
+        uint32_t r = xo;
+        for (int k = 1; k < nd; ++k) {
+          wo *= tb.wt[k][r & 15u];
+          to |= tb.bits[k][r & 15u];
+          r >>= 4;
+        }
+        if (nhi == 0) {
+          dp_fix_add(y, to, wo);
+        } else {
+#pragma unroll 4
+          for (uint32_t x0 = 0; x0 < inner; ++x0) dp_fix_add(y, to | tb.bits[0][x0], wo * tb.wt[0][x0]);
+        }
+      }
+    }
+    __syncwarp();   // the tables are rewritten for the next state
+  }
+}
+
+// The interventions of a closed loop, y = x M_mu: x[s] moves to s ^ masks[s] (mask bits at gene N and above, outside
+// smask = 2^N - 1, are ignored), into the same fixed-point accumulator.
+__global__ void __launch_bounds__(256) dp_flip_push_kernel(const double* __restrict__ x, const uint32_t* __restrict__ masks,
+                                                           unsigned long long* __restrict__ y, uint32_t smask, uint32_t s0,
+                                                           uint32_t count) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < count; i += gridDim.x * blockDim.x) {
+    const uint32_t s = s0 + i;
+    const double xs = x[s];
+    if (xs != 0.0) dp_fix_add(y, (s ^ masks[s]) & smask, xs);
+  }
+}
+
+// Fixed point to fp64 in place: v[s] = units * 2^-63.
+__global__ void __launch_bounds__(256) dp_fix_kernel(unsigned long long* __restrict__ v, uint32_t s0, uint32_t count) {
+  for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < count; i += gridDim.x * blockDim.x) {
+    const uint32_t s = s0 + i;
+    v[s] = (unsigned long long)__double_as_longlong(__ull2double_rn(v[s]) * (1.0 / kDpFixOne));
   }
 }
 

@@ -1518,6 +1518,29 @@ int64_t pbn_dp_workspace_bytes(const pbn_handle* h) {
   return (int64_t)24 << h->net.n_genes;   // two (fp64 value, u32 endpoint) buffers of the relaxation; expect uses the first
 }
 
+// out = K_p in over all 2^N states: the low genes tile by tile in shared memory, then one in-place pass per higher gene.
+static int dp_kp(pbn_handle* h, const double* in, double* out, cudaStream_t stream) {
+  const int N = h->net.n_genes;
+  const uint32_t S = 1u << N;
+  const double p = h->perturb_p;
+  const int tb = N < kKpTileBits ? N : kKpTileBits;
+  const uint32_t tiles = S >> tb, per = kDpSliceStates >> tb;
+  int rc;
+  for (uint32_t t0 = 0; t0 < tiles; t0 += per) {
+    const uint32_t nt = tiles - t0 < per ? tiles - t0 : per;
+    if ((rc = launch(h, dp_kp_low_kernel, grid_for(h, (int64_t)nt * 256, 256, 8), 256, 0, stream, false, in, out, tb,
+                     t0, nt, p)) != PBN_OK)
+      return rc;
+  }
+  for (int b = tb; b < N; ++b)
+    for (uint32_t j0 = 0; j0 < S / 2; j0 += kDpSliceStates) {
+      const uint32_t cnt = S / 2 - j0 < kDpSliceStates ? S / 2 - j0 : kDpSliceStates;
+      if ((rc = launch(h, dp_kp_bit_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, out, b, j0, cnt, p)) != PBN_OK)
+        return rc;
+    }
+  return PBN_OK;
+}
+
 int pbn_dp_expect(pbn_handle* h, const double* func_prob, const double* u_in, double* w, void* workspace, void* stream_) {
   int model, rc;
   if ((rc = dp_model(h, "pbn_dp_expect", &model)) != PBN_OK) return rc;
@@ -1530,22 +1553,7 @@ int pbn_dp_expect(pbn_handle* h, const double* func_prob, const double* u_in, do
   cudaStream_t stream = static_cast<cudaStream_t>(stream_);
   DeviceGuard guard(h->device);
   double* kpu = static_cast<double*>(workspace);
-  if (model != PBN_PERT_NONE) {   // kpu = K_p u_in: low genes tile by tile in shared memory, then one pass per higher gene
-    const int tb = N < kKpTileBits ? N : kKpTileBits;
-    const uint32_t tiles = S >> tb, per = kDpSliceStates >> tb;
-    for (uint32_t t0 = 0; t0 < tiles; t0 += per) {
-      const uint32_t nt = tiles - t0 < per ? tiles - t0 : per;
-      if ((rc = launch(h, dp_kp_low_kernel, grid_for(h, (int64_t)nt * 256, 256, 8), 256, 0, stream, false, u_in, kpu, tb,
-                       t0, nt, p)) != PBN_OK)
-        return rc;
-    }
-    for (int b = tb; b < N; ++b)
-      for (uint32_t j0 = 0; j0 < S / 2; j0 += kDpSliceStates) {
-        const uint32_t cnt = S / 2 - j0 < kDpSliceStates ? S / 2 - j0 : kDpSliceStates;
-        if ((rc = launch(h, dp_kp_bit_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, kpu, b, j0, cnt, p)) != PBN_OK)
-          return rc;
-      }
-  }
+  if (model != PBN_PERT_NONE && (rc = dp_kp(h, u_in, kpu, stream)) != PBN_OK) return rc;
   const double c = std::pow(1.0 - p, (double)N);
   for (uint32_t s0 = 0; s0 < S; s0 += kDpSliceStates) {
     const uint32_t cnt = S - s0 < kDpSliceStates ? S - s0 : kDpSliceStates;
@@ -1555,6 +1563,70 @@ int pbn_dp_expect(pbn_handle* h, const double* func_prob, const double* u_in, do
     if (model == PBN_PERT_A &&
         (rc = launch(h, dp_mix_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, w, kpu, u_in, c, s0, cnt)) != PBN_OK)
       return rc;
+  }
+  return PBN_OK;
+}
+
+// acc (2^N u64 fixed-point units) -> fp64 in place.
+static int dp_fix(pbn_handle* h, unsigned long long* acc, cudaStream_t stream) {
+  const uint32_t S = 1u << h->net.n_genes;
+  for (uint32_t s0 = 0; s0 < S; s0 += kDpSliceStates) {
+    const uint32_t cnt = S - s0 < kDpSliceStates ? S - s0 : kDpSliceStates;
+    const int rc = launch(h, dp_fix_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, acc, s0, cnt);
+    if (rc != PBN_OK) return rc;
+  }
+  return PBN_OK;
+}
+
+// The forward operator, by the transposes of expect's steps (K_p is symmetric):
+//   NONE: y = x' F;   B: y = (x' F) K_p;   A: y = c (x' F) + x' K_p - c x',   x' = x M_mu (masks) or x.
+// Workspace: [0, 2^N) holds x M_mu, [2^N, 2^(N+1)) the push of model B or x' K_p of model A.
+int pbn_dp_push(pbn_handle* h, const double* func_prob, const double* x_in, const uint32_t* masks, double* y,
+                void* workspace, void* stream_) {
+  int model, rc;
+  if ((rc = dp_model(h, "pbn_dp_push", &model)) != PBN_OK) return rc;
+  if (!func_prob || !x_in || !y) return fail(PBN_ERR_INVALID, "pbn_dp_push: null array");
+  if (x_in == y) return fail(PBN_ERR_INVALID, "pbn_dp_push: y must not alias x_in");
+  if ((model != PBN_PERT_NONE || masks) && !workspace)
+    return fail(PBN_ERR_INVALID, "pbn_dp_push: perturbation or masks need the workspace");
+  const int N = h->net.n_genes;
+  const uint32_t S = 1u << N;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  double* ws = static_cast<double*>(workspace);
+  double* second = ws ? ws + S : nullptr;
+  const double* src = x_in;
+  if (masks) {
+    unsigned long long* acc = reinterpret_cast<unsigned long long*>(ws);
+    PBN_CUDA(cudaMemsetAsync(acc, 0, (size_t)S * sizeof(double), stream));
+    for (uint32_t s0 = 0; s0 < S; s0 += kDpSliceStates) {
+      const uint32_t cnt = S - s0 < kDpSliceStates ? S - s0 : kDpSliceStates;
+      if ((rc = launch(h, dp_flip_push_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, x_in, masks, acc, S - 1u,
+                       s0, cnt)) != PBN_OK)
+        return rc;
+    }
+    if ((rc = dp_fix(h, acc, stream)) != PBN_OK) return rc;
+    src = ws;
+  }
+  if (model == PBN_PERT_A && (rc = dp_kp(h, src, second, stream)) != PBN_OK) return rc;
+  unsigned long long* acc = reinterpret_cast<unsigned long long*>(model == PBN_PERT_B ? second : y);
+  PBN_CUDA(cudaMemsetAsync(acc, 0, (size_t)S * sizeof(double), stream));
+  for (uint32_t s0 = 0; s0 < S; s0 += kDpSliceStates) {
+    const uint32_t cnt = S - s0 < kDpSliceStates ? S - s0 : kDpSliceStates;
+    if ((rc = launch(h, dp_push_kernel, grid_for(h, (int64_t)cnt * 32, kDpWarps * 32, 8), kDpWarps * 32, 0, stream, false,
+                     h->net, func_prob, src, acc, s0, cnt)) != PBN_OK)
+      return rc;
+  }
+  if ((rc = dp_fix(h, acc, stream)) != PBN_OK) return rc;
+  if (model == PBN_PERT_B) return dp_kp(h, second, y, stream);
+  if (model == PBN_PERT_A) {
+    const double c = std::pow(1.0 - h->perturb_p, (double)N);
+    for (uint32_t s0 = 0; s0 < S; s0 += kDpSliceStates) {
+      const uint32_t cnt = S - s0 < kDpSliceStates ? S - s0 : kDpSliceStates;
+      if ((rc = launch(h, dp_mix_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, y, second, src, c, s0, cnt)) !=
+          PBN_OK)
+        return rc;
+    }
   }
   return PBN_OK;
 }
