@@ -466,6 +466,23 @@ int pbn_closure_reach(pbn_handle* h, const uint64_t* list, int64_t count, uint8_
                       const unsigned long long* tags, const uint64_t* slot_state,
                       const unsigned long long* slot_index, int64_t capacity, int32_t* changed, void* stream);
 
+/* ---- Exhaustive attractor search: backward reachability over every state (N <= PBN_DP_MAX_GENES) ----------------
+ * Without perturbation every state reaches an attractor (a sink SCC of the STG above) and attractors are closed.  So
+ * mark the states of the attractors found so far (pbn_reach_mark) and repeat pbn_reach_sweep -- "mark s if some
+ * successor of s is marked" -- until a sweep marks nothing: if every state is then marked, no other attractor exists;
+ * otherwise the unmarked states are closed under successors and hold at least one attractor not found yet.  The fixed
+ * point is the set of states that reach a marked seed; it does not depend on the order of the marks within a sweep
+ * (csrc/discover.cuh).  Both calls run on the caller's stream without synchronising or allocating, in launches of at
+ * most 2^22 states.
+ * marks: DEVICE uint32 [max(1, 2^N / 32)], bit (s & 31) of word s >> 5 = state s.  *newly (DEVICE u64) is
+ * increased by the number of bits the call set.  Perturbation-free STG whatever the handle's perturb_p.
+ * N > PBN_DP_MAX_GENES: PBN_ERR_UNSUPPORTED; NULL marks / newly: PBN_ERR_INVALID. */
+/* Set the bits of states[0, n_states) (DEVICE u64, one index per state); states >= 2^N are ignored. */
+int pbn_reach_mark(pbn_handle* h, uint32_t* marks, const uint64_t* states, int64_t n_states,
+                   unsigned long long* newly, void* stream);
+/* One sweep over every unmarked state. */
+int pbn_reach_sweep(pbn_handle* h, uint32_t* marks, unsigned long long* newly, void* stream);
+
 /* ---- Exact optimal control: finite-horizon dynamic programming over every state (N <= PBN_DP_MAX_GENES) ----------
  * The env is a finite Markov decision process, so for networks whose 2^N states fit on the GPU the best possible policy
  * of a target can be computed exactly by backward induction -- the yardstick an agent's strategy lengths and returns are

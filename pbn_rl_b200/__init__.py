@@ -14,11 +14,12 @@ __all__ = [
     "sorted_id_permutation", "BoolFunction", "IsplError", "compile_expression", "logic_functions_from_ispl",
     "parse_ispl", "render_ispl", "PBNNetwork", "pack_states", "unpack_states", "VecPBNEnv",
     "solve_control", "ControlSolution", "TabularPolicy", "policy_values", "tabulate_policy", "expected_all_pairs",
-    "StateDistribution", "propagate", "stationary_distribution",
+    "StateDistribution", "propagate", "stationary_distribution", "find_attractors_exhaustive",
 ]
 
 _CONTROL = ("solve_control", "ControlSolution", "TabularPolicy", "policy_values", "tabulate_policy", "expected_all_pairs")
 _STEADY_STATE = ("StateDistribution", "propagate", "stationary_distribution")
+_DISCOVER = ("find_attractors_exhaustive",)
 
 
 def __getattr__(name):
@@ -35,4 +36,7 @@ def __getattr__(name):
     if name in _STEADY_STATE:
         from . import steady_state
         return getattr(steady_state, name)
+    if name in _DISCOVER:
+        from . import discover
+        return getattr(discover, name)
     raise AttributeError(name)

@@ -279,4 +279,87 @@ __global__ void __launch_bounds__(128) closure_reach_kernel(const __grid_constan
   }
 }
 
+// ---- exhaustive attractor search: backward reachability over every state (N <= PBN_DP_MAX_GENES) ----
+// marks holds one bit per state (bit s & 31 of word s >> 5).  The caller marks the states of the attractors known so
+// far (reach_mark_kernel); a sweep then marks every unmarked state one of whose successors is marked, and the caller
+// repeats sweeps until one marks nothing.  The result is the set of states that reach a known attractor -- the least
+// fixed point, whatever order the bits land in: a bit set early in a sweep may be seen later in the same sweep, which
+// only saves sweeps.  At p = 0 every state reaches a sink SCC and sink SCCs are closed, so a fixed point with every bit
+// set proves that the known attractors are all of them.  Successors are those of the perturbation-free STG, the
+// relation of successor_descriptor: a gene is free when some predictor yields 1 and some yields 0.
+
+// The valid state bits of a marks word: all 32, or the 2^N of the single partial word when N < 5.
+__device__ __forceinline__ uint32_t reach_valid_bits(int n_genes) {
+  return n_genes >= 5 ? 0xFFFFFFFFu : (1u << (1u << n_genes)) - 1u;
+}
+
+// One warp per marks word (32 states), words [w0, w0 + count); a word whose valid bits are all set is skipped.  For
+// each unmarked state s of the word, lane g < N evaluates gene g's predictors and two ballots give the fixed genes and
+// the free ones.  The free genes split into L (genes 0..4, inside one marks word) and H (genes 5 and up, which pick the
+// word): a successor t lies in word ((fixed | c) >> 5) for c a subset of H, at a bit of the mask M (lane b of a third
+// ballot: (b ^ fixed) & 31 & ~L == 0).  The lanes walk those 2^|H| words 32 at a time -- lane l takes the subset of
+// H's five lowest genes given by the bits of l, the remaining genes of H advance in the loop -- and stop at the first
+// word with a marked bit under M.  *newly gains the number of bits the sweep set.
+__global__ void __launch_bounds__(256) reach_sweep_kernel(const __grid_constant__ NetParams n, uint32_t* __restrict__ marks,
+                                                          uint32_t w0, uint32_t count,
+                                                          unsigned long long* __restrict__ newly) {
+  const uint32_t lane = threadIdx.x & 31u;
+  const uint32_t valid = reach_valid_bits(n.n_genes);
+  uint32_t set = 0;   // bits this warp set (counted by lane 0)
+  for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < count; i += (gridDim.x * blockDim.x) >> 5) {
+    const uint32_t w = w0 + i;
+    uint32_t todo = __shfl_sync(0xFFFFFFFFu, lane == 0 ? ~__ldcg(marks + w) & valid : 0u, 0);
+    while (todo) {
+      const uint32_t b = __ffs(todo) - 1;
+      todo &= todo - 1u;
+      const uint32_t s = (w << 5) | b;
+      bool can1 = false, can0 = false;
+      if ((int)lane < n.n_genes) {
+        const uint64_t st[1] = {s};
+        for (int f = n.func_offset[lane]; f < n.func_offset[lane + 1]; ++f) {
+          if (eval_func<1>(n, f, st)) can1 = true; else can0 = true;
+        }
+      }
+      const uint32_t one = __ballot_sync(0xFFFFFFFFu, can1), zero = __ballot_sync(0xFFFFFFFFu, can0);
+      const uint32_t fr = one & zero, fixed = one & ~zero;
+      const uint32_t m = __ballot_sync(0xFFFFFFFFu, ((lane ^ fixed) & 31u & ~fr) == 0u);
+      const uint32_t base = fixed >> 5, hw = fr >> 5;   // word index: base | (a subset of hw); base & hw = 0
+      uint32_t hhi = hw, clo = 0;
+      int k = 0;
+      for (; k < 5 && hhi; ++k) {
+        const uint32_t g = hhi & (0u - hhi);
+        hhi ^= g;
+        if ((lane >> k) & 1u) clo |= g;
+      }
+      const bool active = (lane >> k) == 0u;
+      bool hit = false;
+      uint32_t chi = 0;
+      do {
+        hit = __any_sync(0xFFFFFFFFu, active && (__ldcg(marks + (base | clo | chi)) & m) != 0u);
+        chi = (chi - hhi) & hhi;   // the next subset of hhi in increasing order; 0 again after the last
+      } while (!hit && chi != 0u);
+      if (hit && lane == 0) {
+        const uint32_t bit = 1u << b;
+        if (!(atomicOr(marks + w, bit) & bit)) ++set;
+      }
+    }
+  }
+  if (lane == 0 && set != 0u) atomicAdd(newly, (unsigned long long)set);
+}
+
+// Set the bits of states[0, n_states); states >= n_valid (= 2^N) are ignored.  *newly gains the number of bits set.
+__global__ void __launch_bounds__(256) reach_mark_kernel(uint32_t* __restrict__ marks, const uint64_t* __restrict__ states,
+                                                         int64_t n_states, uint64_t n_valid,
+                                                         unsigned long long* __restrict__ newly) {
+  uint32_t set = 0;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n_states; i += (int64_t)gridDim.x * blockDim.x) {
+    const uint64_t s = states[i];
+    if (s >= n_valid) continue;
+    const uint32_t bit = 1u << (s & 31u);
+    if (!(atomicOr(marks + (s >> 5), bit) & bit)) ++set;
+  }
+  set = __reduce_add_sync(0xFFFFFFFFu, set);
+  if ((threadIdx.x & 31u) == 0 && set != 0u) atomicAdd(newly, (unsigned long long)set);
+}
+
 }  // namespace pbn

@@ -1667,4 +1667,45 @@ int pbn_dp_improve(pbn_handle* h, const double* w, uint64_t flip_genes, int32_t 
   return PBN_OK;
 }
 
+// ---- exhaustive attractor search: backward reachability over a bitset of every state (discover.cuh) ----
+static int reach_args(const pbn_handle* h, const char* who, const uint32_t* marks, const unsigned long long* newly) {
+  if (!h) return fail(PBN_ERR_INVALID, "%s: null handle", who);
+  if (h->net.n_genes > PBN_DP_MAX_GENES)
+    return fail(PBN_ERR_UNSUPPORTED, "%s: %d genes, the state bitset covers at most %d", who, h->net.n_genes, PBN_DP_MAX_GENES);
+  if (!marks || !newly) return fail(PBN_ERR_INVALID, "%s: null marks or newly", who);
+  return PBN_OK;
+}
+
+int pbn_reach_mark(pbn_handle* h, uint32_t* marks, const uint64_t* states, int64_t n_states, unsigned long long* newly,
+                   void* stream_) {
+  int rc;
+  if ((rc = reach_args(h, "pbn_reach_mark", marks, newly)) != PBN_OK) return rc;
+  if (n_states < 0 || (n_states > 0 && !states)) return fail(PBN_ERR_INVALID, "pbn_reach_mark: bad state list");
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  for (int64_t i0 = 0; i0 < n_states; i0 += kDpSliceStates) {
+    const int64_t cnt = n_states - i0 < (int64_t)kDpSliceStates ? n_states - i0 : (int64_t)kDpSliceStates;
+    if ((rc = launch(h, reach_mark_kernel, grid_for(h, cnt, 256, 8), 256, 0, stream, false, marks, states + i0, cnt,
+                     (uint64_t)1 << h->net.n_genes, newly)) != PBN_OK)
+      return rc;
+  }
+  return PBN_OK;
+}
+
+int pbn_reach_sweep(pbn_handle* h, uint32_t* marks, unsigned long long* newly, void* stream_) {
+  int rc;
+  if ((rc = reach_args(h, "pbn_reach_sweep", marks, newly)) != PBN_OK) return rc;
+  const uint32_t S = 1u << h->net.n_genes;
+  const uint32_t words = S > 32u ? S >> 5 : 1u, per = kDpSliceStates >> 5;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  DeviceGuard guard(h->device);
+  for (uint32_t w0 = 0; w0 < words; w0 += per) {
+    const uint32_t cnt = words - w0 < per ? words - w0 : per;
+    if ((rc = launch(h, reach_sweep_kernel, grid_for(h, (int64_t)cnt * 32, 256, 8), 256, 0, stream, false, h->net, marks,
+                     w0, cnt, newly)) != PBN_OK)
+      return rc;
+  }
+  return PBN_OK;
+}
+
 }  // extern "C"

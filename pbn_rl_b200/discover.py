@@ -13,6 +13,9 @@ Here:
   relation (successor descriptors from ``pbn_successor_sets``).  A closed set's sink SCCs are sink SCCs of
   the whole STG, so every attractor returned is exact (closed and strongly connected); what is sampled is
   only *which* attractors are found (those with a basin the rollouts hit).
+* :func:`find_attractors_exhaustive` -- for N <= 28: all attractors, with a certificate.  Backward reachability
+  over a device bitset of all 2^N states (``pbn_reach_sweep``) from the attractors found so far; states that stay
+  unmarked are closed under successors and hold the attractors not found yet, which rollouts from them find.
 * :func:`steady_state_histogram` -- visit counts of (projected) states over many perturbed steps.
 * :func:`steady_state_statistics` / :class:`StateRecorder` -- per-gene ON frequencies and the distribution of the
   state projected onto up to 12 genes, counted on the device (``pbn_rollout_record`` inside the rollout kernel,
@@ -26,13 +29,15 @@ from typing import Callable, Dict, List, Optional, Sequence, Tuple, Union
 import numpy as np
 import torch
 
+from . import _cabi
 from ._cabi import check
 from .attractors import AttractorSet
 from .network import PBNNetwork
 from .vec_env import VecPBNEnv
 
 __all__ = ["VisitCounter", "find_attractors_rollout", "attractor_reached_from", "basin_labels", "steady_state_histogram", "successor_descriptors",
-           "forward_closure", "sink_sccs_of_closed_set", "StateRecorder", "steady_state_statistics"]
+           "forward_closure", "sink_sccs_of_closed_set", "StateRecorder", "steady_state_statistics",
+           "ReachMarks", "find_attractors_exhaustive"]
 
 
 def _words_to_int(words: Sequence[int]) -> int:
@@ -315,6 +320,151 @@ def find_attractors_rollout(network: PBNNetwork, n_rollouts: int = 1 << 16, burn
     info = {"n_rollouts": e, "burn_in": int(burn_in), "distinct_end_states": int(len(counts)),
             "basin_fraction": [hits[i] / e for i in perm], "unresolved": unresolved,
             "states": [attractors[i] for i in perm]}
+    return AttractorSet(attrs, n), info
+
+
+class ReachMarks:
+    """Device bitset of every state of ``env``'s network (N <= 28; ``pbn_reach_mark`` / ``pbn_reach_sweep``): bit
+    ``s & 31`` of word ``s >> 5`` of :attr:`marks` is state ``s``.  :meth:`mark` sets the states of a list;
+    :meth:`close` sweeps "mark ``s`` if a successor of ``s`` (perturbation-free STG) is marked" until a sweep marks
+    nothing, which leaves exactly the states that reach a marked one.  :attr:`count` is the number of marked states."""
+
+    def __init__(self, env: VecPBNEnv):
+        n = env.n_genes
+        if n > _cabi.DP_MAX_GENES:
+            raise _cabi.PbnError(_cabi.PBN_ERR_UNSUPPORTED, "the state bitset covers at most %d genes, the network has %d"
+                                 % (_cabi.DP_MAX_GENES, n))
+        self.env, self.n = env, n
+        self.marks = torch.zeros((max(1, (1 << n) >> 5),), dtype=torch.int32, device=env.device)
+        self.newly = torch.zeros((1,), dtype=torch.int64, device=env.device)
+        self.count = 0
+        self.sweeps = 0
+
+    def mark(self, states: Sequence[int]) -> int:
+        """Set the bits of ``states``; returns how many were not set before."""
+        env = self.env
+        st = torch.as_tensor(np.asarray(list(states), dtype=np.int64)).to(env.device)
+        self.newly.zero_()
+        check(env.lib.pbn_reach_mark(env._h, self.marks.data_ptr(), st.data_ptr(), st.shape[0], self.newly.data_ptr(),
+                                     env._stream()))
+        k = int(self.newly.item())
+        self.count += k
+        return k
+
+    def sweep(self) -> int:
+        """One sweep; returns the number of states it marked."""
+        env = self.env
+        self.newly.zero_()
+        check(env.lib.pbn_reach_sweep(env._h, self.marks.data_ptr(), self.newly.data_ptr(), env._stream()))
+        self.sweeps += 1
+        k = int(self.newly.item())
+        self.count += k
+        return k
+
+    def close(self) -> int:
+        """Sweep to the fixed point; returns the number of states marked on the way."""
+        total = 0
+        while True:
+            k = self.sweep()
+            if k == 0:
+                return total
+            total += k
+
+    @property
+    def uncovered(self) -> int:
+        return (1 << self.n) - self.count
+
+    def unmarked_sample(self, k: int) -> List[int]:
+        """At most ``k`` unmarked states, deterministically: the lowest unmarked state of ``k`` words spread evenly
+        over the words that hold one."""
+        valid = 0xFFFFFFFF if self.n >= 5 else (1 << (1 << self.n)) - 1
+        free = (~self.marks) & (valid - (1 << 32) if valid >= 1 << 31 else valid)
+        words = torch.nonzero(free != 0).reshape(-1)
+        if words.numel() == 0:
+            return []
+        pick = torch.linspace(0, words.numel() - 1, min(int(k), words.numel()), dtype=torch.float64, device=words.device).round().long()
+        words = torch.unique(words[pick])
+        bits = (free[words].to(torch.int64) & 0xFFFFFFFF).cpu().tolist()
+        return [(int(w) << 5) | ((b & -b).bit_length() - 1) for w, b in zip(words.cpu().tolist(), bits)]
+
+
+def find_attractors_exhaustive(network: PBNNetwork, device: Union[str, torch.device] = "cuda:0",
+                               seed_rollouts: int = 1 << 16, burn_in: int = 256, max_attractor_states: int = 1 << 14,
+                               seed: int = 0x5EED, max_unresolved: int = 8):
+    """Every attractor (sink SCC of the perturbation-free STG) of a network of up to 28 genes, with a certificate.
+
+    1. Seed: :func:`find_attractors_rollout` with ``seed_rollouts`` rollouts (0: none); the states of its attractors
+       are marked in a device bitset of all 2^N states (:class:`ReachMarks`).
+    2. Sweep: backward reachability to the marked states, to its fixed point.
+    3. Discover: if states stay unmarked, they are closed under successors and hold an attractor not found yet.  Up to
+       1024 of them (a deterministic sample) roll out ``burn_in`` perturbation-free updates and
+       :func:`attractor_reached_from` finds the attractor of each distinct end state; the new attractors are marked and
+       the search goes back to 2.
+    4. Stop when every state is marked (``complete=True``: every state reaches a listed attractor, so no other one
+       exists), or when a round finds no new attractor because every closure exceeded ``max_attractor_states`` or the
+       closure's free-gene limit (``complete=False``, with what was found).  A round stops trying end states after
+       ``max_unresolved`` failed closures (the end states of one attractor that is too large all fail alike).
+
+    Returns ``(AttractorSet, info)`` sorted as :func:`find_attractors_stg` sorts (states ascending inside an attractor,
+    attractors by their smallest state); ``info`` holds ``complete``, ``uncovered`` (states left unmarked), ``sweeps``,
+    ``rounds`` (discovery rounds; ``sweeps`` may differ from run to run, since a bit set early in a sweep can be seen
+    later in the same sweep, but the marks and the attractors do not), ``seeded`` (attractors the seeding found) and ``states`` (member lists).
+    N > 28 raises ``PbnError(PBN_ERR_UNSUPPORTED)``."""
+    n = network.n_genes
+    if n > _cabi.DP_MAX_GENES:
+        raise _cabi.PbnError(_cabi.PBN_ERR_UNSUPPORTED, "exhaustive attractor search covers at most %d genes, the network "
+                             "has %d" % (_cabi.DP_MAX_GENES, n))
+    attractors: List[List[int]] = []
+    if int(seed_rollouts) > 0:
+        _, rinfo = find_attractors_rollout(network, n_rollouts=int(seed_rollouts), burn_in=burn_in, device=device,
+                                           seed=seed, max_attractor_states=max_attractor_states)
+        attractors = [list(m) for m in rinfo["states"]]
+    seeded = len(attractors)
+    e = 1024
+    env = VecPBNEnv(network, e, None, device=device, seed=seed, horizon=0, bins=1, perturb_p=0.0)
+    try:
+        reach = ReachMarks(env)
+        owner = set()
+        for m in attractors:
+            owner.update(m)
+            reach.mark(m)
+        ws = _ClosureWorkspace(env, max_attractor_states)
+        rounds = 0
+        while True:
+            reach.close()
+            if reach.uncovered == 0:
+                break
+            starts = reach.unmarked_sample(e)
+            rounds += 1
+            st = torch.tensor(starts + [starts[0]] * (e - len(starts)), dtype=torch.int64).reshape(e, 1)
+            env.set_state(st, packed=True)
+            env.rollout(int(burn_in), stats=False)
+            ends = torch.unique(env.state[:, 0]).cpu().tolist()
+            found = failed = 0
+            for s in ends:
+                if s in owner:
+                    continue
+                members = attractor_reached_from(env, int(s), ws, max_states=max_attractor_states)
+                if members is None:
+                    failed += 1
+                    if failed >= max_unresolved:
+                        break
+                    continue
+                if members[0] in owner:
+                    continue
+                attractors.append(members)
+                owner.update(members)
+                reach.mark(members)
+                found += 1
+            if found == 0:
+                break
+        info = {"complete": reach.uncovered == 0, "uncovered": reach.uncovered, "sweeps": reach.sweeps,
+                "rounds": rounds, "seeded": seeded}
+    finally:
+        env.close()
+    attractors.sort(key=lambda m: m[0])
+    info["states"] = attractors
+    attrs = [[tuple((s >> i) & 1 for i in range(n)) for s in m] for m in attractors]
     return AttractorSet(attrs, n), info
 
 
