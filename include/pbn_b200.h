@@ -466,7 +466,7 @@ int pbn_closure_reach(pbn_handle* h, const uint64_t* list, int64_t count, uint8_
                       const unsigned long long* tags, const uint64_t* slot_state,
                       const unsigned long long* slot_index, int64_t capacity, int32_t* changed, void* stream);
 
-/* ---- Exhaustive attractor search: backward reachability over every state (N <= PBN_DP_MAX_GENES) ----------------
+/* ---- Exhaustive attractor search: backward reachability over every state (N <= PBN_REACH_MAX_GENES) -------------
  * Without perturbation every state reaches an attractor (a sink SCC of the STG above) and attractors are closed.  So
  * mark the states of the attractors found so far (pbn_reach_mark) and repeat pbn_reach_sweep -- "mark s if some
  * successor of s is marked" -- until a sweep marks nothing: if every state is then marked, no other attractor exists;
@@ -476,7 +476,9 @@ int pbn_closure_reach(pbn_handle* h, const uint64_t* list, int64_t count, uint8_
  * most 2^22 states.
  * marks: DEVICE uint32 [max(1, 2^N / 32)], bit (s & 31) of word s >> 5 = state s.  *newly (DEVICE u64) is
  * increased by the number of bits the call set.  Perturbation-free STG whatever the handle's perturb_p.
- * N > PBN_DP_MAX_GENES: PBN_ERR_UNSUPPORTED; NULL marks / newly: PBN_ERR_INVALID. */
+ * N > PBN_REACH_MAX_GENES: PBN_ERR_UNSUPPORTED; NULL marks / newly: PBN_ERR_INVALID.
+ * The limit is not the DP's: the bitset needs one bit per state (2 GiB at 34 genes). */
+#define PBN_REACH_MAX_GENES 34
 /* Set the bits of states[0, n_states) (DEVICE u64, one index per state); states >= 2^N are ignored. */
 int pbn_reach_mark(pbn_handle* h, uint32_t* marks, const uint64_t* states, int64_t n_states,
                    unsigned long long* newly, void* stream);

@@ -18,6 +18,7 @@ PBN_OK = 0
 PBN_ERR_INVALID = -1
 PBN_ERR_UNSUPPORTED = -3
 DP_MAX_GENES = 28  # PBN_DP_MAX_GENES
+REACH_MAX_GENES = 34  # PBN_REACH_MAX_GENES
 PERT_MODES = {"none": 0, "A": 1, "B": 2, "C": 3}
 KERNEL_KINDS = {"auto": 0, "scalar": 1, "sliced": 2}
 STEP_AUTORESET = 1

@@ -279,7 +279,7 @@ __global__ void __launch_bounds__(128) closure_reach_kernel(const __grid_constan
   }
 }
 
-// ---- exhaustive attractor search: backward reachability over every state (N <= PBN_DP_MAX_GENES) ----
+// ---- exhaustive attractor search: backward reachability over every state (N <= PBN_REACH_MAX_GENES) ----
 // marks holds one bit per state (bit s & 31 of word s >> 5).  The caller marks the states of the attractors known so
 // far (reach_mark_kernel); a sweep then marks every unmarked state one of whose successors is marked, and the caller
 // repeats sweeps until one marks nothing.  The result is the set of states that reach a known attractor -- the least
@@ -293,13 +293,30 @@ __device__ __forceinline__ uint32_t reach_valid_bits(int n_genes) {
   return n_genes >= 5 ? 0xFFFFFFFFu : (1u << (1u << n_genes)) - 1u;
 }
 
+// Ballots over the warp of whether some predictor of the lane's gene g sets it to 1 / to 0 in state st (g >= N: neither).
+__device__ __forceinline__ void reach_gene_ballots(const NetParams& n, const uint64_t (&st)[1], int g, uint32_t& one,
+                                                   uint32_t& zero) {
+  bool can1 = false, can0 = false;
+  if (g < n.n_genes) {
+    for (int f = n.func_offset[g]; f < n.func_offset[g + 1]; ++f) {
+      if (eval_func<1>(n, f, st)) can1 = true; else can0 = true;
+    }
+  }
+  one = __ballot_sync(0xFFFFFFFFu, can1);
+  zero = __ballot_sync(0xFFFFFFFFu, can0);
+}
+
 // One warp per marks word (32 states), words [w0, w0 + count); a word whose valid bits are all set is skipped.  For
-// each unmarked state s of the word, lane g < N evaluates gene g's predictors and two ballots give the fixed genes and
-// the free ones.  The free genes split into L (genes 0..4, inside one marks word) and H (genes 5 and up, which pick the
-// word): a successor t lies in word ((fixed | c) >> 5) for c a subset of H, at a bit of the mask M (lane b of a third
-// ballot: (b ^ fixed) & 31 & ~L == 0).  The lanes walk those 2^|H| words 32 at a time -- lane l takes the subset of
-// H's five lowest genes given by the bits of l, the remaining genes of H advance in the loop -- and stop at the first
-// word with a marked bit under M.  *newly gains the number of bits the sweep set.
+// each unmarked state s of the word, lane g evaluates gene g's predictors (and gene g + 32's in a second pass in the
+// kWide instance, for 32 < N <= 37) and ballots give the fixed genes and the free ones.  The free genes split into L
+// (genes 0..4, inside one marks word) and H (genes 5 and up, which pick the word): a successor t lies in word
+// ((fixed | c) >> 5) for c a subset of H, at a bit of the mask M (lane b of a third ballot:
+// (b ^ fixed) & 31 & ~L == 0).  The lanes walk those 2^|H| words 32 at a time -- lane l takes the subset of H's five
+// lowest genes given by the bits of l, the remaining genes of H advance in the loop -- and stop at the first word with
+// a marked bit under M.  *newly gains the number of bits the sweep set.
+// Word indices (at most 2^(N-5)) stay u32 up to N = 37.  The narrow instance (N <= 32) keeps 32-bit state indices;
+// it is the faster of the two at 28 genes (DESIGN.md §3.8).
+template <bool kWide>
 __global__ void __launch_bounds__(256) reach_sweep_kernel(const __grid_constant__ NetParams n, uint32_t* __restrict__ marks,
                                                           uint32_t w0, uint32_t count,
                                                           unsigned long long* __restrict__ newly) {
@@ -312,18 +329,14 @@ __global__ void __launch_bounds__(256) reach_sweep_kernel(const __grid_constant_
     while (todo) {
       const uint32_t b = __ffs(todo) - 1;
       todo &= todo - 1u;
-      const uint32_t s = (w << 5) | b;
-      bool can1 = false, can0 = false;
-      if ((int)lane < n.n_genes) {
-        const uint64_t st[1] = {s};
-        for (int f = n.func_offset[lane]; f < n.func_offset[lane + 1]; ++f) {
-          if (eval_func<1>(n, f, st)) can1 = true; else can0 = true;
-        }
-      }
-      const uint32_t one = __ballot_sync(0xFFFFFFFFu, can1), zero = __ballot_sync(0xFFFFFFFFu, can0);
-      const uint32_t fr = one & zero, fixed = one & ~zero;
+      const uint64_t st[1] = {kWide ? ((uint64_t)w << 5) | b : (uint64_t)((w << 5) | b)};
+      uint32_t one_lo, zero_lo, one_hi = 0, zero_hi = 0;
+      reach_gene_ballots(n, st, (int)lane, one_lo, zero_lo);
+      if (kWide) reach_gene_ballots(n, st, (int)lane + 32, one_hi, zero_hi);
+      const uint32_t fr = one_lo & zero_lo, fixed = one_lo & ~zero_lo;
       const uint32_t m = __ballot_sync(0xFFFFFFFFu, ((lane ^ fixed) & 31u & ~fr) == 0u);
-      const uint32_t base = fixed >> 5, hw = fr >> 5;   // word index: base | (a subset of hw); base & hw = 0
+      // word index: base | (a subset of hw); base & hw = 0.  Gene g >= 5 is bit g - 5: genes 32.. are bits 27..
+      const uint32_t base = (fixed >> 5) | ((one_hi & ~zero_hi) << 27), hw = (fr >> 5) | ((one_hi & zero_hi) << 27);
       uint32_t hhi = hw, clo = 0;
       int k = 0;
       for (; k < 5 && hhi; ++k) {

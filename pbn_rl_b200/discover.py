@@ -13,7 +13,7 @@ Here:
   relation (successor descriptors from ``pbn_successor_sets``).  A closed set's sink SCCs are sink SCCs of
   the whole STG, so every attractor returned is exact (closed and strongly connected); what is sampled is
   only *which* attractors are found (those with a basin the rollouts hit).
-* :func:`find_attractors_exhaustive` -- for N <= 28: all attractors, with a certificate.  Backward reachability
+* :func:`find_attractors_exhaustive` -- for N <= 34: all attractors, with a certificate.  Backward reachability
   over a device bitset of all 2^N states (``pbn_reach_sweep``) from the attractors found so far; states that stay
   unmarked are closed under successors and hold the attractors not found yet, which rollouts from them find.
 * :func:`steady_state_histogram` -- visit counts of (projected) states over many perturbed steps.
@@ -324,16 +324,16 @@ def find_attractors_rollout(network: PBNNetwork, n_rollouts: int = 1 << 16, burn
 
 
 class ReachMarks:
-    """Device bitset of every state of ``env``'s network (N <= 28; ``pbn_reach_mark`` / ``pbn_reach_sweep``): bit
-    ``s & 31`` of word ``s >> 5`` of :attr:`marks` is state ``s``.  :meth:`mark` sets the states of a list;
+    """Device bitset of every state of ``env``'s network (N <= 34, 2 GiB at 34 genes; ``pbn_reach_mark`` /
+    ``pbn_reach_sweep``): bit ``s & 31`` of word ``s >> 5`` of :attr:`marks` is state ``s``.  :meth:`mark` sets the states of a list;
     :meth:`close` sweeps "mark ``s`` if a successor of ``s`` (perturbation-free STG) is marked" until a sweep marks
     nothing, which leaves exactly the states that reach a marked one.  :attr:`count` is the number of marked states."""
 
     def __init__(self, env: VecPBNEnv):
         n = env.n_genes
-        if n > _cabi.DP_MAX_GENES:
+        if n > _cabi.REACH_MAX_GENES:
             raise _cabi.PbnError(_cabi.PBN_ERR_UNSUPPORTED, "the state bitset covers at most %d genes, the network has %d"
-                                 % (_cabi.DP_MAX_GENES, n))
+                                 % (_cabi.REACH_MAX_GENES, n))
         self.env, self.n = env, n
         self.marks = torch.zeros((max(1, (1 << n) >> 5),), dtype=torch.int32, device=env.device)
         self.newly = torch.zeros((1,), dtype=torch.int64, device=env.device)
@@ -376,22 +376,37 @@ class ReachMarks:
 
     def unmarked_sample(self, k: int) -> List[int]:
         """At most ``k`` unmarked states, deterministically: the lowest unmarked state of ``k`` words spread evenly
-        over the words that hold one."""
+        over the words that hold one.  The bitset is read in chunks of 2^22 words (16 MiB), twice: once to count the
+        words that hold an unmarked state, once to fetch the chosen ones."""
         valid = 0xFFFFFFFF if self.n >= 5 else (1 << (1 << self.n)) - 1
-        free = (~self.marks) & (valid - (1 << 32) if valid >= 1 << 31 else valid)
-        words = torch.nonzero(free != 0).reshape(-1)
-        if words.numel() == 0:
+        valid = valid - (1 << 32) if valid >= 1 << 31 else valid          # as an int32
+        chunk = 1 << 22
+        starts = range(0, self.marks.numel(), chunk)
+        free = lambda c: (~self.marks[c:c + chunk]) & valid
+        per = torch.stack([torch.count_nonzero(free(c)) for c in starts]).cpu().tolist()
+        total = sum(per)
+        if total == 0:
             return []
-        pick = torch.linspace(0, words.numel() - 1, min(int(k), words.numel()), dtype=torch.float64, device=words.device).round().long()
-        words = torch.unique(words[pick])
-        bits = (free[words].to(torch.int64) & 0xFFFFFFFF).cpu().tolist()
-        return [(int(w) << 5) | ((b & -b).bit_length() - 1) for w, b in zip(words.cpu().tolist(), bits)]
+        pick = torch.linspace(0, total - 1, min(int(k), total), dtype=torch.float64, device=self.marks.device).round().long()
+        pick = torch.unique(pick).cpu()           # ranks among the words that hold an unmarked state, ascending
+        out: List[int] = []
+        first = 0
+        for c, cnt in zip(starts, per):
+            sel = pick[(pick >= first) & (pick < first + cnt)] - first
+            first += cnt
+            if sel.numel() == 0:
+                continue
+            f = free(c)
+            words = torch.nonzero(f != 0).reshape(-1)[sel.to(f.device)]
+            bits = (f[words].to(torch.int64) & 0xFFFFFFFF).cpu().tolist()
+            out += [((c + int(w)) << 5) | ((b & -b).bit_length() - 1) for w, b in zip(words.cpu().tolist(), bits)]
+        return out
 
 
 def find_attractors_exhaustive(network: PBNNetwork, device: Union[str, torch.device] = "cuda:0",
                                seed_rollouts: int = 1 << 16, burn_in: int = 256, max_attractor_states: int = 1 << 14,
                                seed: int = 0x5EED, max_unresolved: int = 8):
-    """Every attractor (sink SCC of the perturbation-free STG) of a network of up to 28 genes, with a certificate.
+    """Every attractor (sink SCC of the perturbation-free STG) of a network of up to 34 genes, with a certificate.
 
     1. Seed: :func:`find_attractors_rollout` with ``seed_rollouts`` rollouts (0: none); the states of its attractors
        are marked in a device bitset of all 2^N states (:class:`ReachMarks`).
@@ -409,11 +424,12 @@ def find_attractors_exhaustive(network: PBNNetwork, device: Union[str, torch.dev
     attractors by their smallest state); ``info`` holds ``complete``, ``uncovered`` (states left unmarked), ``sweeps``,
     ``rounds`` (discovery rounds; ``sweeps`` may differ from run to run, since a bit set early in a sweep can be seen
     later in the same sweep, but the marks and the attractors do not), ``seeded`` (attractors the seeding found) and ``states`` (member lists).
-    N > 28 raises ``PbnError(PBN_ERR_UNSUPPORTED)``."""
+    The bitset takes 2^N / 8 bytes of device memory: 32 MiB at 28 genes, 2 GiB at 34.
+    N > 34 raises ``PbnError(PBN_ERR_UNSUPPORTED)``."""
     n = network.n_genes
-    if n > _cabi.DP_MAX_GENES:
+    if n > _cabi.REACH_MAX_GENES:
         raise _cabi.PbnError(_cabi.PBN_ERR_UNSUPPORTED, "exhaustive attractor search covers at most %d genes, the network "
-                             "has %d" % (_cabi.DP_MAX_GENES, n))
+                             "has %d" % (_cabi.REACH_MAX_GENES, n))
     attractors: List[List[int]] = []
     if int(seed_rollouts) > 0:
         _, rinfo = find_attractors_rollout(network, n_rollouts=int(seed_rollouts), burn_in=burn_in, device=device,

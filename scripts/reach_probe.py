@@ -11,7 +11,13 @@ the 20-gene network again with a closure limit of 2^20 states:
 4. Bittner-28 only: one pbn_dp_expect at p = 0, for comparison with a sweep.
 Writes <out>/r08_reach_probe.json; the card's name and power limit are read in the same run.
 
-    python scripts/reach_probe.py [--out profiles]
+--wide: above 28 genes, where the bitset (1 GiB at 33 genes, 2 GiB at 34) no longer fits the L2.  Bittner-28 again as
+the reference, bb33 (33 genes, one predictor per gene) and trap_network(34) (tests/test_gpu_reach_wide.py: three of its
+six attractors have basins of one or two states, which the seeding rollouts miss).  Steps 1, 2 and 4 as above, plus the
+first sweep's device time per state; step 3 is left out, since at 34 genes it would sweep a quarter of the states
+that walk their whole successor sets, several times.  Writes <out>/r09_reach_wide_probe.json.
+
+    python scripts/reach_probe.py [--out profiles] [--wide]
 """
 import argparse
 import json
@@ -50,7 +56,7 @@ def sweep_times(env, seeds):
             return out, reach
 
 
-def case(name, net, **kw):
+def case(name, net, partial=True, **kw):
     from pbn_rl_b200 import VecPBNEnv
     from pbn_rl_b200.discover import find_attractors_exhaustive, find_attractors_rollout
     rec = {"case": name, "n_genes": net.n_genes, "args": kw}
@@ -72,9 +78,10 @@ def case(name, net, **kw):
     full, reach = sweep_times(env, [s for m in states for s in m])
     rec["cover_sweeps"] = [{"s": t, "marked": k} for t, k in full]
     rec["cover_device_s"] = sum(t for t, _ in full)
+    rec["first_sweep_ns_per_state"] = full[0][0] / (1 << net.n_genes) * 1e9
     rec["covered"] = reach.count
     rec["skip_sweep_s"] = timed(reach.sweep)[0]
-    if len(states) > 1:
+    if partial and len(states) > 1:
         big = max(range(len(rinfo["states"])), key=lambda i: rinfo["basin_fraction"][i])
         left = rinfo["states"][big]
         part, reach = sweep_times(env, [s for m in states if m != left for s in m])
@@ -99,20 +106,29 @@ def case(name, net, **kw):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--out", default=str(ROOT / "profiles"))
+    ap.add_argument("--wide", action="store_true", help="Bittner-28, bb33 and trap_network(34): r09_reach_wide_probe.json")
     args = ap.parse_args()
-    from helpers import make_network, product_net
+    from helpers import GOLD, make_network, product_net
     from pbn_rl_b200 import PBNNetwork
     pbn28 = product_net("pbn28")
-    net20 = PBNNetwork.from_expressions(*make_network(20, 3, 4, seed=20))
-    net24 = PBNNetwork.from_expressions(*make_network(24, 2, 3, seed=24))
-    runs = [("Bittner-28", pbn28, {}), ("make_network(20, 3, 4, seed=20)", net20, {}),
-            ("make_network(24, 2, 3, seed=24)", net24, {}),
-            ("make_network(20, 3, 4, seed=20)", net20, {"max_attractor_states": 1 << 20})]
+    if args.wide:
+        from pbn_rl_b200.formats import network_from_bnet
+        from test_gpu_reach_wide import trap_network
+        runs = [("Bittner-28", pbn28, {}), ("bb33", network_from_bnet(GOLD / "bb33.bnet"), {"partial": False}),
+                ("trap_network(34)", PBNNetwork.from_expressions(*trap_network(34)), {"partial": False})]
+        fname = "r09_reach_wide_probe.json"
+    else:
+        net20 = PBNNetwork.from_expressions(*make_network(20, 3, 4, seed=20))
+        net24 = PBNNetwork.from_expressions(*make_network(24, 2, 3, seed=24))
+        runs = [("Bittner-28", pbn28, {}), ("make_network(20, 3, 4, seed=20)", net20, {}),
+                ("make_network(24, 2, 3, seed=24)", net24, {}),
+                ("make_network(20, 3, 4, seed=20)", net20, {"max_attractor_states": 1 << 20})]
+        fname = "r08_reach_probe.json"
     out = {"card": card(), "torch": torch.__version__, "cases": []}
     Path(args.out).mkdir(parents=True, exist_ok=True)
     for name, net, kw in runs:   # the file is rewritten after every case
         out["cases"].append(case(name, net, **kw))
-        (Path(args.out) / "r08_reach_probe.json").write_text(json.dumps(out, indent=1) + "\n")
+        (Path(args.out) / fname).write_text(json.dumps(out, indent=1) + "\n")
 
 
 if __name__ == "__main__":
