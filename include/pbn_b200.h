@@ -484,6 +484,13 @@ int pbn_reach_mark(pbn_handle* h, uint32_t* marks, const uint64_t* states, int64
                    unsigned long long* newly, void* stream);
 /* One sweep over every unmarked state. */
 int pbn_reach_sweep(pbn_handle* h, uint32_t* marks, unsigned long long* newly, void* stream);
+/* Forward closure: one sweep that expands every state of `set` not yet in `done` (both DEVICE uint32 bitsets in the
+ * marks layout): the bits of all its successors are set in `set`, and the state's bit in `done`.  Repeated until a
+ * sweep expands nothing, `set` is the forward closure of its initial bits and `done` equals it.  newly: DEVICE u64 [2],
+ * increased by the number of bits set in `set` and by the number of states expanded.  Bitsets of 2^N / 8 bytes, one
+ * bit per state, whatever the closure's size or its states' free genes.  Same refusals as pbn_reach_sweep (NULL
+ * done: PBN_ERR_INVALID). */
+int pbn_reach_forward(pbn_handle* h, uint32_t* set, uint32_t* done, unsigned long long* newly, void* stream);
 
 /* ---- Exact optimal control: finite-horizon dynamic programming over every state (N <= PBN_DP_MAX_GENES) ----------
  * The env is a finite Markov decision process, so for networks whose 2^N states fit on the GPU the best possible policy

@@ -41,7 +41,7 @@ EXPORTS = (
     "pbn_resident_words", "pbn_resident_import", "pbn_resident_export", "pbn_reward_table", "pbn_attractor_hash_slots",
     "pbn_per_tree_floats", "pbn_per_init", "pbn_per_push", "pbn_per_update", "pbn_per_sample",
     "pbn_dp_workspace_bytes", "pbn_dp_expect", "pbn_dp_improve", "pbn_dp_push",
-    "pbn_reach_mark", "pbn_reach_sweep",
+    "pbn_reach_mark", "pbn_reach_sweep", "pbn_reach_forward",
 )
 
 
@@ -219,6 +219,8 @@ def load_library(path: Optional[os.PathLike] = None) -> C.CDLL:
     lib.pbn_reach_mark.restype = C.c_int
     lib.pbn_reach_sweep.argtypes = [vp, vp, vp, vp]
     lib.pbn_reach_sweep.restype = C.c_int
+    lib.pbn_reach_forward.argtypes = [vp, vp, vp, vp, vp]
+    lib.pbn_reach_forward.restype = C.c_int
     lib.pbn_attractor_hash_slots.argtypes = [vp]
     lib.pbn_attractor_hash_slots.restype = C.c_int
     lib.pbn_reward_table.argtypes = [vp, vp, i32]

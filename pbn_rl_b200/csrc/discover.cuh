@@ -360,6 +360,62 @@ __global__ void __launch_bounds__(256) reach_sweep_kernel(const __grid_constant_
   if (lane == 0 && set != 0u) atomicAdd(newly, (unsigned long long)set);
 }
 
+// One sweep of forward reachability over two bitsets of every state: set (reached) and done (already expanded), both in
+// the marks layout.  One warp per word, words [w0, w0 + count): each state of set[w] & ~done[w] is expanded -- the
+// ballots, base, H and M of reach_sweep_kernel -- and every word of its successor set gets atomicOr(set + word, M), issued
+// only when a plain read shows a bit of M missing.  The warp then records the expanded states in done[w]; only this warp
+// writes done[w] within a sweep.  A state set earlier in the same sweep may be expanded later in it, which only saves
+// sweeps.  The caller repeats sweeps until one expands nothing: set is then the forward closure of its initial bits and
+// each of its states was expanded exactly once.  newly[0] gains the number of bits set, newly[1] the states expanded.
+template <bool kWide>
+__global__ void __launch_bounds__(256) reach_forward_kernel(const __grid_constant__ NetParams n, uint32_t* __restrict__ set,
+                                                            uint32_t* __restrict__ done, uint32_t w0, uint32_t count,
+                                                            unsigned long long* __restrict__ newly) {
+  const uint32_t lane = threadIdx.x & 31u;
+  const uint32_t valid = reach_valid_bits(n.n_genes);
+  unsigned long long reached = 0;   // bits this lane set
+  uint32_t expanded = 0;            // states this warp expanded (counted by lane 0)
+  for (uint32_t i = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; i < count; i += (gridDim.x * blockDim.x) >> 5) {
+    const uint32_t w = w0 + i;
+    const uint32_t d = lane == 0 ? __ldcg(done + w) : 0u;
+    const uint32_t take = __shfl_sync(0xFFFFFFFFu, lane == 0 ? __ldcg(set + w) & ~d & valid : 0u, 0);
+    if (take == 0u) continue;
+    uint32_t todo = take;
+    while (todo) {
+      const uint32_t b = __ffs(todo) - 1;
+      todo &= todo - 1u;
+      const uint64_t st[1] = {kWide ? ((uint64_t)w << 5) | b : (uint64_t)((w << 5) | b)};
+      uint32_t one_lo, zero_lo, one_hi = 0, zero_hi = 0;
+      reach_gene_ballots(n, st, (int)lane, one_lo, zero_lo);
+      if (kWide) reach_gene_ballots(n, st, (int)lane + 32, one_hi, zero_hi);
+      const uint32_t fr = one_lo & zero_lo, fixed = one_lo & ~zero_lo;
+      const uint32_t m = __ballot_sync(0xFFFFFFFFu, ((lane ^ fixed) & 31u & ~fr) == 0u);
+      const uint32_t base = (fixed >> 5) | ((one_hi & ~zero_hi) << 27), hw = (fr >> 5) | ((one_hi & zero_hi) << 27);
+      uint32_t hhi = hw, clo = 0;
+      int k = 0;
+      for (; k < 5 && hhi; ++k) {
+        const uint32_t g = hhi & (0u - hhi);
+        hhi ^= g;
+        if ((lane >> k) & 1u) clo |= g;
+      }
+      if ((lane >> k) == 0u) {
+        uint32_t chi = 0;
+        do {
+          uint32_t* const p = set + (base | clo | chi);
+          if ((__ldcg(p) & m) != m) reached += __popc(m & ~atomicOr(p, m));
+          chi = (chi - hhi) & hhi;
+        } while (chi != 0u);
+      }
+    }
+    if (lane == 0) {
+      done[w] = d | take;
+      expanded += __popc(take);
+    }
+  }
+  if (reached != 0ull) atomicAdd(newly, reached);
+  if (lane == 0 && expanded != 0u) atomicAdd(newly + 1, (unsigned long long)expanded);
+}
+
 // Set the bits of states[0, n_states); states >= n_valid (= 2^N) are ignored.  *newly gains the number of bits set.
 __global__ void __launch_bounds__(256) reach_mark_kernel(uint32_t* __restrict__ marks, const uint64_t* __restrict__ states,
                                                          int64_t n_states, uint64_t n_valid,

@@ -1710,4 +1710,22 @@ int pbn_reach_sweep(pbn_handle* h, uint32_t* marks, unsigned long long* newly, v
   return PBN_OK;
 }
 
+int pbn_reach_forward(pbn_handle* h, uint32_t* set, uint32_t* done, unsigned long long* newly, void* stream_) {
+  int rc;
+  if ((rc = reach_args(h, "pbn_reach_forward", set, newly)) != PBN_OK) return rc;
+  if (!done) return fail(PBN_ERR_INVALID, "pbn_reach_forward: null done");
+  const uint64_t S = 1ull << h->net.n_genes;
+  const uint64_t words = S > 32u ? S >> 5 : 1u, per = kDpSliceStates >> 5;
+  cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+  const auto kernel = h->net.n_genes > 32 ? reach_forward_kernel<true> : reach_forward_kernel<false>;
+  DeviceGuard guard(h->device);
+  for (uint64_t w0 = 0; w0 < words; w0 += per) {
+    const uint64_t cnt = words - w0 < per ? words - w0 : per;
+    if ((rc = launch(h, kernel, grid_for(h, (int64_t)cnt * 32, 256, 8), 256, 0, stream, false, h->net, set, done,
+                     (uint32_t)w0, (uint32_t)cnt, newly)) != PBN_OK)
+      return rc;
+  }
+  return PBN_OK;
+}
+
 }  // extern "C"

@@ -16,6 +16,8 @@ Here:
 * :func:`find_attractors_exhaustive` -- for N <= 34: all attractors, with a certificate.  Backward reachability
   over a device bitset of all 2^N states (``pbn_reach_sweep``) from the attractors found so far; states that stay
   unmarked are closed under successors and hold the attractors not found yet, which rollouts from them find.
+* :func:`attractor_in_closure` -- for N <= 34: the attractor reached from a state, of any size, by a forward closure
+  over a device bitset of all 2^N states (``pbn_reach_forward``) and a backward sweep that tests it for a sink SCC.
 * :func:`steady_state_histogram` -- visit counts of (projected) states over many perturbed steps.
 * :func:`steady_state_statistics` / :class:`StateRecorder` -- per-gene ON frequencies and the distribution of the
   state projected onto up to 12 genes, counted on the device (``pbn_rollout_record`` inside the rollout kernel,
@@ -37,7 +39,7 @@ from .vec_env import VecPBNEnv
 
 __all__ = ["VisitCounter", "find_attractors_rollout", "attractor_reached_from", "basin_labels", "steady_state_histogram", "successor_descriptors",
            "forward_closure", "sink_sccs_of_closed_set", "StateRecorder", "steady_state_statistics",
-           "ReachMarks", "find_attractors_exhaustive"]
+           "ReachMarks", "attractor_in_closure", "find_attractors_exhaustive"]
 
 
 def _words_to_int(words: Sequence[int]) -> int:
@@ -329,15 +331,22 @@ class ReachMarks:
     :meth:`close` sweeps "mark ``s`` if a successor of ``s`` (perturbation-free STG) is marked" until a sweep marks
     nothing, which leaves exactly the states that reach a marked one.  :attr:`count` is the number of marked states."""
 
-    def __init__(self, env: VecPBNEnv):
+    def __init__(self, env: VecPBNEnv, marks: Optional[torch.Tensor] = None, count: int = 0):
+        """A cleared bitset, or the caller's ``marks`` (int32 ``[max(1, 2^N / 32)]`` on ``env``'s device, used in place)
+        of which ``count`` valid state bits are set."""
         n = env.n_genes
         if n > _cabi.REACH_MAX_GENES:
             raise _cabi.PbnError(_cabi.PBN_ERR_UNSUPPORTED, "the state bitset covers at most %d genes, the network has %d"
                                  % (_cabi.REACH_MAX_GENES, n))
         self.env, self.n = env, n
-        self.marks = torch.zeros((max(1, (1 << n) >> 5),), dtype=torch.int32, device=env.device)
+        words = max(1, (1 << n) >> 5)
+        if marks is None:
+            marks = torch.zeros((words,), dtype=torch.int32, device=env.device)
+        elif marks.dtype != torch.int32 or marks.shape != (words,) or marks.device != env.device or not marks.is_contiguous():
+            raise ValueError("marks must be a contiguous int32 tensor of %d words on %s" % (words, env.device))
+        self.marks = marks
         self.newly = torch.zeros((1,), dtype=torch.int64, device=env.device)
-        self.count = 0
+        self.count = int(count)
         self.sweeps = 0
 
     def mark(self, states: Sequence[int]) -> int:
@@ -403,9 +412,113 @@ class ReachMarks:
         return out
 
 
+def _bitset_states(bits: torch.Tensor, limit: Optional[int] = None) -> List[int]:
+    """The states whose bits are set in ``bits`` (marks layout), ascending; only the first ``limit`` if given.  Read in
+    chunks of 2^22 words, so that no full-size copy of the bitset is made."""
+    chunk, out = 1 << 22, []
+    shifts = torch.arange(32, dtype=torch.int32, device=bits.device)
+    for c in range(0, bits.numel(), chunk):
+        f = bits[c:c + chunk]
+        words = torch.nonzero(f).reshape(-1)
+        if limit is not None:
+            words = words[:limit - len(out)]
+        if words.numel() == 0:
+            continue
+        wb = torch.nonzero((f[words].unsqueeze(1) >> shifts) & 1)        # (row, bit), row-major: ascending states
+        out += (((words[wb[:, 0]] + c) << 5) | wb[:, 1]).cpu().tolist()
+        if limit is not None and len(out) >= limit:
+            return out[:limit]
+    return out
+
+
+def _bit(bits: torch.Tensor, s: int) -> int:
+    return (int(bits[s >> 5].item()) >> (s & 31)) & 1
+
+
+class _ForwardWorkspace:
+    """Device buffers of :func:`attractor_in_closure`: two bitsets of every state (the closure ``set`` and ``done``,
+    which holds the expanded states and then the sink test's marks), the sweep counters, and totals over its calls."""
+
+    def __init__(self, env: VecPBNEnv):
+        n = env.n_genes
+        if n > _cabi.REACH_MAX_GENES:
+            raise _cabi.PbnError(_cabi.PBN_ERR_UNSUPPORTED, "the state bitset covers at most %d genes, the network has %d"
+                                 % (_cabi.REACH_MAX_GENES, n))
+        self.env, self.n = env, n
+        self.set = torch.zeros((max(1, (1 << n) >> 5),), dtype=torch.int32, device=env.device)
+        self.done = torch.zeros_like(self.set)
+        self.newly = torch.zeros((2,), dtype=torch.int64, device=env.device)
+        self.forward_sweeps = 0    # pbn_reach_forward calls
+        self.backward_sweeps = 0   # pbn_reach_sweep calls of the sink tests
+        self.closures = 0          # forward closures (one per call, plus one per restart)
+
+    def _mark(self, bits: torch.Tensor, s: int) -> None:
+        st = torch.tensor([s], dtype=torch.int64, device=bits.device)
+        check(self.env.lib.pbn_reach_mark(self.env._h, bits.data_ptr(), st.data_ptr(), 1, self.newly.data_ptr(),
+                                          self.env._stream()))
+
+    def close(self, s: int) -> int:
+        """``set`` := the forward closure of ``s``, ``done`` := the same; returns its size."""
+        env = self.env
+        self.set.zero_()
+        self.done.zero_()
+        self._mark(self.set, s)
+        self.closures += 1
+        size = 1
+        while True:
+            self.newly.zero_()
+            check(env.lib.pbn_reach_forward(env._h, self.set.data_ptr(), self.done.data_ptr(), self.newly.data_ptr(),
+                                            env._stream()))
+            self.forward_sweeps += 1
+            reached, expanded = self.newly.tolist()
+            size += reached
+            if expanded == 0:
+                return size
+
+
+def attractor_in_closure(env: VecPBNEnv, seed_state: int, max_states: Optional[int] = None, burn_in: int = 64,
+                         ws: Optional[_ForwardWorkspace] = None, return_bits: bool = False):
+    """The attractor (sink SCC of the perturbation-free STG) reached from ``seed_state``, of any size, for N <= 34.
+
+    1. ``F`` := the forward closure of the candidate ``s`` (first ``seed_state``), swept on the device to its fixed point
+       (``pbn_reach_forward``).  ``F`` is closed under successors.
+    2. ``B`` := ``~F | {s}``, then backward reachability to its fixed point (``pbn_reach_sweep``): the states of ``F``
+       left unmarked are those that do not reach ``s``.  If there are none, ``F`` is strongly connected: the attractor.
+    3. Otherwise those states are closed under successors and exclude ``s``: one of them, moved on by a ``burn_in``-step
+       rollout of ``env`` if that stays among them, is the next candidate.  Its closure is strictly smaller than ``F``.
+
+    Returns ``(size, members)``: ``members`` is the sorted list of states, or ``None`` when ``size > max_states``
+    (``None``: no limit).  With ``return_bits=True`` also the attractor's bitset (int32 words, bit ``s & 31`` of word
+    ``s >> 5``), which is the workspace's and valid until its next use.  Restarts leave ``env``'s states where their
+    rollouts ended; rollouts are skipped when ``env`` perturbs.  Holds two bitsets of 2^N / 8 bytes on the device
+    (``ws``, made if not given): 4 GiB at 34 genes.  N > 34 raises ``PbnError(PBN_ERR_UNSUPPORTED)``."""
+    ws = ws or _ForwardWorkspace(env)
+    n, cand = env.n_genes, int(seed_state)
+    if not 0 <= cand < 1 << n:
+        raise ValueError("seed_state must be a state of the %d-gene network" % n)
+    while True:
+        size = ws.close(cand)
+        ws.done.bitwise_not_()                      # done == F at the fixed point: B = ~F | {cand}
+        ws._mark(ws.done, cand)
+        test = ReachMarks(env, marks=ws.done, count=(1 << n) - size + 1)
+        test.close()
+        ws.backward_sweeps += test.sweeps
+        if test.uncovered == 0:
+            break
+        cand = test.unmarked_sample(1)[0]
+        if int(burn_in) > 0 and env.perturb_p == 0.0:
+            env.set_state(torch.full((env.num_envs, env.n_words), cand, dtype=torch.int64), packed=True)
+            env.rollout(int(burn_in), stats=False)
+            moved = int(env.state[0, 0].item())
+            if _bit(ws.done, moved) == 0:           # still in F and still short of the old candidate
+                cand = moved
+    members = _bitset_states(ws.set) if max_states is None or size <= int(max_states) else None
+    return (size, members, ws.set) if return_bits else (size, members)
+
+
 def find_attractors_exhaustive(network: PBNNetwork, device: Union[str, torch.device] = "cuda:0",
                                seed_rollouts: int = 1 << 16, burn_in: int = 256, max_attractor_states: int = 1 << 14,
-                               seed: int = 0x5EED, max_unresolved: int = 8):
+                               seed: int = 0x5EED, max_unresolved: int = 8, closure: str = "hash"):
     """Every attractor (sink SCC of the perturbation-free STG) of a network of up to 34 genes, with a certificate.
 
     1. Seed: :func:`find_attractors_rollout` with ``seed_rollouts`` rollouts (0: none); the states of its attractors
@@ -420,6 +533,17 @@ def find_attractors_exhaustive(network: PBNNetwork, device: Union[str, torch.dev
        closure's free-gene limit (``complete=False``, with what was found).  A round stops trying end states after
        ``max_unresolved`` failed closures (the end states of one attractor that is too large all fail alike).
 
+    ``closure`` picks how step 3 finds an attractor:
+
+    * ``"hash"`` (default): :func:`attractor_reached_from`, a closure listed in a device hash set, limited to
+      ``max_attractor_states`` states and 16 free genes per state, as described above.
+    * ``"bitset"``: :func:`attractor_in_closure`, a closure over two more bitsets of every state, with no limit.  Every
+      attractor found is marked, however large; those of more than ``max_attractor_states`` states are not listed but
+      reported in ``info["oversized"]`` as ``(size, smallest state)``, sorted by smallest state.  The search always
+      ends with every state marked (``uncovered == 0``), and ``complete`` is ``not oversized``.  ``info`` also holds
+      ``forward_sweeps``, ``backward_sweeps`` (those of the sink tests) and ``closures`` of the attractor searches.
+      Three bitsets of 2^N / 8 bytes: 6 GiB at 34 genes.
+
     Returns ``(AttractorSet, info)`` sorted as :func:`find_attractors_stg` sorts (states ascending inside an attractor,
     attractors by their smallest state); ``info`` holds ``complete``, ``uncovered`` (states left unmarked), ``sweeps``,
     ``rounds`` (discovery rounds; ``sweeps`` may differ from run to run, since a bit set early in a sweep can be seen
@@ -427,9 +551,12 @@ def find_attractors_exhaustive(network: PBNNetwork, device: Union[str, torch.dev
     The bitset takes 2^N / 8 bytes of device memory: 32 MiB at 28 genes, 2 GiB at 34.
     N > 34 raises ``PbnError(PBN_ERR_UNSUPPORTED)``."""
     n = network.n_genes
+    if closure not in ("hash", "bitset"):
+        raise ValueError("closure must be 'hash' or 'bitset', not %r" % (closure,))
     if n > _cabi.REACH_MAX_GENES:
         raise _cabi.PbnError(_cabi.PBN_ERR_UNSUPPORTED, "exhaustive attractor search covers at most %d genes, the network "
                              "has %d" % (_cabi.REACH_MAX_GENES, n))
+    bitset = closure == "bitset"
     attractors: List[List[int]] = []
     if int(seed_rollouts) > 0:
         _, rinfo = find_attractors_rollout(network, n_rollouts=int(seed_rollouts), burn_in=burn_in, device=device,
@@ -444,10 +571,12 @@ def find_attractors_exhaustive(network: PBNNetwork, device: Union[str, torch.dev
         for m in attractors:
             owner.update(m)
             reach.mark(m)
-        ws = _ClosureWorkspace(env, max_attractor_states)
+        ws = _ForwardWorkspace(env) if bitset else _ClosureWorkspace(env, max_attractor_states)
+        oversized: List[Tuple[int, int]] = []
         rounds = 0
         while True:
-            reach.close()
+            if not (bitset and reach.count == 0):      # with nothing marked a sweep marks nothing, at full cost
+                reach.close()
             if reach.uncovered == 0:
                 break
             starts = reach.unmarked_sample(e)
@@ -458,6 +587,22 @@ def find_attractors_exhaustive(network: PBNNetwork, device: Union[str, torch.dev
             ends = torch.unique(env.state[:, 0]).cpu().tolist()
             found = failed = 0
             for s in ends:
+                if bitset:
+                    if _bit(reach.marks, s):         # in an attractor found earlier in this round
+                        continue
+                    size, members, bits = attractor_in_closure(env, int(s), max_attractor_states, burn_in=burn_in, ws=ws,
+                                                               return_bits=True)
+                    first = members[0] if members is not None else _bitset_states(bits, 1)[0]
+                    if _bit(reach.marks, first):
+                        continue
+                    reach.marks.bitwise_or_(bits)     # disjoint from the marks: no state of it reaches another attractor
+                    reach.count += size
+                    if members is None:
+                        oversized.append((size, first))
+                    else:
+                        attractors.append(members)
+                    found += 1
+                    continue
                 if s in owner:
                     continue
                 members = attractor_reached_from(env, int(s), ws, max_states=max_attractor_states)
@@ -476,6 +621,9 @@ def find_attractors_exhaustive(network: PBNNetwork, device: Union[str, torch.dev
                 break
         info = {"complete": reach.uncovered == 0, "uncovered": reach.uncovered, "sweeps": reach.sweeps,
                 "rounds": rounds, "seeded": seeded}
+        if bitset:
+            info.update(complete=reach.uncovered == 0 and not oversized, oversized=sorted(oversized, key=lambda o: o[1]),
+                        forward_sweeps=ws.forward_sweeps, backward_sweeps=ws.backward_sweeps, closures=ws.closures)
     finally:
         env.close()
     attractors.sort(key=lambda m: m[0])
