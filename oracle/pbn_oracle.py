@@ -550,8 +550,14 @@ def sliced_survival(p: float, n: int) -> np.ndarray:
     return out
 
 
+def perturb_block(q: int, i: int) -> int:
+    """Block index of block i of perturbation sub-stream q: 64q + i for the first 64 blocks, then 256 + 192q + (i - 64)
+    (a walk over 8N slots draws up to 8N + 1 words, so the stream never reuses a word)."""
+    return 64 * q + i if i < 64 else 256 + 192 * q + (i - 64)
+
+
 class _WordStream:
-    """Sequential 32-bit words of one (group, step, kind, sub-stream q) stream: blocks 64q + i."""
+    """Sequential 32-bit words of one (group, step, kind, sub-stream q) stream: blocks perturb_block(q, i)."""
 
     def __init__(self, gid, step_ctr, kind, k0, k1, q=0, first_word=0):
         self.gid, self.step, self.kind, self.k0, self.k1, self.q = gid, step_ctr, kind, k0, k1, q
@@ -561,7 +567,7 @@ class _WordStream:
     def word(self):
         if (self.next & 3) == 0 or self.blk is None:
             r = philox4x32(*_ctr(np.array([self.gid], dtype=np.uint64), self.step, self.kind,
-                                 64 * self.q + ((self.next >> 2) & 63)), self.k0, self.k1)
+                                 perturb_block(self.q, self.next >> 2)), self.k0, self.k1)
             self.blk = [int(x[0]) for x in r]
         w = self.blk[self.next & 3]
         self.next += 1

@@ -57,6 +57,13 @@ __device__ __forceinline__ Philox4 philox_stream_rk(uint64_t id, uint64_t step, 
   return philox4x32_10_rk((uint32_t)id, (uint32_t)(id >> 32), (uint32_t)step, c3, rk);
 }
 
+// Block i of the sliced kernels' perturbation sub-stream q (0..3).  The walk draws one word per event plus one, up to
+// 8N + 1 = 769 words (193 blocks) at N = 96: blocks 64q + i for the first 64, then 256 + 192q + (i - 64), so a dense
+// walk never wraps onto words it has already used.
+__device__ __forceinline__ uint32_t pert_block(uint32_t q, uint32_t i) {
+  return i < 64u ? 64u * q + i : 256u + 192u * q + (i - 64u);
+}
+
 // Counter layout shared by every stream of the library (include/pbn_b200.h "Random streams").
 __device__ __forceinline__ Philox4 philox_stream(uint64_t id, uint64_t step, uint32_t kind, uint32_t idx,
                                                  uint32_t k0, uint32_t k1) {

@@ -287,11 +287,11 @@ __device__ __forceinline__ void step_planes_body(const StepParams& p, const Plan
         // pos iff u < S[rem] -- one table read settles the usual case, the search runs for real events only)
         const uint32_t ws = w & 3u;
         uint32_t mb = 0u, k = 0u;
-        Philox4 blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, 64u * ws, n.rk);
+        Philox4 blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, pert_block(ws, 0u), n.rk);
         int pos = -1;
         uint32_t s_rem = kSurvTable[kSlots];
         while (true) {
-          if (k != 0u && (k & 3u) == 0u) blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, 64u * ws + ((k >> 2) & 63u), n.rk);
+          if (k != 0u && (k & 3u) == 0u) blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, pert_block(ws, k >> 2), n.rk);
           const uint32_t u = pick4(blk, k & 3u);
           ++k;
           if (u < s_rem) break;

@@ -37,7 +37,8 @@
 //           bit b of the plane if they are still at 3 there and no earlier slot of the group has claimed bit b of this
 //           plane; blocks are consumed until no slot of the group is at 3 anywhere in the column.  Exactly uniform
 //           1-of-3, all choices independent (no random pair is used twice).  sel = s0 + 2*s1.
-//   PERTURB: sub-stream q = b >> 3 (Philox blocks (PERTURB, 64q + i)) covers the 8 slice bits
+//   PERTURB: sub-stream q = b >> 3 (Philox blocks (PERTURB, pert_block(q, i)), philox.cuh and DESIGN.md §4: 64q + i
+//           for i < 64, then 256 + 192q + (i - 64)) covers the 8 slice bits
 //           8q..8q+7: geometric skipping over slots gene*8 + (b & 7) with survival table S[0..8N].
 //   RESET:  per env (global env id), as in the scalar kernel.
 //
@@ -259,11 +260,11 @@ __device__ __forceinline__ void draw_pert_events(const NetParams& n, uint32_t* e
     // none is left in the rem slots after pos iff u < S[rem]: one table read settles the usual case, the search runs
     // for real events only
     uint32_t s_rem = kSurvTable[kSlots];
-    Philox4 blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, 64u * w, n.rk);
+    Philox4 blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, pert_block(w, 0u), n.rk);
     int pos = -1;
 #pragma unroll 1
     for (uint32_t k = 0;; ++k) {   // up to kEvCap events are packed
-      if (k != 0u && (k & 3u) == 0u) blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, 64u * w + ((k >> 2) & 63u), n.rk);   // rare
+      if (k != 0u && (k & 3u) == 0u) blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, pert_block(w, k >> 2), n.rk);   // rare
       const uint32_t u = pick4(blk, k & 3u);
       if (u < s_rem) break;
       pos += pert_search(n, u);
@@ -557,7 +558,7 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
       int pos = -1;
       while (true) {
         if ((pert_next & 3u) == 0u)
-          pert_blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, 64u * w + ((pert_next >> 2) & 63u), n.rk);
+          pert_blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, pert_block(w, pert_next >> 2), n.rk);
         const uint32_t u = pick4(pert_blk, pert_next & 3u);
         ++pert_next;
         pos += (u < s_last) ? kSlots + 1 : pert_search(n, u);
@@ -700,7 +701,7 @@ __device__ __forceinline__ void tile_step(const StepParams& p, const SlicedSmemL
         int pos = -1;
         while (true) {
           if ((pert_next & 3u) == 0u)
-            pert_blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, 64u * w + ((pert_next >> 2) & 63u), n.rk);
+            pert_blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, pert_block(w, pert_next >> 2), n.rk);
           const uint32_t u = pick4(pert_blk, pert_next & 3u);
           ++pert_next;
           pos += (u < s_last) ? kSlots + 1 : pert_search(n, u);
@@ -1292,7 +1293,7 @@ __global__ void __launch_bounds__(PBN_THREADS, PBN_MIN_BLOCKS) pbn_rollout_slice
             Philox4 blk = {0u, 0u, 0u, 0u};
             int pos = -1;
             while (true) {
-              if ((pert_next & 3u) == 0u) blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, 64u * w + ((pert_next >> 2) & 63u), n.rk);
+              if ((pert_next & 3u) == 0u) blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, pert_block(w, pert_next >> 2), n.rk);
               const uint32_t u = pick4(blk, pert_next & 3u);
               ++pert_next;
               pos += (u < s_last) ? kSlots + 1 : pert_search(n, u);
@@ -1317,7 +1318,7 @@ __global__ void __launch_bounds__(PBN_THREADS, PBN_MIN_BLOCKS) pbn_rollout_slice
           Philox4 blk = {0u, 0u, 0u, 0u};
           int pos = -1;
           while (true) {
-            if ((pert_next & 3u) == 0u) blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, 64u * w + ((pert_next >> 2) & 63u), n.rk);
+            if ((pert_next & 3u) == 0u) blk = philox_stream_rk(gid, step_ctr, PBN_RNG_PERTURB, pert_block(w, pert_next >> 2), n.rk);
             const uint32_t u = pick4(blk, pert_next & 3u);
             ++pert_next;
             pos += (u < s_last) ? kSlots + 1 : pert_search(n, u);

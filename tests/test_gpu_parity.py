@@ -288,12 +288,13 @@ def test_large_batch_properties(kernel):
 
 
 @pytest.mark.parametrize("name,e,p", [("pbn28", 1 << 17, 1e-5), ("pbn28", 8192, 0.3), ("pbn70", 1 << 15, 2e-5),
-                                      ("pbn70", 4096, 0.2), ("pbn7", 1 << 16, 3e-4)])
+                                      ("pbn70", 4096, 0.2), ("pbn7", 1 << 16, 3e-4), ("pbn70", 4096, 0.6)])
 def test_perturbation_stream_extremes(name, e, p):
     """The geometric skip of the sliced kernel (float first guess + exact table window, binary search as
     fallback; events pre-drawn into packed words, overflow redone in phase D) against the oracle's plain walk
     over the survival table: very rare events (the float guess is least accurate) and very frequent ones
-    (every thread overflows its pre-drawn list)."""
+    (every thread overflows its pre-drawn list; at pbn70 and p = 0.6 a sub-stream's walk draws about 336 words, past its
+    first 64 Philox blocks into the range pert_block continues it in)."""
     import torch
     from oracle import pbn_oracle as O
     case = random_case(name, e, seed=13)
